@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the DDPM/DDIM hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload train|ddim]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload train|ddim] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -224,6 +224,36 @@ def _build_ours(config, dev):
     return model, diff, opt, EMA(model, decay=ema_decay), make_grad_scaler("cuda", True), gf_train, img
 
 
+DUMP_SAMPLE = 1 << 21          # elements kept per parameter-sized array: 8 MB each in float32, 32 MB for all four
+
+
+def dump_outputs(out_dir, model, opt, ema, scaler, ret, losses):
+    """Write what the timed `train_one_epoch` call hands back to its caller, as .npy files: its return value, the per-step
+    losses, and the model state the last step left behind (parameters, AdamW moments, EMA shadow; flattened in
+    `model.parameters()` order and sampled at the same fixed, seeded indices, sorted).  The gradients are not written:
+    the step zeroes them."""
+    import numpy as np
+    params = list(model.parameters())
+    n = sum(p.numel() for p in params)
+    idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+
+    def sampled(ts):
+        return torch.cat([t.detach().reshape(-1).cpu() for t in ts])[idx].numpy().astype(np.float32)
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {
+        "avg_loss": np.array([ret[0]], dtype=np.float64),
+        "step_losses": losses.numpy().astype(np.float32),
+        "grad_scale": np.array([scaler.get_scale()], dtype=np.float64),
+        "params": sampled(params),
+        "adam_exp_avg": sampled([opt.state[p]["exp_avg"] for p in params]),
+        "adam_exp_avg_sq": sampled([opt.state[p]["exp_avg_sq"] for p in params]),
+        "ema_shadow": sampled(ema.shadow),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     import contextlib
     import io
@@ -313,6 +343,8 @@ def run_ours(args):
     enqueue_ms = last_enqueue_ms_per_step()           # host loop time per step, excluding the final synchronising loss read
     graph_steps = last_graph_steps()                  # timed steps that ran as ONE CUDA-graph replay each (train_one_epoch._GraphStep)
     pool_misses = _engine.POOL.misses - miss0
+    if args.dump_outputs and rank == 0:               # before the legs below train the same model further
+        dump_outputs(args.dump_outputs, model, opt, ema, scaler, last, last_step_losses())
     # ... which includes back-pressure once the launch queue is full (the GPU is the bottleneck at this batch).  The host's own
     # cost per step is what the same loop takes when the GPU is NOT the limit: the same epoch on two-image batches.
     x_tiny = x_dev[:2].contiguous()
@@ -526,7 +558,13 @@ def main():
     ap.add_argument("--no-ddim", action="store_true", help="skip the DDIM-100 sampling leg")
     ap.add_argument("--ddim-batch", type=int, default=256, help="images per GPU for the DDIM-100 leg")
     ap.add_argument("--profile", action="store_true", help="2 warm-up steps + 1 step, no JSON (for ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed train_one_epoch call returned and left in the model after its last step "
+                         "to DIR/<name>.npy (float32/float64, 32 MB; large arrays as a fixed seeded sample); same "
+                         "arguments give the same inputs, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.profile):
+        ap.error("--dump-outputs needs --impl ours and no --profile")
     if args.impl == "reference":
         run_reference(args)
     else:
