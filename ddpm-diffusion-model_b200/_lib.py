@@ -113,9 +113,7 @@ SIGNATURES = {
     "ddpm_rng_advance": [_vp, _vp],
     "ddpm_set_force_simt": [_i],
     "ddpm_set_tc_mode": [_i, _i],
-    "ddpm_set_tc_v2": [_i],
     "ddpm_set_pdl": [_i],
-    "ddpm_set_gn_slab": [_i],
     "ddpm_abi_struct_sizes": [_vp, _i],
 }
 

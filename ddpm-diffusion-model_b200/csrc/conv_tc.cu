@@ -10,17 +10,10 @@
 // re-read of the activation never happens (neither from HBM nor from L2).  Outputs computed at halo
 // positions are discarded by the epilogue, which keeps the output halo zero.
 //
-// Warp roles (192 threads): warp 0 = TMA producer, warp 1 = TMEM allocator + single-thread MMA
-// issuer, warps 2..5 = epilogue (tcgen05.ld -> +bias +time-bias +residual -> bf16 -> global).
-// Two mbarrier rings: A patches (one per K-chunk) and B weight tiles (TPB taps x NT x 16ch).
-// Accumulators: MT tiles of 128 x NT fp32 in TMEM (MT*NT <= 256 columns so two CTAs share an SM and
-// one CTA's epilogue overlaps the other's main loop).
-//
 // Replaces cuDNN behind nn.Conv2d 3x3 s1 / 1x1 (unet_backbone.py:22,32,35,60; attention.py:53-54)
 // for fprop and, with flipped/transposed weights, dgrad.
 #include "common.cuh"
 #include <cuda.h>
-#include <cooperative_groups.h>
 #include <type_traits>
 #include <cudaTypedefs.h>
 
@@ -28,11 +21,13 @@
 #define KC 16                 // channels per K-chunk (one UMMA K step for bf16)
 
 static int sm_count();
-static int g_tc_mode = 1;     // 0: SWIZZLE_NONE ("interleave") operand layout, 1: SWIZZLE_32B (default)
-static int g_tc_baseoff = 0;  // measured on B200: the swizzle is a pure function of the smem address, so row-shifted
-                              // descriptors need base_offset = 0 (setting it from the address gives wrong results)
-static int g_tc_exp = 0;      // diagnostics only (tools/kbench.py): bit0 skip A loads after the first ring fill, bit1 same for B
-extern "C" int ddpm_set_tc_mode(int mode, int baseoff) { g_tc_mode = mode & 1; g_tc_exp = mode >> 4; g_tc_baseoff = baseoff; return 0; }
+// path-forcing flags of ddpm_set_tc_mode (mode >> 4, see ddpm_b200.h), read by the launch planners below
+static int g_tc_exp = 0;
+extern "C" int ddpm_set_tc_mode(int mode, int base_offset) {
+    if ((mode & 15) != 1 || base_offset != 0 || ((mode >> 4) & ~(32 | 64 | 128 | 1024))) return DDPM_E_ARG;
+    g_tc_exp = mode >> 4;
+    return 0;
+}
 
 // ------------------------------------------------------------------------------------------------
 // PTX wrappers
@@ -66,14 +61,6 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* m, uin
     asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
                  ::"r"(smem_u32(dst)), "l"(m), "r"(smem_u32(bar)), "r"(c0), "r"(c1) : "memory");
 }
-__device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2) {
-    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-                 ::"r"(smem_u32(dst)), "l"(m), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-__device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2, int c3) {
-    asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-                 ::"r"(smem_u32(dst)), "l"(m), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
 
 __device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t ncols) {
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(ncols) : "memory");
@@ -100,18 +87,9 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t* r) {
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
-// shared-memory matrix descriptor (cute::UMMA::SmemDescriptor bit layout)
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes, uint32_t layout, uint32_t base_off) {
-    uint64_t d = 0;
-    d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-    d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
-    d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32;
-    d |= (uint64_t)1 << 46;                       // descriptor version (Blackwell)
-    d |= (uint64_t)(base_off & 7) << 49;
-    d |= (uint64_t)(layout & 7) << 61;
-    return d;
-}
-
+// Shared-memory matrix descriptors (cute::UMMA::SmemDescriptor bit layout: start address >> 4, LBO >> 4 at bit 16,
+// SBO >> 4 at bit 32, version 1 at bit 46, layout at bit 61).  The base offset (bits 49-51) stays 0: the swizzle is a
+// pure function of the shared-memory address, so row-shifted descriptors need no correction (measured on B200).
 // The MMA-issuing thread is a single lane: every integer instruction between two tcgen05.mma costs
 // ~5 cycles of dependent latency, and a loop that rebuilds both 64-bit descriptors (shifts, masks,
 // tap / 3, tap % 3) per MMA was measured at 137-230 cycles per MMA -- above the 48-128 cycle tensor
@@ -126,204 +104,6 @@ __device__ __forceinline__ uint32_t desc_hi(uint32_t sbo_bytes, uint32_t layout)
 }
 __device__ __forceinline__ uint32_t desc_lo(uint32_t saddr, uint32_t lbo_bytes) {
     return ((saddr >> 4) & 0x3FFF) | (((lbo_bytes >> 4) & 0x3FFF) << 16);
-}
-
-// ------------------------------------------------------------------------------------------------
-// kernel
-// ------------------------------------------------------------------------------------------------
-struct TcParams {
-    TV out, res;
-    const float* bias; const float* tbias; int tbias_pitch; int bias_n;
-    int Cin, Cout, NT;          // NT: output-channel tile (UMMA N), multiple of 16, <= 256
-    int taps, tpb;              // 9 (3x3) or 1; taps per B stage (3 or 1)
-    int Hp, Wp, H, W, Qtot;     // padded geometry shared by input and output
-    int P, seg;                 // patch rows per A stage = nseg * seg (seg = TMA box height, multiple of 8)
-    int SA, SB;                 // ring depths
-    int a_stage_bytes, b_stage_bytes;
-    int tmem_cols;              // power of two >= MT*NT
-    int has_res, accum;
-    int baseoff, exp;
-    int sub;                    // 1: stride-2 conv = stride-1 conv kept at even (y, x) only
-};
-
-template <int MT, bool SW32>
-__global__ void __launch_bounds__(TC_THREADS) conv_tc_kernel(const __grid_constant__ CUtensorMap tmA,
-                                                              const __grid_constant__ CUtensorMap tmB, TcParams p) {
-    extern __shared__ __align__(1024) uint8_t smem_raw[];
-    uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    uint8_t* a_ring = smem;
-    uint8_t* b_ring = a_ring + (size_t)p.SA * p.a_stage_bytes;
-    uint64_t* bars = (uint64_t*)(b_ring + (size_t)p.SB * p.b_stage_bytes);
-    uint64_t* a_full = bars;            uint64_t* a_empty = a_full + p.SA;
-    uint64_t* b_full = a_empty + p.SA;  uint64_t* b_empty = b_full + p.SB;
-    uint64_t* acc_full = b_empty + p.SB;
-    uint32_t* tmem_slot = (uint32_t*)(acc_full + 1);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int Q0 = blockIdx.x * (128 * MT);
-    const int n0 = blockIdx.y * p.NT;
-    const int KCH = p.Cin / KC;                         // K chunks
-    const int BG = p.taps / p.tpb;                      // B stages per K chunk
-    const int row_bytes = SW32 ? 32 : 16;               // bytes between consecutive pixel rows in smem
-    const int halo_rows = (p.taps == 9) ? p.Wp + 1 : 0; // rows in front of the tile inside the patch
-
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < p.SA; ++i) { mbar_init(&a_full[i], 1); mbar_init(&a_empty[i], 1); }
-        for (int i = 0; i < p.SB; ++i) { mbar_init(&b_full[i], 1); mbar_init(&b_empty[i], 1); }
-        mbar_init(acc_full, 1);
-        fence_barrier_init();
-    }
-    if (warp == 1) tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-
-    if (warp == 0) {
-        // ===================================================================== TMA producer
-        if (lane == 0) {
-            int sb = 0; uint32_t pb = 0;
-            for (int kc = 0; kc < KCH; ++kc) {
-                const int sa = kc % p.SA; const uint32_t pa = (kc / p.SA) & 1;
-                mbar_wait(&a_empty[sa], pa ^ 1);
-                uint8_t* adst = a_ring + (size_t)sa * p.a_stage_bytes;
-                const bool skipA = (p.exp & 1) && kc >= p.SA;
-                if (skipA) mbar_arrive(&a_full[sa]); else mbar_expect_tx(&a_full[sa], (uint32_t)(p.P * 32));
-                const int row0 = Q0 - halo_rows;
-                for (int r = 0; r < p.P && !skipA; r += p.seg) {          // one TMA box of `seg` rows per op
-                    if (SW32) {
-                        tma_load_2d(adst + (size_t)r * 32, &tmA, &a_full[sa], kc * KC, row0 + r);
-                    } else {
-                        tma_load_3d(adst + (size_t)r * 16, &tmA, &a_full[sa], 0, row0 + r, kc * 2);
-                        tma_load_3d(adst + (size_t)p.P * 16 + (size_t)r * 16, &tmA, &a_full[sa], 0, row0 + r, kc * 2 + 1);
-                    }
-                }
-                for (int g = 0; g < BG; ++g) {
-                    mbar_wait(&b_empty[sb], pb ^ 1);
-                    uint8_t* bdst = b_ring + (size_t)sb * p.b_stage_bytes;
-                    const bool skipB = (p.exp & 2) && (kc * BG + g) >= p.SB;
-                    if (skipB) mbar_arrive(&b_full[sb]); else mbar_expect_tx(&b_full[sb], (uint32_t)(p.tpb * p.NT * 32));
-                    for (int t = 0; t < p.tpb && !skipB; ++t) {
-                        const int tap = g * p.tpb + t;
-                        if (SW32) tma_load_3d(bdst + (size_t)t * p.NT * 32, &tmB, &b_full[sb], kc * KC, tap, n0);
-                        else tma_load_4d(bdst + (size_t)t * p.NT * 32, &tmB, &b_full[sb], 0, n0, kc * 2, tap);
-                    }
-                    if (++sb == p.SB) { sb = 0; pb ^= 1; }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ===================================================================== MMA issuer
-        if (lane == 0) {
-            const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(p.NT >> 3) << 17) | ((128u >> 4) << 24);
-            const uint32_t layout = SW32 ? 6u : 0u;
-            const uint32_t a_lbo = SW32 ? 16u : (uint32_t)p.P * 16u;
-            const uint32_t b_lbo = SW32 ? 16u : (uint32_t)p.NT * 16u;
-            const uint32_t sbo = SW32 ? 256u : 128u;
-            int sb = 0; uint32_t pb = 0;
-            for (int kc = 0; kc < KCH; ++kc) {
-                const int sa = kc % p.SA; const uint32_t pa = (kc / p.SA) & 1;
-                mbar_wait(&a_full[sa], pa);
-                tc_fence_after();
-                const uint32_t a_base = smem_u32(a_ring + (size_t)sa * p.a_stage_bytes);
-                for (int g = 0; g < BG; ++g) {
-                    mbar_wait(&b_full[sb], pb);
-                    tc_fence_after();
-                    const uint32_t b_base = smem_u32(b_ring + (size_t)sb * p.b_stage_bytes);
-                    for (int t = 0; t < p.tpb; ++t) {
-                        const int tap = g * p.tpb + t;
-                        const int shift = (p.taps == 9) ? (tap / 3) * p.Wp + (tap % 3) : 0;
-                        const uint32_t baddr = b_base + (uint32_t)(t * p.NT * 32);
-                        const uint64_t bdesc = make_desc(baddr, b_lbo, sbo, layout, 0);
-#pragma unroll
-                        for (int mt = 0; mt < MT; ++mt) {
-                            const uint32_t aaddr = a_base + (uint32_t)((mt * 128 + shift) * row_bytes);
-                            const uint32_t boff = (SW32 && p.baseoff) ? ((aaddr >> 7) & 7u) : 0u;
-                            const uint64_t adesc = make_desc(aaddr, a_lbo, sbo, layout, boff);
-                            umma_bf16(tmem_base + (uint32_t)(mt * p.NT), adesc, bdesc, idesc, (kc | tap) != 0 ? 1u : 0u);
-                        }
-                    }
-                    umma_commit(&b_empty[sb]);
-                    if (++sb == p.SB) { sb = 0; pb ^= 1; }
-                }
-                umma_commit(&a_empty[sa]);
-            }
-            umma_commit(acc_full);
-        }
-    } else {
-        // ===================================================================== epilogue
-        const int qd = warp & 3;                         // TMEM lane quarter this warp may read
-        mbar_wait(acc_full, 0);
-        tc_fence_after();
-        const int HpWp = p.Hp * p.Wp;
-#pragma unroll 1
-        for (int mt = 0; mt < MT; ++mt) {
-            const int Q = Q0 + mt * 128 + qd * 32 + lane;
-            bool valid = Q < p.Qtot;
-            int n = 0, y = 0, x = 0;
-            if (valid) {
-                n = Q / HpWp; int r = Q - n * HpWp; int yp = r / p.Wp; int xp = r - yp * p.Wp;
-                y = yp - 1; x = xp - 1;
-                valid = y >= 0 && y < p.H && x >= 0 && x < p.W;
-                if (p.sub) { valid = valid && ((y | x) & 1) == 0; y >>= 1; x >>= 1; }
-            }
-            bf16* orow = valid ? p.out.at<bf16>(n, y, x, n0) : nullptr;
-            const bf16* rrow = (valid && p.has_res) ? p.res.at<bf16>(n, y, x, n0) : nullptr;
-            const float* tb = (valid && p.tbias) ? p.tbias + (size_t)n * p.tbias_pitch + n0 : nullptr;
-#pragma unroll 1
-            for (int c0 = 0; c0 < p.NT; c0 += 16) {
-                uint32_t r[16];
-                tmem_ld16(tmem_base + ((uint32_t)(qd * 32) << 16) + (uint32_t)(mt * p.NT + c0), r);
-                tmem_ld_wait();
-                if (valid && n0 + c0 < p.Cout) {
-                    float v[16];
-#pragma unroll
-                    for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-                    if (p.bias) {
-#pragma unroll
-                        for (int i = 0; i < 16; ++i) if (n0 + c0 + i < p.bias_n) v[i] += __ldg(p.bias + n0 + c0 + i);
-                    }
-                    if (tb) {
-#pragma unroll
-                        for (int i = 0; i < 16; ++i) v[i] += __ldg(tb + c0 + i);
-                    }
-                    if (rrow) {
-                        uint4 a = *reinterpret_cast<const uint4*>(rrow + c0), b = *reinterpret_cast<const uint4*>(rrow + c0 + 8);
-                        const __nv_bfloat162* ha = reinterpret_cast<const __nv_bfloat162*>(&a);
-                        const __nv_bfloat162* hb = reinterpret_cast<const __nv_bfloat162*>(&b);
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            float2 fa = __bfloat1622float2(ha[i]), fb = __bfloat1622float2(hb[i]);
-                            v[2 * i] += fa.x; v[2 * i + 1] += fa.y; v[8 + 2 * i] += fb.x; v[8 + 2 * i + 1] += fb.y;
-                        }
-                    }
-                    if (p.accum) {
-                        uint4 a = *reinterpret_cast<const uint4*>(orow + c0), b = *reinterpret_cast<const uint4*>(orow + c0 + 8);
-                        const __nv_bfloat162* ha = reinterpret_cast<const __nv_bfloat162*>(&a);
-                        const __nv_bfloat162* hb = reinterpret_cast<const __nv_bfloat162*>(&b);
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            float2 fa = __bfloat1622float2(ha[i]), fb = __bfloat1622float2(hb[i]);
-                            v[2 * i] += fa.x; v[2 * i + 1] += fa.y; v[8 + 2 * i] += fb.x; v[8 + 2 * i + 1] += fb.y;
-                        }
-                    }
-                    uint4 o0, o1;
-                    __nv_bfloat162* h0 = reinterpret_cast<__nv_bfloat162*>(&o0);
-                    __nv_bfloat162* h1 = reinterpret_cast<__nv_bfloat162*>(&o1);
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        h0[i] = __floats2bfloat162_rn(v[2 * i], v[2 * i + 1]);
-                        h1[i] = __floats2bfloat162_rn(v[8 + 2 * i], v[8 + 2 * i + 1]);
-                    }
-                    *reinterpret_cast<uint4*>(orow + c0) = o0;
-                    *reinterpret_cast<uint4*>(orow + c0 + 8) = o1;
-                }
-            }
-        }
-        tc_fence_before();
-    }
-    __syncthreads();
-    if (warp == 1) { tc_fence_after(); tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols); }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -351,7 +131,7 @@ static int encode(CUtensorMap* m, void* base, int rank, const uint64_t* dims, co
     return r == CUDA_SUCCESS ? 0 : 1;   // cudaErrorInvalidValue
 }
 
-// shared with norm_kernels.cu (slab GroupNorm): bf16 tiled tensor map, swizzle_bytes in {0, 32, 64, 128}
+// shared with attn_tc.cu: bf16 tiled tensor map, swizzle_bytes in {0, 32, 64, 128}
 int ddpm_encode_tiled_bf16(CUtensorMap* m, void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
                            const uint32_t* box, int swizzle_bytes) {
     int rc = get_encode(); if (rc) return rc;
@@ -366,11 +146,10 @@ static int pick_nt(int Cout) {
     return 0;
 }
 
-int g_tc_v2_flag();
 int conv_tc_supported(const ddpm_conv_args* a) {
     const bool up = a->mode == DDPM_CONV_UP2X_PHASE;
     if (a->dtype != DDPM_BF16 || (a->mode != DDPM_CONV_NORMAL && !up) || a->a_silu || a->z.ptr) return 0;
-    if (up) { if (a->KH != 2 || a->KW != 2 || a->stride != 1 || !g_tc_v2_flag() || g_tc_mode != 1 || a->res.ptr || a->in2.ptr || (a->epi & DDPM_EPI_ACCUM)) return 0; }
+    if (up) { if (a->KH != 2 || a->KW != 2 || a->stride != 1 || a->res.ptr || a->in2.ptr || (a->epi & DDPM_EPI_ACCUM)) return 0; }
     else if (!((a->KH == 3 && a->KW == 3 && a->pad == 1) || (a->KH == 1 && a->KW == 1 && a->pad == 0))) return 0;
     const ddpm_tensor &in = a->in, &out = a->out;
     if (in.halo != 1 || out.halo != 1 || in.N != out.N) return 0;
@@ -384,97 +163,23 @@ int conv_tc_supported(const ddpm_conv_args* a) {
     if (pick_nt(out.C) == 0) return 0;
     if (in.W + 2 > 300) return 0;         // patch would not fit the A ring (large images: later round)
     if (a->gn_ab) {                       // GroupNorm (+SiLU) on the input operand: persistent pair kernel, stride-1 3x3 / 1x1 only
-        if (!g_tc_v2_flag() || g_tc_mode != 1 || up || a->stride != 1 || (a->epi & DDPM_EPI_DSILU)) return 0;
+        if (up || a->stride != 1 || (a->epi & DDPM_EPI_DSILU)) return 0;
         if (((uintptr_t)a->gn_ab & 15) || a->gn_act < 0 || a->gn_act > 1) return 0;
     }
     if (a->in2.ptr) {                     // fused 1x1 second operand: persistent pair kernel, 3x3 stride-1 main conv only
         const ddpm_tensor& i2 = a->in2;
-        if (!g_tc_v2_flag() || g_tc_mode != 1 || a->KH != 3 || a->stride != 1 || (a->epi & DDPM_EPI_DSILU)) return 0;
+        if (a->KH != 3 || a->stride != 1 || (a->epi & DDPM_EPI_DSILU)) return 0;
         if (i2.halo != 1 || i2.C % 16 || i2.pitch % 8 || ((uintptr_t)i2.ptr & 15) || ((uintptr_t)a->w2 & 15)) return 0;
     }
     return 1;
 }
 
-template <int MT, bool SW32>
-static int launch(const CUtensorMap& tmA, const CUtensorMap& tmB, const TcParams& p, dim3 grid, size_t smem, cudaStream_t st) {
-    static size_t configured = 0;
-    if (smem > configured) {
-        CUDA_TRY(cudaFuncSetAttribute(conv_tc_kernel<MT, SW32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured = smem;
-    }
-    conv_tc_kernel<MT, SW32><<<grid, TC_THREADS, smem, st>>>(tmA, tmB, p);
-    LAUNCH_OK();
-    return 0;
-}
-
-static int conv_tc2_launch(const ddpm_conv_args* a, cudaStream_t st);
-extern int g_tc_v2_flag();
-int conv_tc_launch(const ddpm_conv_args* a, cudaStream_t st) {
-    int rc = get_encode(); if (rc) return rc;
-    if (g_tc_v2_flag() && g_tc_mode == 1) return conv_tc2_launch(a, st);
-    const bool sw32 = g_tc_mode == 1;
-    TcParams p;
-    p.out = TV(a->out);
-    p.has_res = a->res.ptr != nullptr; p.res = p.has_res ? TV(a->res) : TV(a->out);
-    p.bias = a->bias; p.tbias = a->tbias; p.tbias_pitch = a->tbias_pitch;
-    p.bias_n = a->bias_n > 0 ? a->bias_n : a->out.C;
-    p.Cin = a->in.C; p.Cout = a->out.C; p.NT = pick_nt(p.Cout);
-    p.taps = a->KH * a->KW; p.tpb = p.taps == 9 ? 3 : 1;
-    p.Hp = a->in.H + 2; p.Wp = a->in.W + 2; p.H = a->in.H; p.W = a->in.W;
-    p.Qtot = a->in.N * p.Hp * p.Wp;
-    p.accum = (a->epi & DDPM_EPI_ACCUM) ? 1 : 0;
-    p.baseoff = g_tc_baseoff; p.exp = g_tc_exp;
-    p.sub = a->stride == 2 ? 1 : 0;
-    int MT = 256 / p.NT; if (MT >= 2) MT = 2; if (MT < 1) MT = 1;
-    int halo_rows = p.taps == 9 ? p.Wp + 1 : 0;
-    {
-        int need = 128 * MT + 2 * halo_rows;
-        int nseg = (need + 255) / 256;
-        p.seg = (((need + nseg - 1) / nseg) + 7) & ~7;
-        p.P = p.seg * nseg;
-    }
-    p.a_stage_bytes = (p.P * 32 + 1023) & ~1023;
-    p.b_stage_bytes = (p.tpb * p.NT * 32 + 1023) & ~1023;
-    p.tmem_cols = 32; while (p.tmem_cols < MT * p.NT) p.tmem_cols <<= 1;
-    // ring depths inside ~110 KB so two CTAs are co-resident per SM
-    const int budget = 108 * 1024;
-    p.SA = 3; p.SB = 4;
-    while (p.SA > 2 && p.SA * p.a_stage_bytes + p.SB * p.b_stage_bytes > budget) --p.SA;
-    while (p.SB > 2 && p.SA * p.a_stage_bytes + p.SB * p.b_stage_bytes > budget) --p.SB;
-    size_t smem = (size_t)p.SA * p.a_stage_bytes + (size_t)p.SB * p.b_stage_bytes + 8 * (2 * p.SA + 2 * p.SB + 1) + 16 + 1024;
-    if (smem > 227 * 1024) return DDPM_E_ARG;
-
-    CUtensorMap tmA, tmB;
-    const uint64_t rows = (uint64_t)p.Qtot;
-    const uint32_t abox_rows = (uint32_t)p.seg;
-    if (sw32) {
-        uint64_t da[2] = {(uint64_t)p.Cin, rows}; uint64_t sa[1] = {(uint64_t)a->in.pitch * 2};
-        uint32_t ba[2] = {KC, abox_rows};
-        if (encode(&tmA, a->in.ptr, 2, da, sa, ba, CU_TENSOR_MAP_SWIZZLE_32B)) return 1;
-        uint64_t db[3] = {(uint64_t)p.Cin, (uint64_t)p.taps, (uint64_t)p.Cout};
-        uint64_t sb[2] = {(uint64_t)p.Cin * 2, (uint64_t)p.taps * p.Cin * 2};
-        uint32_t bb[3] = {KC, 1, (uint32_t)p.NT};
-        if (encode(&tmB, (void*)a->w, 3, db, sb, bb, CU_TENSOR_MAP_SWIZZLE_32B)) return 1;
-    } else {
-        uint64_t da[3] = {8, rows, (uint64_t)p.Cin / 8}; uint64_t sa[2] = {(uint64_t)a->in.pitch * 2, 16};
-        uint32_t ba[3] = {8, abox_rows, 1};
-        if (encode(&tmA, a->in.ptr, 3, da, sa, ba, CU_TENSOR_MAP_SWIZZLE_NONE)) return 1;
-        uint64_t db[4] = {8, (uint64_t)p.Cout, (uint64_t)p.Cin / 8, (uint64_t)p.taps};
-        uint64_t sb[3] = {(uint64_t)p.taps * p.Cin * 2, 16, (uint64_t)p.Cin * 2};
-        uint32_t bb[4] = {8, (uint32_t)p.NT, 2, 1};
-        if (encode(&tmB, (void*)a->w, 4, db, sb, bb, CU_TENSOR_MAP_SWIZZLE_NONE)) return 1;
-    }
-    dim3 grid(ceil_div(p.Qtot, 128 * MT), p.Cout / p.NT);
-    if (MT == 2) return sw32 ? launch<2, true>(tmA, tmB, p, grid, smem, st) : launch<2, false>(tmA, tmB, p, grid, smem, st);
-    return sw32 ? launch<1, true>(tmA, tmB, p, grid, smem, st) : launch<1, false>(tmA, tmB, p, grid, smem, st);
-}
-
 // ================================================================================================
-// v2: persistent CTA-PAIR kernel (cta_group::2), TMEM double-buffered
+// persistent CTA-PAIR kernel (cta_group::2), TMEM double-buffered
 //
-// Why (ncu, profiles/r1_ncu_prof_conv_tc_192_64.txt): v1 re-fetches the whole 9-tap weight slab for every
-// 128/256-pixel tile -- 87 % of its 3.3 GB of L2->SM traffic at 192->192@64 -- and two co-resident CTAs
-// fall into lock-step, so the tensor pipe is active 33 % of the time.  Here
+// Why (ncu, profiles/r1_ncu_prof_conv_tc_192_64.txt): a kernel with one 128/256-pixel tile per CTA re-fetches the
+// whole 9-tap weight slab for every tile -- 87 % of its 3.3 GB of L2->SM traffic at 192->192@64 -- and two
+// co-resident CTAs fall into lock-step, so the tensor pipe is active 33 % of the time.  Here
 //   * two CTAs of a cluster (one TPC) issue M=256 MMAs: each CTA stages its own 128*MT pixel rows (A) but
 //     only HALF of the weight tile (B); the tensor cores of both SMs read both halves -> B traffic / 2;
 //   * one CTA per SM, ~200 KB operand ring (6-8 K-chunks in flight, covers the TMA round trip);
@@ -634,7 +339,7 @@ struct Tc2Params {
     int S;                        // ring depth
     int a_chunk_bytes, b_chunk_bytes, stage_bytes;
     int pix_tiles, items;
-    int has_res, accum, sub, exp;
+    int has_res, accum, sub;
     int vec_bias, vec_tbias;      // 16-byte aligned -> float4 loads in the epilogue
     int v256;                     // out (and res) rows are 32-byte aligned -> 256-bit loads / stores
     int b_res;                    // 1: this CTA's half of the weight tile (all K-chunks, all taps) stays resident in shared
@@ -732,11 +437,10 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
                     const bool second = FUSED2 && st >= NST - KCH2;               // a chunk of the fused 1x1 operand
                     const int kc0 = second ? st - (NST - KCH2) : st * p.KS, nk = second ? 1 : min(p.KS, KCH - kc0);
                     const uint32_t fbar = mapa_u32(smem_u32(&full[s]), 0);
-                    const bool skipA = (p.exp & 1) && g >= (uint32_t)p.S, skipB = (p.exp & 2) && g >= (uint32_t)p.S;   // diagnostics
-                    const bool loadB = !skipB && !(p.b_res && it != pair);       // resident weights arrive with the first item only
+                    const bool loadB = !(p.b_res && it != pair);                 // resident weights arrive with the first item only
                     const int bbytes = second ? p.b2_chunk_bytes : p.b_chunk_bytes;
                     // GNA: the patch lands on this CTA's own afull[s] (the transform warps wait there); full[s] counts weights only
-                    const uint32_t tx = (uint32_t)(2 * nk * ((skipA || GNA ? 0 : p.P * 32) + (loadB ? bbytes : 0)));
+                    const uint32_t tx = (uint32_t)(2 * nk * ((GNA ? 0 : p.P * 32) + (loadB ? bbytes : 0)));
                     if (leader) { if (tx) mbar_expect_tx(&full[s], tx); else mbar_arrive(&full[s]); }
                     if (GNA) mbar_expect_tx(&afull[s], (uint32_t)(nk * p.P * 32));
                     uint8_t* sbase = ring + (size_t)s * p.stage_bytes;
@@ -751,7 +455,7 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
                         if (GNA) {
                             for (int r = 0; r < p.P; r += p.seg) tma_load_2d(adst + (size_t)r * 32, mA, &afull[s], (kc0 + k) * KC, row0 + r);
                         } else {
-                            for (int r = 0; r < p.P && !skipA; r += p.seg)
+                            for (int r = 0; r < p.P; r += p.seg)
                                 tma2_load_2d(adst + (size_t)r * 32, mA, fbar, (kc0 + k) * KC, row0 + r);
                         }
                         if (loadB) tma2_load_3d(bdst, mB, fbar, (kc0 + k) * KC, nrow0, 0);
@@ -891,7 +595,7 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
             for (int st = 0; st < NST; ++st, ++g) {
                 const uint32_t s = g % (uint32_t)p.S; const uint32_t ph = (g / (uint32_t)p.S) & 1;
                 mbar_wait(&afull[s], ph);
-                if (!(FUSED2 && st >= NST - KCH2) && !(p.exp & 4096)) {      // exp bit 12: skip the transform (timing diagnostic)
+                if (!(FUSED2 && st >= NST - KCH2)) {
                     const int kc0 = st * p.KS, nk = min(p.KS, KCH - kc0);
                     for (int k = 0; k < nk; ++k) {
                         const uint32_t abase = ring_u + s * (uint32_t)p.stage_bytes + (uint32_t)k * chunk_stride;
@@ -939,8 +643,8 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
                     if (p.up) { y = 2 * y + p.py; x = 2 * x + p.px; }
                 }
                 orow_a[mt] = valid ? p.out.at<bf16>(n, y, x, n0) : nullptr;
-                rrow_a[mt] = (valid && p.has_res && !(p.exp & 16)) ? p.res.at<bf16>(n, y, x, n0) : nullptr;   // exp bit 4: timing-only
-                tb_a[mt] = (valid && p.tbias && !(p.exp & 16)) ? p.tbias + (size_t)n * p.tbias_pitch + n0 : nullptr;
+                rrow_a[mt] = (valid && p.has_res) ? p.res.at<bf16>(n, y, x, n0) : nullptr;
+                tb_a[mt] = (valid && p.tbias) ? p.tbias + (size_t)n * p.tbias_pitch + n0 : nullptr;
                 const bf16* pf = rrow_a[mt] ? rrow_a[mt] : ((p.accum && valid) ? orow_a[mt] : nullptr);
                 if (pf) {
                     for (int c = blk_lo << 4; c < (blk_hi << 4); c += 64)
@@ -951,7 +655,7 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
             tc_fence_after();
             const uint32_t dbase = tmem_base + buf * (uint32_t)cols_per_buf;
 #pragma unroll
-            for (int mt = 0; mt < ((p.exp & 4) ? 0 : MT); ++mt) {      // exp bit 2: skip the epilogue (diagnostic)
+            for (int mt = 0; mt < MT; ++mt) {
                 bf16* orow = orow_a[mt]; const bf16* rrow = rrow_a[mt]; const float* tb = tb_a[mt];
                 const bool valid = orow != nullptr;
                 // (staging the tile in shared memory to emit full 128-byte lines per store instruction was measured
@@ -972,7 +676,7 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
                                 if (p.v256) { U8 t; ldg256(rrow + c, t); rr[q][0] = t.lo; rr[q][1] = t.hi; }
                                 else { rr[q][0] = *reinterpret_cast<const uint4*>(rrow + c); rr[q][1] = *reinterpret_cast<const uint4*>(rrow + c + 8); }
                             }
-                            if (p.accum && valid && !(p.exp & 16)) {
+                            if (p.accum && valid) {
                                 if (p.v256) { U8 t; ldg256(orow + c, t); ra[q][0] = t.lo; ra[q][1] = t.hi; }
                                 else { ra[q][0] = *reinterpret_cast<const uint4*>(orow + c); ra[q][1] = *reinterpret_cast<const uint4*>(orow + c + 8); }
                             }
@@ -1014,7 +718,7 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
                                     v[2 * i] += fa.x; v[2 * i + 1] += fa.y; v[8 + 2 * i] += fb.x; v[8 + 2 * i + 1] += fb.y;
                                 }
                             }
-                            if (p.accum && !(p.exp & 16)) {
+                            if (p.accum) {
                                 const __nv_bfloat162* ha = reinterpret_cast<const __nv_bfloat162*>(&ra[q][0]);
                                 const __nv_bfloat162* hb = reinterpret_cast<const __nv_bfloat162*>(&ra[q][1]);
 #pragma unroll
@@ -1031,10 +735,8 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
                                 h0[i] = __floats2bfloat162_rn(v[2 * i], v[2 * i + 1]);
                                 h1[i] = __floats2bfloat162_rn(v[8 + 2 * i], v[8 + 2 * i + 1]);
                             }
-                            if (!(p.exp & 8) || o0.x == 0x12345678u) {        // exp bit 3: no global stores (diagnostic)
-                                if (p.v256) stg256(orow + c, o0, o1);
-                                else { *reinterpret_cast<uint4*>(orow + c) = o0; *reinterpret_cast<uint4*>(orow + c + 8) = o1; }
-                            }
+                            if (p.v256) stg256(orow + c, o0, o1);
+                            else { *reinterpret_cast<uint4*>(orow + c) = o0; *reinterpret_cast<uint4*>(orow + c + 8) = o1; }
                         }
                     }
                 }
@@ -1050,11 +752,8 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
     if (warp == 1) { tc_fence_after(); tmem_dealloc2(tmem_base, 512u); }
 }
 
-static int g_tc_v2 = 1;
-extern "C" int ddpm_set_tc_v2(int on) { g_tc_v2 = on; return 0; }
-int g_tc_v2_flag() { return g_tc_v2; }
-
-static int conv_tc2_launch(const ddpm_conv_args* a, cudaStream_t st) {
+int conv_tc_launch(const ddpm_conv_args* a, cudaStream_t st) {
+    int rc = get_encode(); if (rc) return rc;
     Tc2Params p;
     p.out = TV(a->out);
     p.has_res = a->res.ptr != nullptr; p.res = p.has_res ? TV(a->res) : TV(a->out);
@@ -1063,7 +762,7 @@ static int conv_tc2_launch(const ddpm_conv_args* a, cudaStream_t st) {
     p.Cin = a->in.C; p.Cout = a->out.C; p.NT = pick_nt(p.Cout);
     // Channel tiles of at most 128: with MT = 2 the weight slab is then shared by 256 pixel rows per CTA and the
     // A-patch halo is amortised over two M-tiles -> 26 % less L2->SM traffic per FLOP than NT = 192, MT = 1
-    // (measured +8..14 % on every Cout = 192 layer); bit 5 of the experiment flags restores the wide tile.
+    // (measured +8..14 % on every Cout = 192 layer); ddpm_set_tc_mode flag 32 keeps the wide tile.
     if (!(g_tc_exp & 32) && p.NT % 32 == 0 && p.NT > 128) p.NT /= 2;
     p.n_tiles = p.Cout / p.NT;
     p.taps = a->KH * a->KW;
@@ -1071,7 +770,7 @@ static int conv_tc2_launch(const ddpm_conv_args* a, cudaStream_t st) {
     p.Hp = a->in.H + 2; p.Wp = a->in.W + 2; p.H = a->in.H; p.W = a->in.W;
     p.Qtot = a->in.N * p.Hp * p.Wp;
     p.accum = (a->epi & DDPM_EPI_ACCUM) ? 1 : 0;
-    p.sub = a->stride == 2 ? 1 : 0; p.exp = g_tc_exp;
+    p.sub = a->stride == 2 ? 1 : 0;
     p.vec_bias = a->bias && (((uintptr_t)a->bias & 15) == 0);
     p.vec_tbias = a->tbias && (((uintptr_t)a->tbias & 15) == 0) && (a->tbias_pitch % 4 == 0);
     p.v256 = (((uintptr_t)a->out.ptr & 31) == 0) && (a->out.pitch % 16 == 0) &&
@@ -1197,23 +896,8 @@ struct WgTcParams {
     // D_bias[co][*] = sum_Q dY[Q][co] (halo rows of dY are zero), instead of a separate pass over dY
     float* ws_bias;             // [split][mtile][128] partials (NULL: no bias gradient)
     float* dbias;               // fp32 [CoutV], accumulated by the reduce kernel
-    float* dw;                  // fp32 OIHW gradient; non-NULL: cooperative launch, the split-K partials are reduced
-                                // by the same kernel behind a grid barrier (no second launch)
-    int cl3;                    // 1: the three filter-row CTAs of a (split, ci tile, co tile) form a cluster (1,3,1) and
-                                //    share ONE multicast TMA load of the dY tile (L2->SM traffic of dY / 3)
 };
 
-__device__ __forceinline__ void wgrad_reduce_body(const float* __restrict__ ws, float* __restrict__ dw, int splits, const WgTcParams& p,
-                                                  int gtid, int gthreads);
-// one load, delivered to the same shared-memory offset (and signalling the same barrier offset) in every CTA of `mask`
-__device__ __forceinline__ void tma_load_2d_mc(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, uint16_t mask) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-                 ::"r"(smem_u32(dst)), "l"(m), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask) : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {      // arrives on `bar` in every CTA of `mask`
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(smem_u32(bar)), "h"(mask) : "memory");
-}
 __global__ void __launch_bounds__(TC_THREADS) wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmY,
                                                                const __grid_constant__ CUtensorMap tmA, WgTcParams p) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -1225,11 +909,9 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc_kernel(const __grid_const
     uint32_t* tmem_slot = (uint32_t*)(acc_full + 1);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int split = blockIdx.x, mtile = blockIdx.z;
-    // cluster mode: blockIdx.y = ntile * 3 + ky, so that the cluster (1,3,1) holds the three filter rows of one ci tile
-    const uint32_t crank = p.cl3 ? cluster_ctarank() : 0u;
-    const int ky = p.cl3 ? (int)crank : (int)blockIdx.y / p.n_tiles;
-    const int ntile = p.cl3 ? (int)blockIdx.y / 3 : (int)blockIdx.y - ky * p.n_tiles;
-    const int grp = ky * p.n_tiles + ntile;                     // workspace / bias-dealing index (same in both modes)
+    const int ky = (int)blockIdx.y / p.n_tiles;
+    const int ntile = (int)blockIdx.y - ky * p.n_tiles;
+    const int grp = ky * p.n_tiles + ntile;                     // workspace / bias-dealing index
     // the K-steps of the bias reduction are dealt round-robin to the gridDim.y groups that stream the same dY
     // rows (putting all of them on group 0 made those CTAs the critical path: +11..16 % kernel time)
     const bool do_bias = p.ws_bias != nullptr;
@@ -1243,9 +925,7 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc_kernel(const __grid_const
     if (threadIdx.x == 0) {
         asm volatile("prefetch.tensormap [%0];" ::"l"(&tmY) : "memory");
         asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA) : "memory");
-        // cluster mode: rank 0 multicasts dY into all three CTAs, so ITS empty[s] collects the release of all three
-        // MMA warps (the others' commits arrive remotely); ranks 1, 2 only wait for their own
-        for (int i = 0; i < WG_STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], (p.cl3 && crank == 0) ? 3 : 1); }
+        for (int i = 0; i < WG_STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
         mbar_init(acc_full, 1);
         fence_barrier_init();
     }
@@ -1256,7 +936,6 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc_kernel(const __grid_const
     }
     tc_fence_before();
     __syncthreads();
-    if (p.cl3) cluster_sync_all();                       // peers' barriers are initialised before anyone signals them
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     const uint32_t bias_col = (uint32_t)(p.ntap * p.NT);
@@ -1270,13 +949,8 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc_kernel(const __grid_const
                 uint8_t* dst = smem + (size_t)s * p.stage_bytes;
                 mbar_expect_tx(&full[s], (uint32_t)(y_bytes + p.nblkA * WG_ROWS * 128));
                 const int Q = (s_beg + i) * WG_KQ;
-                if (!p.cl3) {
-                    tma_load_2d(dst, &tmY, &full[s], m0, Q);
-                    tma_load_2d(dst + WG_KQ * 128, &tmY, &full[s], m0 + 64, Q);
-                } else if (crank == 0) {                 // every CTA armed / will arm its own full[s] with the same byte count
-                    tma_load_2d_mc(dst, &tmY, &full[s], m0, Q, (uint16_t)7);
-                    tma_load_2d_mc(dst + WG_KQ * 128, &tmY, &full[s], m0 + 64, Q, (uint16_t)7);
-                }
+                tma_load_2d(dst, &tmY, &full[s], m0, Q);
+                tma_load_2d(dst + WG_KQ * 128, &tmY, &full[s], m0 + 64, Q);
                 const int rowA = p.ntap == 3 ? Q + (ky - 1) * p.Wp - 1 : Q;
                 for (int b = 0; b < p.nblkA; ++b)
                     tma_load_2d(dst + y_bytes + (size_t)b * WG_ROWS * 128, &tmA, &full[s], n0 + 64 * b, rowA);
@@ -1295,10 +969,9 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc_kernel(const __grid_const
             const bool three = p.ntap == 3;
             const uint32_t idesc_b = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) | ((16u >> 3) << 17) | ((128u >> 4) << 24);
             const uint64_t ones_desc = desc_pack(desc_lo(smem_u32(ones), 2048u), hi);
-            const uint16_t relmask = (uint16_t)((1u << crank) | 1u);   // release the stage here and at the multicasting rank 0
             // two copies of the loop: a predicated-off bias MMA in the common loop cost 11 % (measured A/B)
-            auto run = [&](auto with_bias, auto with_three, auto with_cl3) {
-                constexpr bool BIAS = decltype(with_bias)::value, THREE = decltype(with_three)::value, CL3 = decltype(with_cl3)::value;
+            auto run = [&](auto with_bias, auto with_three) {
+                constexpr bool BIAS = decltype(with_bias)::value, THREE = decltype(with_three)::value;
                 uint32_t acc = 0, accb = 0;
                 int kmod = ((s_beg * (WG_KQ / 16)) % ngrp);                 // (global K-step index) mod ngrp
                 for (int i = 0; i < nst; ++i) {
@@ -1320,17 +993,13 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc_kernel(const __grid_const
                         }
                     }
                     acc = 1;
-                    if (el) { if (CL3) umma_commit_mc(&empty[s], relmask); else umma_commit(&empty[s]); }
+                    if (el) umma_commit(&empty[s]);
                     __syncwarp();
                 }
             };
             // every run-time flag of the issue loop is a compile-time constant of its copy (the loop is that sensitive)
-            auto go = [&](auto b) {
-                if (!three) run(b, std::false_type{}, std::false_type{});
-                else if (p.cl3) run(b, std::true_type{}, std::true_type{});
-                else run(b, std::true_type{}, std::false_type{});
-            };
-            if (do_bias) go(std::true_type{}); else go(std::false_type{});
+            if (do_bias) { if (three) run(std::true_type{}, std::true_type{}); else run(std::true_type{}, std::false_type{}); }
+            else { if (three) run(std::false_type{}, std::true_type{}); else run(std::false_type{}, std::false_type{}); }
             if (el) umma_commit(acc_full);
             __syncwarp();
         }
@@ -1366,15 +1035,7 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc_kernel(const __grid_const
         tc_fence_before();
     }
     __syncthreads();
-    if (p.cl3) cluster_sync_all();                       // nobody exits while peers may still signal its barriers
     if (warp == 1) { tc_fence_after(); tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols); }
-    if (p.dw) {
-        // split-K reduction in the same (cooperative) launch: every CTA's partial tile is in the workspace after the
-        // grid barrier; all threads of the grid then sum disjoint slices of the gradient
-        cooperative_groups::this_grid().sync();
-        const int bid = (blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x;
-        wgrad_reduce_body(p.ws, p.dw, gridDim.x, p, bid * TC_THREADS + threadIdx.x, gridDim.x * gridDim.y * gridDim.z * TC_THREADS);
-    }
 }
 
 // ================================================================================================
@@ -1536,8 +1197,9 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc2_kernel(const __grid_cons
 }
 
 // dw[co][ci][ky][kx] += sum_split ws[split][mtile][ky*n_tiles+ntile][co%128][kx*NT + ci%NT]
-__device__ __forceinline__ void wgrad_reduce_body(const float* __restrict__ ws, float* __restrict__ dw, int splits, const WgTcParams& p,
-                                                  int gtid, int gthreads) {
+__global__ void wgrad_reduce_kernel(const float* __restrict__ ws, float* __restrict__ dw, int splits, WgTcParams p) {
+    pdl_enter();
+    const int gtid = blockIdx.x * blockDim.x + threadIdx.x, gthreads = gridDim.x * blockDim.x;
     const int taps = p.ntap * p.ntap;
     const int total = p.CoutV * taps * p.CinV;
     const int grps = p.ntap * p.n_tiles, cols = p.ntap * p.NT;
@@ -1570,10 +1232,6 @@ __device__ __forceinline__ void wgrad_reduce_body(const float* __restrict__ ws, 
         }
     }
 }
-__global__ void wgrad_reduce_kernel(const float* __restrict__ ws, float* __restrict__ dw, int splits, WgTcParams p) {
-    pdl_enter();
-    wgrad_reduce_body(ws, dw, splits, p, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
-}
 
 static int sm_count() {
     static int n = 0;
@@ -1589,45 +1247,17 @@ static int wg_pick_nt(int Cin) {
     return 0;
 }
 
-static size_t wg_smem_bytes(const WgTcParams& p) { return (size_t)WG_STAGES * p.stage_bytes + 2048 + 8 * (2 * WG_STAGES + 1) + 16 + 1024; }
-static int wg_set_smem(size_t smem) {
-    static size_t configured = 0;
-    if (smem > configured) {
-        CUDA_TRY(cudaFuncSetAttribute(wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured = smem;
-    }
-    return 0;
-}
-// how many (1,3,1) clusters of 178 KB CTAs the device holds at once (GPCs whose SM count is not a multiple of 3 leave
-// SMs idle: 48 clusters = 144 of 148 SMs on B200); a grid larger than that would run a second, nearly empty wave
-static int wg_max_clusters(size_t smem) {
-    static size_t key[4] = {0, 0, 0, 0}; static int val[4] = {0, 0, 0, 0};
-    for (int i = 0; i < 4; ++i) if (key[i] == smem) return val[i];
-    int n = 0;
-    if (wg_set_smem(smem) == 0) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(1, 3, 1); cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = smem;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = 1; at[0].val.clusterDim.y = 3; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        if (cudaOccupancyMaxActiveClusters(&n, wgrad_tc_kernel, &cfg) != cudaSuccess) { n = 0; cudaGetLastError(); }
-    }
-    for (int i = 0; i < 4; ++i) if (key[i] == 0) { key[i] = smem; val[i] = n; break; }
-    return n;
-}
-
 static int wg_pair(const WgTcParams& p) {
-    // the pair kernel: an even number of 128-row output-channel tiles (Cout in (128,256], (384,512], ...); bit 10 of the
-    // experiment flags turns it off (A/B against the single-CTA kernel).  It is never given the programmatic-dependent-launch
+    // the pair kernel: an even number of 128-row output-channel tiles (Cout in (128,256], (384,512], ...); ddpm_set_tc_mode
+    // flag 1024 turns it off (A/B against the single-CTA kernel).  It is never given the programmatic-dependent-launch
     // attribute: launched that way on the MAIN stream it dead-locked the GPU in 4 of 10 CelebA256 bench runs (0 of 6 without
-    // the attribute, 0 of 4 with the single-CTA kernel; mechanism not found -- DESIGN.md section 4.4).
+    // the attribute, 0 of 4 with the single-CTA kernel; mechanism not found -- DESIGN.md section 6.2).
     if (g_tc_exp & 1024) return 0;
     // Measured (profiles/r2_kbench_wgrad_pair_vs_single.txt): -9 % on the large Cout = 192 layers, +5 % on 384->192 @ 16 / 8
     // (four ci tiles x few pixels: the halved split count costs more than the smaller patch saves) -> small problems with
     // many ci tiles stay on the single-CTA kernel.
     if (p.n_tiles > 2 && p.stages_total < 1500) return 0;
-    return (p.m_tiles % 2 == 0) && !p.cl3 && p.NT % 16 == 0;
+    return (p.m_tiles % 2 == 0) && p.NT % 16 == 0;
 }
 static void wg_plan(const ddpm_wgrad_args* a, WgTcParams* p, int* splits) {
     p->Cin = a->act.C; p->Cout = a->dy.C; p->NT = wg_pick_nt(p->Cin);
@@ -1643,15 +1273,6 @@ static void wg_plan(const ddpm_wgrad_args* a, WgTcParams* p, int* splits) {
     // one CTA per SM (176 KB of shared memory): the grid must not exceed ONE wave, or the second,
     // nearly empty wave doubles the kernel's duration -> floor, not ceil
     int sp = sm_count() / yz;
-    p->cl3 = 0;
-    // Measured: no gain (2.84 vs 2.72 ms of wgrad per step without PDL, and clusters of 178 KB CTAs interact badly with
-    // programmatic dependent launch: 3.65 ms) -- the kernel is bound by the tensor core's SHARED-MEMORY operand reads
-    // (M=128, N=96, K=16: 4 KB + 3 KB per 48-cycle MMA = 146 B/clk against 128 B/clk), not by L2->SM traffic.  Opt-in
-    // through bit 9 of the experiment flags.
-    if (p->ntap == 3 && (g_tc_exp & 512)) {
-        const int mc = wg_max_clusters(wg_smem_bytes(*p));
-        if (mc >= p->n_tiles * p->m_tiles) { p->cl3 = 1; sp = mc / (p->n_tiles * p->m_tiles); }
-    }
     int max_sp = (p->stages_total + 7) / 8; if (max_sp < 1) max_sp = 1;
     if (sp > max_sp) sp = max_sp;
     if (sp < 1) sp = 1;
@@ -1698,7 +1319,6 @@ int wgrad_tc_launch(const ddpm_wgrad_args* a, cudaStream_t st) {
         uint32_t b[2] = {64, WG_ROWS};
         if (encode(&tmA, a->act.ptr, 2, d, s, b, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
     }
-    dim3 grid(splits, p.ntap * p.n_tiles, p.m_tiles);
     if (wg_pair(p)) {
         const size_t smem2 = (size_t)WG2_STAGES * p.stage_bytes + 2048 + 8 * (2 * WG2_STAGES + 1) + 16 + 1024;
         static size_t configured2 = 0;
@@ -1706,49 +1326,21 @@ int wgrad_tc_launch(const ddpm_wgrad_args* a, cudaStream_t st) {
             CUDA_TRY(cudaFuncSetAttribute(wgrad_tc2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
             configured2 = smem2;
         }
-        p.dw = nullptr;
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3(p.m_tiles, p.ntap * p.n_tiles, splits); cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = smem2; cfg.stream = st;
-        cudaLaunchAttribute at[2]; unsigned nat = 1;
+        cudaLaunchAttribute at[1];                    // no PDL attribute: see wg_pair()
         at[0].id = cudaLaunchAttributeClusterDimension;
         at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        if (g_tc_exp & 2048) pdl_attr(at, &nat);      // experiments only (bit 11): see wg_pair()
-        cfg.attrs = at; cfg.numAttrs = nat;
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, wgrad_tc2_kernel, tmY, tmA, p));
-        LAUNCH_OK();
-        int total = p.CoutV * p.ntap * p.ntap * p.CinV;
-        int rg = (total + 255) / 256; if (rg > 148 * 8) rg = 148 * 8;
-        CUDA_TRY(launch_pdl(wgrad_reduce_kernel, dim3(rg), dim3(256), 0, st, (const float*)p.ws, a->dw, splits, p));
-        LAUNCH_OK();
-        return 0;
-    }
-    size_t smem = wg_smem_bytes(p);
-    rc = wg_set_smem(smem); if (rc) return rc;
-    // In-kernel split-K reduction behind a cooperative grid barrier: measured SLOWER on B200 (a cooperative launch costs
-    // ~50 us: 96->96@64 100 -> 153 us), so it stays an experiment (bit 8 of the flags); default = separate reduce kernel.
-    const bool fused = (g_tc_exp & 256) && !p.cl3 && (int)(grid.x * grid.y * grid.z) <= sm_count();
-    p.dw = fused ? a->dw : nullptr;
-    if (fused) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = grid; cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeCooperative; at[0].val.cooperative = 1;
         cfg.attrs = at; cfg.numAttrs = 1;
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, wgrad_tc_kernel, tmY, tmA, p));
-        LAUNCH_OK();
-        return 0;
-    }
-    if (p.cl3) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = grid; cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-        cudaLaunchAttribute at[2]; unsigned nat = 1;
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = 1; at[0].val.clusterDim.y = 3; at[0].val.clusterDim.z = 1;
-        pdl_attr(at, &nat);
-        cfg.attrs = at; cfg.numAttrs = nat;
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, wgrad_tc_kernel, tmY, tmA, p));
+        CUDA_TRY(cudaLaunchKernelEx(&cfg, wgrad_tc2_kernel, tmY, tmA, p));
     } else {
-        CUDA_TRY(launch_pdl(wgrad_tc_kernel, grid, dim3(TC_THREADS), smem, st, tmY, tmA, p));
+        const size_t smem = (size_t)WG_STAGES * p.stage_bytes + 2048 + 8 * (2 * WG_STAGES + 1) + 16 + 1024;
+        static size_t configured = 0;
+        if (smem > configured) {
+            CUDA_TRY(cudaFuncSetAttribute(wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            configured = smem;
+        }
+        CUDA_TRY(launch_pdl(wgrad_tc_kernel, dim3(splits, p.ntap * p.n_tiles, p.m_tiles), dim3(TC_THREADS), smem, st, tmY, tmA, p));
     }
     LAUNCH_OK();
     int total = p.CoutV * p.ntap * p.ntap * p.CinV;

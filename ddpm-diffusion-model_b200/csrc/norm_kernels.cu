@@ -8,11 +8,9 @@
 // vector position `cv` and walks pixels, so global accesses are 16 B per lane and contiguous along C.
 //
 // HBM roofline (bf16 activations): gn_stats 2 B/elem, gn_apply 4 B/elem, gn_bwd 2x(4)+2 = 10 B/elem.
-#include <stdlib.h>
 #include "common.cuh"
 
 #include <cooperative_groups.h>
-#include <cuda.h>
 #include <unordered_map>
 namespace cg = cooperative_groups;
 
@@ -499,504 +497,19 @@ __global__ void __launch_bounds__(NT, STASH ? GN_BWD_OCC : 2) gn_bwd_kernel(GnP 
     }
 }
 
-// ================================================================================================
-// "Slab" variants (bf16): TMA in, shared memory, TMA out -- every tensor crosses HBM exactly once and the
-// streaming kernels' per-packet address arithmetic disappears.
-//
-// What the measurements said about the streaming kernels above (round 2): cutting their DRAM traffic alone does not
-// help (a cp.async version that kept the share in shared memory ran at the same speed), and shaving their address
-// arithmetic alone does not help either -- they are bound by the instructions + latency of moving 16-byte packets
-// with one LDGSTS / LDS / STG per packet per thread (~30 instructions per element forward, ~41 backward).  Here a
-// cluster of CS CTAs owns an image and each CTA
-//   * receives its rows of the image (forward: x; backward: x and dy) with a handful of bulk tensor copies
-//     (cp.async.bulk.tensor.4d over the (c, x, y, n) view of the halo'd NHWC buffer -- the halo columns are simply
-//     not part of the box), in up to four row groups, each signalling its own mbarrier,
-//   * reduces the moments from shared memory as the row groups land (LDS.128 + FP only), exchanges them through
-//     distributed shared memory,
-//   * transforms the rows IN PLACE in shared memory and hands every finished row group to a bulk tensor STORE
-//     (cp.async.bulk.tensor ... bulk_group) while the next group is being computed.  The backward's
-//     `dx += ...` is the same store as a bulk REDUCE-ADD (cp.reduce.async.bulk.tensor .add, bf16), so the old dx is
-//     never read by the SM.
-// Per packet of 8 elements that is LDS + unpack + math + pack + STS: ~8 instructions per element forward.
-// A thread reads only the packets it transforms itself (same (cv, pixel lane) mapping in every phase); barriers are
-// needed only between "all threads finished a row group" and its store.
-// ================================================================================================
-extern int ddpm_encode_tiled_bf16(CUtensorMap* m, void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-                                  const uint32_t* box, int swizzle_bytes);      // conv_tc.cu
-__device__ __forceinline__ void unpack_bf16x8(const uint4& q, float* v) {
-    v[0] = __uint_as_float(q.x << 16); v[1] = __uint_as_float(q.x & 0xffff0000u);
-    v[2] = __uint_as_float(q.y << 16); v[3] = __uint_as_float(q.y & 0xffff0000u);
-    v[4] = __uint_as_float(q.z << 16); v[5] = __uint_as_float(q.z & 0xffff0000u);
-    v[6] = __uint_as_float(q.w << 16); v[7] = __uint_as_float(q.w & 0xffff0000u);
-}
-__device__ __forceinline__ uint4 pack_bf16x8(const float* v) {
-    uint4 t;
-    __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(&t);
-#pragma unroll
-    for (int i = 0; i < 4; ++i) h[i] = __floats2bfloat162_rn(v[2 * i], v[2 * i + 1]);
-    return t;
-}
-__device__ __forceinline__ void sts128(uint32_t a, const uint4& v) {
-    asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(a), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-__device__ __forceinline__ void sl_mbar_init(uint32_t bar, uint32_t count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count)); }
-__device__ __forceinline__ void sl_mbar_expect(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void sl_mbar_wait(uint32_t bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "SLW_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra SLD_%=;\n\t"
-        "bra SLW_%=;\n\t"
-        "SLD_%=:\n\t}" ::"r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void sl_tma_load4(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c, int x, int y, int n) {
-    asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-                 ::"r"(dst), "l"(m), "r"(bar), "r"(c), "r"(x), "r"(y), "r"(n) : "memory");
-}
-__device__ __forceinline__ void sl_tma_store4(const CUtensorMap* m, uint32_t src, int c, int x, int y, int n) {
-    asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
-                 ::"l"(m), "r"(src), "r"(c), "r"(x), "r"(y), "r"(n) : "memory");
-}
-__device__ __forceinline__ void sl_tma_add4(const CUtensorMap* m, uint32_t src, int c, int x, int y, int n) {
-    asm volatile("cp.reduce.async.bulk.tensor.4d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
-                 ::"l"(m), "r"(src), "r"(c), "r"(x), "r"(y), "r"(n) : "memory");
-}
-__device__ __forceinline__ void sl_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void sl_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void sl_fence_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-#define SL_MAXQ 4
-struct SlabP {
-    int rows;                   // image rows per CTA (H / CS)
-    int nq;                     // row groups (<= SL_MAXQ); group k = rows [rows*k/nq, rows*(k+1)/nq)
-    int nbox, cb;               // channel boxes per tensor and channels per box (TMA boxes are <= 256 wide)
-    int slab_bytes;             // one tensor's share: rows * W * C * 2
-};
-// Per-thread view: this thread owns channel vector `cv` (8 channels) of pixel lane `prow`; pixels of a row group
-// [g0, g1) (local pixel indices) are visited as p = g0 + prow, + ppi, ...  The shared-memory layout is what the TMA
-// boxes produce: [channel box][local pixel][cb channels].
-struct SlabMap {
-    int ppi, W, rows; uint32_t sthread, spix; bool active;
-    __device__ __forceinline__ SlabMap(const PixMap& m, const SlabP& sp, int W_, uint32_t slab_addr) {
-        const int cvb = sp.cb / 8, box = m.cv / cvb, cvi = m.cv - box * cvb;
-        ppi = m.ppi; W = W_; rows = sp.rows; active = m.active;
-        spix = (uint32_t)(sp.cb * 2);                                  // bytes per pixel inside a box
-        sthread = slab_addr + (uint32_t)box * (uint32_t)(sp.rows * W_) * spix + (uint32_t)(cvi * 16) + (uint32_t)m.prow * spix;
-    }
-    __device__ __forceinline__ uint32_t addr(int p_minus_prow) const { return sthread + (uint32_t)p_minus_prow * spix; }
-};
-// one thread: loads of row group k of `tm` into the slab at `slab_addr`
-__device__ __forceinline__ void slab_issue_loads(const CUtensorMap* tm, uint32_t slab_addr, uint32_t bar, const SlabP& sp, int W, int k,
-                                                 int row0, int n, bool arm, uint32_t arm_bytes) {
-    const int r0 = (sp.rows * k) / sp.nq, r1 = (sp.rows * (k + 1)) / sp.nq;
-    if (arm) sl_mbar_expect(bar, arm_bytes);
-    for (int b = 0; b < sp.nbox; ++b)
-        sl_tma_load4(slab_addr + (uint32_t)(b * sp.rows * W + r0 * W) * (uint32_t)(sp.cb * 2), tm, bar, b * sp.cb, 0, row0 + r0, n);
-    (void)r1;
-}
-
-__global__ void __launch_bounds__(NT, 2) gn_fwd_slab_kernel(const __grid_constant__ CUtensorMap tmX0, const __grid_constant__ CUtensorMap tmX1,
-                                                             const __grid_constant__ CUtensorMap tmX2, const __grid_constant__ CUtensorMap tmX3,
-                                                             const __grid_constant__ CUtensorMap tmO0, const __grid_constant__ CUtensorMap tmO1,
-                                                             const __grid_constant__ CUtensorMap tmO2, const __grid_constant__ CUtensorMap tmO3,
-                                                             GnP a, SlabP sp) {
-    constexpr int VEC = 8;
-    extern __shared__ __align__(128) unsigned char gsm_raw[];
-    unsigned char* gsm = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(gsm_raw) + 127) & ~(uintptr_t)127);
-    const int C = a.x.C, G = a.G, cpg = C / G, W = a.x.W, HW = a.x.H * W;
-    cg::cluster_group cl = cg::this_cluster();
-    const int CS = (int)cl.num_blocks(), rank = (int)cl.block_rank();
-    const int n = blockIdx.x / CS;
-    const PixMap m = make_map<VEC>(C);
-    float (*part)[NT] = reinterpret_cast<float (*)[NT]>(gsm + sp.slab_bytes);           // [VEC][NT]
-    double* chan = reinterpret_cast<double*>(gsm + sp.slab_bytes + VEC * NT * 4);       // [2][C]
-    double* gpart = chan + 2 * C;                                                       // [2][G]  (read by the cluster)
-    float* gm = reinterpret_cast<float*>(gpart + 2 * G);
-    float* gr = gm + G;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(gr + G);                               // [SL_MAXQ]  (2*G floats after an 8-byte aligned base)
-    const uint32_t slab = sm_u32(gsm), bar0 = sm_u32(bars);
-    const int row0 = rank * sp.rows;                                                    // first image row of this CTA
-    const int c0 = m.cv * VEC;
-    const CUtensorMap* tmX[SL_MAXQ] = {&tmX0, &tmX1, &tmX2, &tmX3};
-    const CUtensorMap* tmO[SL_MAXQ] = {&tmO0, &tmO1, &tmO2, &tmO3};
-
-    if (threadIdx.x == 0) {
-        for (int k = 0; k < sp.nq; ++k) sl_mbar_init(bar0 + 8 * k, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    pdl_enter();                                         // everything above overlapped the previous kernel's tail
-    if (threadIdx.x == 0) {
-        for (int k = 0; k < sp.nq; ++k) {
-            const int r0 = (sp.rows * k) / sp.nq, r1 = (sp.rows * (k + 1)) / sp.nq;
-            slab_issue_loads(tmX[k], slab, bar0 + 8 * k, sp, W, k, row0, n, true, (uint32_t)((r1 - r0) * W * C * 2));
-        }
-    }
-    const uint32_t dkey = a.thr16 ? dropout_key(a.rng, a.layer) : 0u;
-    const uint32_t ebase = (uint32_t)n * (uint32_t)HW * (uint32_t)C + (uint32_t)c0 + (uint32_t)(row0 * W) * (uint32_t)C;
-    const SlabMap sm(m, sp, W, slab);
-
-    float acc[2 * VEC];
-#pragma unroll
-    for (int i = 0; i < 2 * VEC; ++i) acc[i] = 0.f;
-    for (int k = 0; k < sp.nq; ++k) {
-        const int g0 = ((sp.rows * k) / sp.nq) * W, g1 = ((sp.rows * (k + 1)) / sp.nq) * W;
-        sl_mbar_wait(bar0 + 8 * k, 0);
-        if (m.active) {
-#pragma unroll 2
-            for (int p = g0; p + m.prow < g1; p += m.ppi) {
-                float v[VEC];
-                unpack_bf16x8(lds128(sm.addr(p)), v);
-#pragma unroll
-                for (int i = 0; i < VEC; ++i) { acc[i] += v[i]; acc[VEC + i] = fmaf(v[i], v[i], acc[VEC + i]); }
-            }
-        }
-    }
-    cta_channel_reduce<VEC, 1>(part, acc, chan, C, m);
-    cta_channel_reduce<VEC, 1>(part, acc + VEC, chan + C, C, m);
-    for (int o = threadIdx.x; o < 2 * G; o += NT) {
-        const int st = o / G, g = o - st * G;
-        double s = 0.0;
-        for (int j = 0; j < cpg; ++j) s += chan[st * C + g * cpg + j];
-        gpart[o] = s;
-    }
-    cluster_arrive(); cluster_wait();                    // every CTA's gpart is complete
-    for (int g = threadIdx.x; g < G; g += NT) {
-        double s = 0.0, q = 0.0;
-        for (int r = 0; r < CS; ++r) {
-            const double* rp = cl.map_shared_rank(gpart, r);
-            s += rp[g]; q += rp[G + g];
-        }
-        if (rank == 0) { a.stats[((size_t)n * G + g) * 2] = s; a.stats[((size_t)n * G + g) * 2 + 1] = q; }
-        const double cnt = (double)cpg * HW, mu = s / cnt;
-        double var = q / cnt - mu * mu; if (var < 0.0) var = 0.0;
-        gm[g] = (float)mu; gr[g] = (float)(1.0 / sqrt(var + (double)a.eps));
-    }
-    cluster_arrive();                                    // remote reads done; waited for before exit
-    __syncthreads();
-
-    float sc[VEC], sh[VEC];
-#pragma unroll
-    for (int i = 0; i < VEC; ++i) {
-        const int c = min(c0 + i, C - 1), g = c / cpg;
-        sc[i] = gr[g] * __ldg(a.gamma + c);
-        sh[i] = __ldg(a.beta + c) - gm[g] * sc[i];
-        if (a.act) { sc[i] *= 0.5f; sh[i] *= 0.5f; }                // the affine produces z/2 directly (silu_half)
-    }
-    for (int k = 0; k < sp.nq; ++k) {
-        const int g0 = ((sp.rows * k) / sp.nq) * W, g1 = ((sp.rows * (k + 1)) / sp.nq) * W;
-        if (m.active) {
-#pragma unroll 2
-            for (int p = g0; p + m.prow < g1; p += m.ppi) {
-                const uint32_t sa = sm.addr(p);
-                float v[VEC];
-                unpack_bf16x8(lds128(sa), v);
-#pragma unroll
-                for (int i = 0; i < VEC; ++i) {
-                    const float z = fmaf(v[i], sc[i], sh[i]);
-                    v[i] = a.act ? silu_half(z) : z;
-                }
-                if (a.thr16) dropout_apply<VEC>(v, dkey, ebase + (uint32_t)(p + m.prow) * (uint32_t)C, a.thr16, a.keep_scale);
-                sts128(sa, pack_bf16x8(v));
-            }
-        }
-        sl_fence_async();                                // my generic-proxy writes -> visible to the bulk store
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            const int r0 = (sp.rows * k) / sp.nq;
-            for (int b = 0; b < sp.nbox; ++b)
-                sl_tma_store4(tmO[k], slab + (uint32_t)(b * sp.rows * W + r0 * W) * (uint32_t)(sp.cb * 2), b * sp.cb, 0, row0 + r0, n);
-            sl_store_commit();
-        }
-    }
-    if (threadIdx.x == 0) sl_store_wait_read();          // shared memory must outlive the bulk stores' reads
-    cluster_wait();                                      // do not exit while peers may still read gpart
-}
-
-template <int OCC>
-__global__ void __launch_bounds__(NT, OCC) gn_bwd_slab_kernel(const __grid_constant__ CUtensorMap tmX0, const __grid_constant__ CUtensorMap tmX1,
-                                                               const __grid_constant__ CUtensorMap tmX2, const __grid_constant__ CUtensorMap tmX3,
-                                                               const __grid_constant__ CUtensorMap tmD0, const __grid_constant__ CUtensorMap tmD1,
-                                                               const __grid_constant__ CUtensorMap tmD2, const __grid_constant__ CUtensorMap tmD3,
-                                                               const __grid_constant__ CUtensorMap tmO0, const __grid_constant__ CUtensorMap tmO1,
-                                                               const __grid_constant__ CUtensorMap tmO2, const __grid_constant__ CUtensorMap tmO3,
-                                                               GnP a, SlabP sp) {
-    constexpr int VEC = 8;
-    extern __shared__ __align__(128) unsigned char gsm_raw[];
-    unsigned char* gsm = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(gsm_raw) + 127) & ~(uintptr_t)127);
-    const int C = a.x.C, G = a.G, cpg = C / G, W = a.x.W, HW = a.x.H * W;
-    cg::cluster_group cl = cg::this_cluster();
-    const int CS = (int)cl.num_blocks(), rank = (int)cl.block_rank();
-    const int n = blockIdx.x / CS;
-    const PixMap m = make_map<VEC>(C);
-    float (*part)[NT] = reinterpret_cast<float (*)[NT]>(gsm + 2 * sp.slab_bytes);        // [VEC][NT]
-    double* chan = reinterpret_cast<double*>(gsm + 2 * sp.slab_bytes + VEC * NT * 4);    // [2][C] (read by the cluster)
-    float* tot = reinterpret_cast<float*>(chan + 2 * C);                                 // [2][C] cluster totals
-    float* gA = tot + 2 * C;
-    float* gB = gA + G;
-    float* gm = gB + G;
-    float* gr = gm + G;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(gr + G);                                // [SL_MAXQ]  (offset is a multiple of 8)
-    const uint32_t slab = sm_u32(gsm), dslab = slab + (uint32_t)sp.slab_bytes, bar0 = sm_u32(bars);
-    const int row0 = rank * sp.rows;
-    const int c0 = m.cv * VEC;
-    const CUtensorMap* tmX[SL_MAXQ] = {&tmX0, &tmX1, &tmX2, &tmX3};
-    const CUtensorMap* tmD[SL_MAXQ] = {&tmD0, &tmD1, &tmD2, &tmD3};
-    const CUtensorMap* tmO[SL_MAXQ] = {&tmO0, &tmO1, &tmO2, &tmO3};
-
-    if (threadIdx.x == 0) {
-        for (int k = 0; k < sp.nq; ++k) sl_mbar_init(bar0 + 8 * k, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    pdl_enter();
-    if (threadIdx.x == 0) {
-        for (int k = 0; k < sp.nq; ++k) {
-            const int r0 = (sp.rows * k) / sp.nq, r1 = (sp.rows * (k + 1)) / sp.nq;
-            slab_issue_loads(tmX[k], slab, bar0 + 8 * k, sp, W, k, row0, n, true, (uint32_t)(2 * (r1 - r0) * W * C * 2));
-            slab_issue_loads(tmD[k], dslab, bar0 + 8 * k, sp, W, k, row0, n, false, 0u);
-        }
-    }
-    for (int g = threadIdx.x; g < G; g += NT) {
-        const double s = a.stats[((size_t)n * G + g) * 2], q = a.stats[((size_t)n * G + g) * 2 + 1];
-        const double cnt = (double)cpg * HW, mu = s / cnt;
-        double var = q / cnt - mu * mu; if (var < 0.0) var = 0.0;
-        gm[g] = (float)mu; gr[g] = (float)(1.0 / sqrt(var + (double)a.eps));
-    }
-    __syncthreads();
-    const uint32_t dkey = a.thr16 ? dropout_key(a.rng, a.layer) : 0u;
-    const uint32_t ebase = (uint32_t)n * (uint32_t)HW * (uint32_t)C + (uint32_t)c0 + (uint32_t)(row0 * W) * (uint32_t)C;
-    const SlabMap sm(m, sp, W, slab);
-    const uint32_t doff = (uint32_t)sp.slab_bytes;
-
-    // ---- phase 1: dz = dy * mask/(1-p) * act'(z) (left in the dy half of the slab), S1 = sum dz, Sx = sum dz*x per channel
-    {
-        float sc[VEC], sh[VEC];
-#pragma unroll
-        for (int i = 0; i < VEC; ++i) {
-            const int c = min(c0 + i, C - 1), g = c / cpg;
-            const float s_ = gr[g] * __ldg(a.gamma + c);
-            sc[i] = 0.5f * s_; sh[i] = 0.5f * (__ldg(a.beta + c) - gm[g] * s_);
-        }
-        const bool fold = a.act && a.thr16;                  // dropout's 1/(1-p) rides on the constants of the SiLU derivative
-        const float hs = fold ? 0.5f * a.keep_scale : 0.5f, dscale = fold ? 1.0f : a.keep_scale;
-        float acc[2 * VEC];
-#pragma unroll
-        for (int i = 0; i < 2 * VEC; ++i) acc[i] = 0.f;
-        for (int k = 0; k < sp.nq; ++k) {
-            const int g0 = ((sp.rows * k) / sp.nq) * W, g1 = ((sp.rows * (k + 1)) / sp.nq) * W;
-            sl_mbar_wait(bar0 + 8 * k, 0);
-            if (m.active) {
-                for (int p = g0; p + m.prow < g1; p += m.ppi) {
-                    const uint32_t sa = sm.addr(p);
-                    float v[VEC], d[VEC];
-                    unpack_bf16x8(lds128(sa), v);
-                    unpack_bf16x8(lds128(sa + doff), d);
-                    if (a.thr16) dropout_apply<VEC>(d, dkey, ebase + (uint32_t)(p + m.prow) * (uint32_t)C, a.thr16, dscale);
-#pragma unroll
-                    for (int i = 0; i < VEC; ++i) {
-                        float dz = d[i];
-                        if (a.act) dz *= dsilu_half_scaled(fmaf(v[i], sc[i], sh[i]), hs);
-                        acc[i] += dz; acc[VEC + i] = fmaf(dz, v[i], acc[VEC + i]);
-                        d[i] = dz;
-                    }
-                    sts128(sa + doff, pack_bf16x8(d));
-                }
-            }
-        }
-        cta_channel_reduce<VEC, 1>(part, acc, chan, C, m);
-        cta_channel_reduce<VEC, 1>(part, acc + VEC, chan + C, C, m);
-    }
-    cluster_arrive(); cluster_wait();                        // every CTA's chan[] is complete
-    for (int c = threadIdx.x; c < C; c += NT) {
-        double s1 = 0.0, sx = 0.0;
-        for (int r = 0; r < CS; ++r) { const double* rp = cl.map_shared_rank(chan, r); s1 += rp[c]; sx += rp[C + c]; }
-        const int g = c / cpg;
-        const double s2 = (double)gr[g] * (sx - (double)gm[g] * s1);       // sum dz*xhat
-        tot[c] = (float)s1; tot[C + c] = (float)s2;
-        if (rank == 0) {
-            if (a.dbeta) atomicAdd(a.dbeta + c, (float)s1);
-            if (a.dgamma) atomicAdd(a.dgamma + c, (float)s2);
-        }
-    }
-    cluster_arrive();                                        // remote reads done; waited for before exit
-    __syncthreads();
-    for (int g = threadIdx.x; g < G; g += NT) {
-        float sa = 0.f, sb = 0.f;
-        for (int j = 0; j < cpg; ++j) {
-            const int c = g * cpg + j;
-            const float gmm = __ldg(a.gamma + c);
-            sa = fmaf(gmm, tot[c], sa); sb = fmaf(gmm, tot[C + c], sb);
-        }
-        const float inv = 1.0f / ((float)cpg * (float)HW);
-        gA[g] = sa * inv; gB[g] = sb * inv;
-    }
-    __syncthreads();
-
-    // ---- phase 2: dx = k0*dz - k1*x + k2, written over dz in the slab, then bulk-stored (or bulk-added) row group by row group
-    float csum[VEC];
-#pragma unroll
-    for (int i = 0; i < VEC; ++i) csum[i] = 0.f;
-    float k0[VEC], k1[VEC], k2[VEC];
-#pragma unroll
-    for (int i = 0; i < VEC; ++i) {
-        const int c = min(c0 + i, C - 1), g = c / cpg;
-        const float r_ = gr[g], m_ = gm[g] * gr[g], g_ = __ldg(a.gamma + c);
-        k0[i] = r_ * g_; k1[i] = r_ * r_ * gB[g]; k2[i] = m_ * r_ * gB[g] - r_ * gA[g];
-    }
-    for (int k = 0; k < sp.nq; ++k) {
-        const int g0 = ((sp.rows * k) / sp.nq) * W, g1 = ((sp.rows * (k + 1)) / sp.nq) * W;
-        if (m.active) {
-#pragma unroll 2
-            for (int p = g0; p + m.prow < g1; p += m.ppi) {
-                const uint32_t sa = sm.addr(p);
-                float v[VEC], d[VEC];
-                unpack_bf16x8(lds128(sa), v);
-                unpack_bf16x8(lds128(sa + doff), d);
-#pragma unroll
-                for (int i = 0; i < VEC; ++i) {
-                    d[i] = fmaf(-v[i], k1[i], fmaf(d[i], k0[i], k2[i]));
-                    csum[i] += d[i];
-                }
-                sts128(sa + doff, pack_bf16x8(d));
-            }
-        }
-        sl_fence_async();
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            const int r0 = (sp.rows * k) / sp.nq;
-            for (int b = 0; b < sp.nbox; ++b) {
-                const uint32_t src = dslab + (uint32_t)(b * sp.rows * W + r0 * W) * (uint32_t)(sp.cb * 2);
-                if (a.accumulate) sl_tma_add4(tmO[k], src, b * sp.cb, 0, row0 + r0, n);
-                else sl_tma_store4(tmO[k], src, b * sp.cb, 0, row0 + r0, n);
-            }
-            sl_store_commit();
-        }
-    }
-    cluster_wait();                                          // peers are done with chan[] -> it can be reused
-    if (a.cs_nc || a.cs_c) {
-        cta_channel_reduce<VEC, 1>(part, csum, chan, C, m);
-        for (int c = threadIdx.x; c < C; c += NT) {
-            const float v = (float)chan[c];
-            if (a.cs_nc) atomicAdd(a.cs_nc + (size_t)n * C + c, v);
-            if (a.cs_c) atomicAdd(a.cs_c + c, v);
-        }
-    }
-    if (threadIdx.x == 0) sl_store_wait_read();
-}
-
-// Plan for the slab kernels: cluster size CS (power of two dividing H) such that the share (x `ntensors`) fits the
-// per-CTA budget -- two CTAs per SM when it fits ~111 KB, else one --, channel boxes of <= 256 channels, <= 4 row groups.
-// Returns 0 when the shape does not qualify (the streaming kernels take it).
-//   ddpm_set_gn_slab / DDPM_B200_GN_SLAB=0 turns the slab kernels off; mode 2 / DDPM_B200_GN_SLAB_CS16=0 forbids the
-//   non-portable cluster size 16
-static int gn_slab_env(const char* name, int dflt) {
-    const char* e = getenv(name);
-    return (e && e[0]) ? atoi(e) : dflt;
-}
-static int g_gn_slab = -1, g_gn_slab_cs16 = -1;
-extern "C" int ddpm_set_gn_slab(int mode) { g_gn_slab = mode != 0; g_gn_slab_cs16 = mode == 1; return 0; }
-static int gn_slab_plan(const ddpm_tensor* x, int ntensors, size_t tables, SlabP* sp, size_t* smem_out, int* occ_out) {
-    // Default OFF: measured on B200 (profiles/r2_kbench_gn_slab_variants.txt) the slab kernels are 5-30 % SLOWER than the
-    // streaming kernels at every bench shape although they halve the instruction count and remove the second pass's
-    // DRAM traffic: with one or two 100-200 KB CTAs per SM the load -> statistics -> cluster exchange -> apply -> store
-    // chain of a CTA is serial and nothing else on the SM covers its bubbles.
-    if (g_gn_slab < 0) { g_gn_slab = gn_slab_env("DDPM_B200_GN_SLAB", 0); g_gn_slab_cs16 = gn_slab_env("DDPM_B200_GN_SLAB_CS16", 1); }
-    if (!g_gn_slab) return 0;
-    const int N = x->N, H = x->H, W = x->W, C = x->C;
-    if (W > 256 || C % 8 || C / 8 > NT) return 0;
-    int nbox = 1;
-    while (C / nbox > 256 || C % nbox || (C / nbox) % 8) { if (++nbox > 4) return 0; }
-    if (((size_t)W * (C / nbox) * 2) % 128) return 0;              // every row group / channel box must start 128-byte aligned in shared memory
-    const size_t fixed = 8 * NT * 4 + tables + 8 * SL_MAXQ + 16 + 128;      // reduction scratch, tables, barriers, alignment slack
-    const size_t two_per_sm = 111 * 1024, one_per_sm = 224 * 1024;
-    auto bytes = [&](int cs) { return (size_t)(H / cs) * W * C * 2 * ntensors + fixed; };
-    auto ok = [&](int cs) { return cs <= H && H % cs == 0 && (H / cs) <= 256; };
-    int cs = 0, occ = 2;
-    for (int c = 1; c <= 8 && !cs; c <<= 1) if (ok(c) && bytes(c) <= two_per_sm) cs = c;
-    if (!cs && g_gn_slab_cs16 && ok(16) && bytes(16) <= two_per_sm) cs = 16;
-    if (!cs) { occ = 1; for (int c = 1; c <= 8 && !cs; c <<= 1) if (ok(c) && bytes(c) <= one_per_sm) cs = c; }
-    if (!cs && g_gn_slab_cs16 && ok(16) && bytes(16) <= one_per_sm) { cs = 16; occ = 1; }
-    if (!cs) return 0;
-    while (cs < 8 && (int64_t)N * cs < 2 * 148 && ok(cs * 2) && (H / (2 * cs)) * W >= 32) cs <<= 1;
-    if (bytes(cs) <= two_per_sm) occ = 2;
-    sp->rows = H / cs; sp->nq = sp->rows < SL_MAXQ ? sp->rows : SL_MAXQ;
-    sp->nbox = nbox; sp->cb = C / nbox; sp->slab_bytes = sp->rows * W * C * 2;
-    *smem_out = bytes(cs); *occ_out = occ;
-    return cs;
-}
-// (c, x, y, n) view of the interior of a halo'd NHWC bf16 buffer; box = [cb][W][rows of row group k][1]
-static int gn_slab_maps(const ddpm_tensor* t, const SlabP& sp, CUtensorMap* out) {
-    const int Hp = t->H + 2 * t->halo, Wp = t->W + 2 * t->halo;
-    char* base = (char*)t->ptr + ((size_t)t->halo * Wp + t->halo) * t->pitch * 2;
-    const uint64_t dims[4] = {(uint64_t)t->C, (uint64_t)t->W, (uint64_t)t->H, (uint64_t)t->N};
-    const uint64_t strides[3] = {(uint64_t)t->pitch * 2, (uint64_t)Wp * t->pitch * 2, (uint64_t)Hp * Wp * t->pitch * 2};
-    for (int k = 0; k < SL_MAXQ; ++k) {
-        const int kk = k < sp.nq ? k : sp.nq - 1;
-        const int r0 = (sp.rows * kk) / sp.nq, r1 = (sp.rows * (kk + 1)) / sp.nq;
-        const uint32_t box[4] = {(uint32_t)sp.cb, (uint32_t)t->W, (uint32_t)(r1 - r0), 1u};
-        int rc = ddpm_encode_tiled_bf16(&out[k], base, 4, dims, strides, box, 0);
-        if (rc) return rc;
-    }
-    return 0;
-}
-static bool gn_slab_tensor_ok(const ddpm_tensor* t) {
-    return (t->pitch % 8) == 0 && (((uintptr_t)t->ptr) % 16) == 0 && t->C % 8 == 0;
-}
-static int launch_slab_cfg(cudaLaunchConfig_t* cfg, cudaLaunchAttribute* at, unsigned* nat, const void* kernel, int grid, int cs, size_t smem,
-                           cudaStream_t st) {
-    static std::unordered_map<const void*, size_t> configured;
-    size_t& have = configured[kernel];
-    if (smem > have) {
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return (int)e;
-        have = smem;
-    }
-    if (cs > 8) {
-        static std::unordered_map<const void*, int> np;
-        int& h2 = np[kernel];
-        if (!h2) {
-            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-            if (e != cudaSuccess) return (int)e;
-            h2 = 1;
-        }
-    }
-    *cfg = cudaLaunchConfig_t{};
-    cfg->gridDim = dim3(grid); cfg->blockDim = dim3(NT); cfg->dynamicSmemBytes = smem; cfg->stream = st;
-    *nat = 1;
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = cs; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    pdl_attr(at, nat);
-    cfg->attrs = at; cfg->numAttrs = *nat;
-    return 0;
-}
-
 // cluster size: enough CTAs per image that a thread sees ~16 packets per phase, at most 8 (portable limit)
-static int gn_max_cluster() {              // experiment: DDPM_B200_GN_CS16=1 allows the non-portable cluster size 16
-    static int v = 0;
-    if (v == 0) { const char* e = getenv("DDPM_B200_GN_CS16"); v = (e && e[0] == '1') ? 16 : 8; }
-    return v;
-}
 static int gn_cluster_size(int HW, int cvs, int N = 1 << 30) {
     const int64_t packets = (int64_t)HW * cvs;
     int cs = 1;
-    // DDPM_B200_GN_CSMAX caps the cluster size (experiment knob).  Round 2 measured smaller clusters for the mid-size shapes
-    // (>= 48 packets per thread instead of >= 12): alone, 192@32 backward 82.8 -> 70.7 us, forward 47.3 -> 40.4, 384@16 backward
-    // 46.6 -> 40.1 (profiles/r2_gn_cluster_granularity.txt) -- but in the train step and in DDIM-100 the same-box A/B showed
-    // no change (11.96 vs 12.04 ms; 6.69 vs 6.63 ms per evaluation, inside the noise), so the rule stays as it was.
-    static int cap = 0;
-    if (cap == 0) { const char* e = getenv("DDPM_B200_GN_CSMAX"); cap = e ? atoi(e) : 8; if (cap < 1) cap = 1; }
-    while (cs < 8 && cs < cap && packets / (cs * NT) >= 24) cs <<= 1;
-    if (cs == 8 && gn_max_cluster() == 16 && packets / (16 * NT) >= 12) cs = 16;
+    // Round 2 measured smaller clusters for the mid-size shapes (>= 48 packets per thread instead of >= 12): alone, 192@32
+    // backward 82.8 -> 70.7 us, forward 47.3 -> 40.4, 384@16 backward 46.6 -> 40.1 (profiles/r2_gn_cluster_granularity.txt)
+    // -- but in the train step and in DDIM-100 the same-box A/B showed no change (11.96 vs 12.04 ms; 6.69 vs 6.63 ms per
+    // evaluation, inside the noise), so the rule stays as it was.
+    while (cs < 8 && packets / (cs * NT) >= 24) cs <<= 1;
     // Very few large images (fewer CTAs than SMs with clusters of 8): clusters of 16 (non-portable size) double the number of
     // CTAs per image -- 256-px sampling at B = 16: 12.3 -> 11.5 ms per evaluation; at B = 32 (256 CTAs already) it measured
-    // 1.4 % SLOWER, hence the N * 8 <= 148 bound.  DDPM_B200_GN_CS16=0 forbids it (A/B).
-    static int allow16 = -1;
-    if (allow16 < 0) { const char* e = getenv("DDPM_B200_GN_CS16"); allow16 = !(e && e[0] == '0'); }
-    if (cs == 8 && allow16 && (int64_t)N * 8 <= 148 && packets / (16 * NT) >= 24) cs = 16;
+    // 1.4 % SLOWER, hence the N * 8 <= 148 bound.
+    if (cs == 8 && (int64_t)N * 8 <= 148 && packets / (16 * NT) >= 24) cs = 16;
     return cs;
 }
 static int log2_exact(int v) { int s = 0; while ((1 << s) < v) ++s; return (1 << s) == v ? s : -1; }
@@ -1056,20 +569,6 @@ static int gn_fwd_dispatch(GnP& p, const ddpm_tensor* x, const ddpm_tensor* out,
         return launch_cluster(gn_fwd_kernel<T, VEC, MODE>, x->N * cs, cs, sm0 + gn_ring_bytes<VEC, 1, GN_PIPE_D_FWD>(), st, p); }
     const bool v8 = vec_ok(x, 8, 2) && (MODE == 1 || MODE == 3 || vec_ok(out, 8, 2));
     const bool v4 = vec_ok(x, 4, 4) && (MODE == 1 || MODE == 3 || vec_ok(out, 4, 4));
-    if (MODE == 0 && dtype == DDPM_BF16 && v8 && gn_slab_tensor_ok(x) && gn_slab_tensor_ok(out)) {
-        size_t smem = 0; int occ = 0; SlabP sp;
-        const int cs = gn_slab_plan(x, 1, sm0, &sp, &smem, &occ);
-        if (cs) {
-            CUtensorMap mx[SL_MAXQ], mo[SL_MAXQ];
-            int rc = gn_slab_maps(x, sp, mx); if (rc) return rc;
-            rc = gn_slab_maps(out, sp, mo); if (rc) return rc;
-            cudaLaunchConfig_t cfg; cudaLaunchAttribute at[2]; unsigned nat;
-            rc = launch_slab_cfg(&cfg, at, &nat, (const void*)gn_fwd_slab_kernel, x->N * cs, cs, smem, st); if (rc) return rc;
-            CUDA_TRY(cudaLaunchKernelEx(&cfg, gn_fwd_slab_kernel, mx[0], mx[1], mx[2], mx[3], mo[0], mo[1], mo[2], mo[3], p, sp));
-            LAUNCH_OK();
-            return 0;
-        }
-    }
     if (dtype == DDPM_BF16) { if (v8) GO(bf16, 8) else GO(bf16, 1) }
     else if (dtype == DDPM_F32) { if (v4) GO(float, 4) else GO(float, 1) }
 #undef GO
@@ -1129,26 +628,6 @@ static int gn_bwd_impl(const ddpm_tensor* x, int dtype, int groups, const double
         const size_t sm = sm0 + gn_ring_bytes<VEC, 3>(); \
         if (p.stash) return launch_cluster(gn_bwd_kernel<T, VEC, true>, x->N * cs, cs, sm, st, p); \
         return launch_cluster(gn_bwd_kernel<T, VEC, false>, x->N * cs, cs, sm, st, p); }
-    // (the slab backward adds into dx with a bulk reduce-add and never sees the old dx, so it cannot also emit the column
-    // sums of the accumulated result -- a combination the UNet backward does not use)
-    if (dtype == DDPM_BF16 && gn_slab_tensor_ok(x) && gn_slab_tensor_ok(dy) && gn_slab_tensor_ok(dx) &&
-        !(accumulate && (cs_nc || cs_c))) {
-        size_t smem = 0; int occ = 0; SlabP sp;
-        const int cs = gn_slab_plan(x, 2, sm0, &sp, &smem, &occ);
-        if (cs) {
-            CUtensorMap mx[SL_MAXQ], md[SL_MAXQ], mo[SL_MAXQ];
-            int rc = gn_slab_maps(x, sp, mx); if (rc) return rc;
-            rc = gn_slab_maps(dy, sp, md); if (rc) return rc;
-            rc = gn_slab_maps(dx, sp, mo); if (rc) return rc;
-            cudaLaunchConfig_t cfg; cudaLaunchAttribute at[2]; unsigned nat;
-            const void* kern = occ == 2 ? (const void*)gn_bwd_slab_kernel<2> : (const void*)gn_bwd_slab_kernel<1>;
-            rc = launch_slab_cfg(&cfg, at, &nat, kern, x->N * cs, cs, smem, st); if (rc) return rc;
-            if (occ == 2) CUDA_TRY(cudaLaunchKernelEx(&cfg, gn_bwd_slab_kernel<2>, mx[0], mx[1], mx[2], mx[3], md[0], md[1], md[2], md[3], mo[0], mo[1], mo[2], mo[3], p, sp));
-            else CUDA_TRY(cudaLaunchKernelEx(&cfg, gn_bwd_slab_kernel<1>, mx[0], mx[1], mx[2], mx[3], md[0], md[1], md[2], md[3], mo[0], mo[1], mo[2], mo[3], p, sp));
-            LAUNCH_OK();
-            return 0;
-        }
-    }
     if (dtype == DDPM_BF16) { if (vec_ok(x, 8, 2) && vec_ok(dy, 8, 2) && vec_ok(dx, 8, 2)) GO(bf16, 8) else GO(bf16, 1) }
     else if (dtype == DDPM_F32) { if (vec_ok(x, 4, 4) && vec_ok(dy, 4, 4) && vec_ok(dx, 4, 4)) GO(float, 4) else GO(float, 1) }
 #undef GO

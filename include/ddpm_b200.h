@@ -145,12 +145,6 @@ int ddpm_gn_bwd_colsum(const ddpm_tensor* x, int dtype, int groups, const double
                        const float* beta, float eps, int act, float p_drop, const uint64_t* rng,
                        uint32_t layer_id, const ddpm_tensor* dy, const ddpm_tensor* dx, int accumulate,
                        float* dgamma, float* dbeta, float* colsum_nc, float* colsum_c, int dy_scratch, void* stream);
-/* Kernel selection for the bf16 GroupNorm forward (fused) / backward: 0 (default) = the streaming kernels; 1 = the CTA's
- * rows of an image arrive by bulk tensor copy, stay in shared memory between the statistics and the apply phase and
- * leave by bulk tensor store / reduce-add where they fit ("slab" kernels: every tensor crosses HBM once); 2 = slab
- * kernels without 16-CTA clusters.  The slab kernels measured slower on B200 (DESIGN.md section 4.2) and are kept for
- * A/B measurements; results are the same up to fp32 summation order (and one extra bf16 rounding when dx accumulates). */
-int ddpm_set_gn_slab(int mode);
 
 /* nearest x2 (unet_backbone.py:63) and its adjoint (2x2 sum) */
 int ddpm_upsample2x(const ddpm_tensor* x, const ddpm_tensor* out, int dtype, void* stream);
@@ -209,13 +203,17 @@ typedef struct {
 int ddpm_conv(const ddpm_conv_args* a, void* stream);
 /* 1 when ddpm_conv would run `a` (with a non-NULL gn_ab) on the fused tensor-core path, else 0 (then ddpm_conv rejects it) */
 int ddpm_conv_gn_fusable(const ddpm_conv_args* a);
-/* test / tuning hooks: force the CUDA-core kernels; choose the tcgen05 operand layout
- * (0 = SWIZZLE_NONE, 1 = SWIZZLE_32B [+ descriptor base_offset]) */
+/* test / tuning hooks: force the CUDA-core kernels */
 int ddpm_set_force_simt(int on);
+/* Force tensor-core paths that the planners otherwise pick only for other shapes (tests, A/B measurements).  Bit 0 of
+ * `mode` must be 1, bits 1-3 and base_offset must be 0, and mode >> 4 is a combination of
+ *   32    convolution: keep a channel tile wider than 128 (NT = 192 / 256) instead of halving it
+ *   64    convolution: stream the weights with every stage instead of keeping them resident in shared memory
+ *   128   convolution: 16-byte instead of 32-byte epilogue loads / stores
+ *   1024  weight gradient: the single-CTA kernel instead of the CTA-pair kernel
+ * (1 restores the default planning).  The flags are read on the host when a call plans its launch; no kernel sees them.
+ * Anything else returns DDPM_E_ARG and leaves the setting unchanged. */
 int ddpm_set_tc_mode(int mode, int base_offset);
-/* 1 (default): persistent CTA-pair kernel (tcgen05 cta_group::2, TMEM double buffering); 0: the
- * first-generation one-tile-per-CTA kernel (kept for A/B measurements) */
-int ddpm_set_tc_v2(int on);
 /* 1 (env DDPM_B200_PDL=1): kernels are launched with programmatic stream serialisation (griddepcontrol): the prologue of
  * kernel i+1 overlaps the tail of kernel i.  0 (default since round 2): plain stream order -- measured neutral at 64 px and
  * 5-25 % slower at 256 px with it on (DESIGN.md section 6). */

@@ -208,10 +208,17 @@ def test_conv_epilogues(pkg):
     assert rel(out.interior().permute(0, 3, 1, 2), ref + F.conv2d(x, w, None, padding=1)) < 2e-5
 
 
+def _halo_max(a):
+    t = a.buf.t.float()
+    return float(max(t[:, 0].abs().max(), t[:, -1].abs().max(), t[:, :, 0].abs().max(), t[:, :, -1].abs().max()))
+
+
 @pytest.mark.parametrize("dt_name", ["f32", "bf16"])
 @pytest.mark.parametrize("shape", [(2, 32, 8, 8), (2, 96, 8, 8), (1, 288, 4, 4), (2, 64, 16, 16), (3, 96, 64, 64),
                                    (2, 192, 16, 16), (2, 192, 32, 32), (2, 96, 12, 20),
-                                   (2, 128, 128, 128)])       # last: few large images -> clusters of 16 CTAs
+                                   (2, 128, 128, 128),        # few large images -> clusters of 16 CTAs
+                                   (130, 192, 16, 16), (2, 288, 64, 64), (3, 96, 24, 24), (2, 384, 32, 32), (5, 192, 8, 8),
+                                   (2, 32, 4, 4)])
 @pytest.mark.parametrize("act", [0, 1])
 def test_groupnorm_fwd_bwd(pkg, shape, act, dt_name):
     _, _lib, engine = pkg
@@ -237,29 +244,33 @@ def test_groupnorm_fwd_bwd(pkg, shape, act, dt_name):
     st = engine.gn_stats(E, xa, gdev.num_groups)
     ya = engine.gn_apply(E, xa, st, gdev, act, 0.0, 0)
     assert rel(_from_act(pkg, E, ya), y) < tol
-    # fused stats+apply (one cluster per image) must agree with the two-launch path and the reference
+    # fused stats+apply (one cluster per image) must agree with the two-launch path and the reference (ATen fp32 on the
+    # bf16-rounded input: without the activation, the bf16 output is within a rounding step of it)
     yf, stf = engine.gn_fwd(E, xa, gdev, act, 0.0, 0)
-    assert rel(_from_act(pkg, E, yf), y) < tol
+    assert rel(_from_act(pkg, E, yf), y) < (6e-3 if dt_name == "bf16" and not act else tol)
     assert torch.allclose(stf, st, rtol=1e-6, atol=1e-6)
     dya = _to_act(pkg, E, dy)
     dxa = engine.gn_bwd(E, xa, st, gdev, act, 0.0, 0, dya, E.act(N, H, W, Cc), False)
     assert rel(_from_act(pkg, E, dxa), xr.grad) < tol
     assert rel(gdev.weight.grad, gn.weight.grad) < tol
     assert rel(gdev.bias.grad, gn.bias.grad) < tol
-    # scratch-dy variant with fused column sums (what the UNet backward uses)
-    gdev.weight.grad = None; gdev.bias.grad = None
-    dyb = _to_act(pkg, E, dy)
-    cs_nc = torch.full((N, Cc), 7.0, device=dev())
-    cbias = torch.nn.Parameter(torch.zeros(Cc, device=dev()))
-    dxb = engine.gn_bwd(E, xa, st, gdev, act, 0.0, 0, dyb, E.act(N, H, W, Cc), False, colsum_nc=cs_nc, colsum_bias=cbias,
-                        dy_scratch=True)
-    got = _from_act(pkg, E, dxb)
-    assert rel(got, xr.grad) < tol
-    assert rel(gdev.weight.grad, gn.weight.grad) < tol
-    # (per-group sums of a GroupNorm gradient are ~0, so compare against the scale of sum|dx|, not of the sum)
+    # scratch-dy variant with fused column sums (what the UNet backward uses), into a new buffer and in place (dx is dy)
     ctol = 1e-5 if dt_name == "f32" else 2e-3
-    assert float((cs_nc.cpu() - got.sum((2, 3))).abs().max()) < ctol * float(got.abs().sum((2, 3)).max())
-    assert float((cbias.grad.cpu() - got.sum((0, 2, 3))).abs().max()) < ctol * float(got.abs().sum((0, 2, 3)).max())
+    for in_place in (False, True):
+        gdev.weight.grad = None; gdev.bias.grad = None
+        dyb = _to_act(pkg, E, dy)
+        cs_nc = torch.full((N, Cc), 7.0, device=dev())
+        cbias = torch.nn.Parameter(torch.zeros(Cc, device=dev()))
+        dxb = engine.gn_bwd(E, xa, st, gdev, act, 0.0, 0, dyb, dyb if in_place else E.act(N, H, W, Cc), False, colsum_nc=cs_nc,
+                            colsum_bias=cbias, dy_scratch=True)
+        assert _halo_max(dxb) == 0.0, in_place
+        got = _from_act(pkg, E, dxb)
+        assert rel(got, xr.grad) < tol, in_place
+        assert rel(gdev.weight.grad, gn.weight.grad) < tol, in_place
+        assert rel(gdev.bias.grad, gn.bias.grad) < tol, in_place
+        # (per-group sums of a GroupNorm gradient are ~0, so compare against the scale of sum|dx|, not of the sum)
+        assert float((cs_nc.cpu() - got.sum((2, 3))).abs().max()) < ctol * float(got.abs().sum((2, 3)).max())
+        assert float((cbias.grad.cpu() - got.sum((0, 2, 3))).abs().max()) < ctol * float(got.abs().sum((0, 2, 3)).max())
     # accumulate variant: dx += ...
     base = torch.randn(N, Cc, H, W)
     if dt_name == "bf16":
@@ -267,6 +278,8 @@ def test_groupnorm_fwd_bwd(pkg, shape, act, dt_name):
     acc = _to_act(pkg, E, base)
     engine.gn_bwd(E, xa, st, gdev, act, 0.0, 0, dya, acc, True)
     assert rel(_from_act(pkg, E, acc), xr.grad + base) < tol
+    # no kernel writes the zero halo
+    assert max(_halo_max(ya), _halo_max(yf), _halo_max(dxa), _halo_max(acc)) == 0.0
 
 
 def test_dropout_statistics(pkg):

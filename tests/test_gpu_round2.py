@@ -339,60 +339,6 @@ def test_grad_norm_diagnostic_uses_the_scale_of_its_own_step():
     assert abs(g - st[0] ** 0.5 / st[2]) < 1e-6 * max(1.0, g) and g > 0
 
 
-@pytest.mark.parametrize("shape", [(3, 96, 64, 64), (2, 192, 32, 32), (2, 384, 32, 32), (5, 192, 8, 8), (2, 288, 64, 64),
-                                   (3, 96, 24, 24), (2, 32, 4, 4), (130, 192, 16, 16)])
-@pytest.mark.parametrize("mode", [1, 2])
-def test_groupnorm_slab_kernels_match_streaming_kernels_and_aten(shape, mode):
-    """The opt-in shared-memory-resident ("slab") GroupNorm kernels -- TMA in / out, clusters of 1..16 CTAs -- against
-    the streaming kernels on identical bf16 inputs (forward with SiLU + dropout, backward with accumulate, fused
-    column sums, in-place dy) and against ATen fp32 on the bf16-rounded input."""
-    from ddpm_diffusion_model_b200 import _lib, engine
-    import torch.nn.functional as F
-    N, Cc, H, W = shape
-    torch.manual_seed(11)
-    rng = torch.tensor([77, 3], dtype=torch.int64, device=dev())
-    E = engine.Exec(dev(), _lib.BF16, True, True, rng=rng)
-    gn = torch.nn.GroupNorm(32, Cc, eps=1e-6).to(dev())
-    with torch.no_grad():
-        gn.weight.normal_(1.0, 0.3); gn.bias.normal_(0.0, 0.3)
-    x = E.act(N, H, W, Cc); x.interior().normal_().mul_(1.7).add_(0.4)
-    dy0 = torch.randn(N, H, W, Cc, device=dev())
-    dx0 = torch.randn(N, H, W, Cc, device=dev())
-    res = {}
-    try:
-        for m in (0, mode):
-            _lib.lib.ddpm_set_gn_slab(m)
-            gn.weight.grad = gn.bias.grad = None
-            bias_p = torch.nn.Parameter(torch.zeros(Cc, device=dev()))
-            y, st = engine.gn_fwd(E, x, gn, 1, 0.2, 5)
-            y_plain, _ = engine.gn_fwd(E, x, gn, 0, 0.0, 0)
-            dy = E.act(N, H, W, Cc); dy.interior().copy_(dy0)
-            dx = E.act(N, H, W, Cc); dx.interior().copy_(dx0)
-            cs = torch.empty(N, Cc, device=dev())
-            engine.gn_bwd(E, x, st, gn, 1, 0.2, 5, dy, dx, True, dy_scratch=True)                 # dx += (bulk reduce-add)
-            dy2 = E.act(N, H, W, Cc); dy2.interior().copy_(dy0)
-            engine.gn_bwd(E, x, st, gn, 1, 0.2, 5, dy2, dy2, False, colsum_nc=cs, colsum_bias=bias_p, dy_scratch=True)   # in place + column sums
-            torch.cuda.synchronize()
-            res[m] = dict(y=y.interior().float().clone(), y_plain=y_plain.interior().float().clone(), st=st.clone(),
-                          dx=dx.interior().float().clone(), dip=dy2.interior().float().clone(), cs=cs.clone(),
-                          dg=gn.weight.grad.clone(), db=gn.bias.grad.clone(), bp=bias_p.grad.clone(),
-                          halo=float(dx.buf.t[:, 0].abs().max() + dx.buf.t[:, :, -1].abs().max() + y.buf.t[:, -1].abs().max()))
-    finally:
-        _lib.lib.ddpm_set_gn_slab(0)
-    a, b = res[0], res[mode]
-    assert b["halo"] == 0.0
-    assert torch.allclose(a["st"], b["st"], rtol=1e-6, atol=1e-4)
-    # same mask, same arithmetic up to fp32 summation order -> bf16 outputs agree to a rounding step
-    for k, tol in (("y", 1e-2), ("y_plain", 1e-2), ("dx", 1e-2), ("dip", 1e-2), ("cs", 1e-2), ("dg", 1e-2), ("db", 1e-2), ("bp", 1e-2)):
-        assert rel(b[k], a[k]) < tol, (k, rel(b[k], a[k]))
-    keep_a, keep_b = a["y"] != 0, b["y"] != 0
-    assert float((keep_a != keep_b).float().mean()) < 1e-3                         # identical dropout mask
-    # independent leg (no dropout, no activation): ATen fp32 group_norm of the bf16-rounded input
-    xr = x.interior().float().permute(0, 3, 1, 2)
-    ref = F.group_norm(xr, 32, gn.weight, gn.bias, eps=1e-6).permute(0, 2, 3, 1)
-    assert rel(b["y_plain"], ref) < 6e-3
-
-
 @pytest.mark.parametrize("case", [(2, 32, 32, 8, 8), (3, 192, 192, 16, 16), (2, 192, 192, 32, 32), (1, 128, 128, 128, 128), (5, 64, 64, 4, 4)])
 def test_upsample_folded_into_the_conv_gather(case, monkeypatch):
     """Upsample = nearest x2 + conv3x3 (unet_backbone.py:56-64) on the tensor-core path: four 2x2-tap phase convolutions

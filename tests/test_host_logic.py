@@ -29,6 +29,21 @@ def test_abi_exports_every_declared_symbol():
     assert lib.ddpm_abi_version() == 1
 
 
+def test_tc_mode_accepts_only_the_path_forcing_flags():
+    """ddpm_set_tc_mode takes bit 0 = 1, base_offset 0 and flags 32 / 64 / 128 / 1024 in mode >> 4; it rejects anything
+    else (such as the flags of removed experimental kernels) instead of silently ignoring it."""
+    from ddpm_diffusion_model_b200 import _lib
+    f = _lib.lib.ddpm_set_tc_mode
+    try:
+        for flags in (0, 32, 64, 128, 1024, 32 | 64 | 128 | 1024):
+            assert f(1 | flags << 4, 0) == 0, flags
+        for mode, base_offset in ((0, 0), (1, 1), (3, 0), (1 | 1 << 4, 0), (1 | 4 << 4, 0), (1 | 256 << 4, 0), (1 | 512 << 4, 0),
+                                  (1 | 2048 << 4, 0), (1 | 4096 << 4, 0), (1 | (1024 | 2048) << 4, 0), (-1, 0)):
+            assert f(mode, base_offset) == -1, (mode, base_offset)
+    finally:
+        assert f(1, 0) == 0
+
+
 def test_struct_layouts_match_header():
     from ddpm_diffusion_model_b200 import _lib
     assert ctypes.sizeof(_lib.Tensor) == 32            # void* + 6 x int32

@@ -18,12 +18,9 @@ ap.add_argument("--no-ddim", action="store_true")
 ap.add_argument("--no-layers", action="store_true")
 ap.add_argument("--c256", action="store_true")
 ap.add_argument("--shape", default=None, help="one 'Cin,Cout,H,k' (for ncu)")
-ap.add_argument("--tcexp", type=int, default=0, help="conv experiment flags (ddpm_set_tc_mode(1 | flags << 4)); timing only")
 args = ap.parse_args()
 dev = torch.device("cuda", 0)
 B = args.batch
-if args.tcexp:
-    _lib.lib.ddpm_set_tc_mode(1 | (args.tcexp << 4), 0)
 
 
 def timeit(fn, reps=None):

@@ -4,7 +4,7 @@ Times every kernel family of the hot path alone, at the shapes of the bench work
 B=128 by default), with CUDA events on the launching stream, and prints achieved TFLOP/s or GB/s
 against MEASURED_PEAKS.json.  Algorithmic bytes / FLOPs per launch are the DESIGN.md figures.
 
-    python tools/kbench.py [--batch 128] [--only conv,wgrad,gn,colsum,ew,param] [--exp] [--json out.json]
+    python tools/kbench.py [--batch 128] [--only conv,wgrad,gn,colsum,ew,param] [--tcexp FLAGS] [--json out.json]
 """
 import argparse, json, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -15,14 +15,11 @@ from ddpm_diffusion_model_b200 import _lib, engine
 ap = argparse.ArgumentParser()
 ap.add_argument("--batch", type=int, default=128)
 ap.add_argument("--only", default="conv,wgrad,gn,colsum,ew,param")
-ap.add_argument("--exp", action="store_true", help="conv: also run with A / B / both TMA loads skipped (diagnostic)")
 ap.add_argument("--reps", type=int, default=10)
 ap.add_argument("--json", default=None)
 ap.add_argument("--epi", action="store_true", help="conv: also time with bias + time-bias + residual epilogue")
-ap.add_argument("--v1", action="store_true", help="conv: also time the first-generation kernel")
 ap.add_argument("--gnshape", default=None, help="restrict gn to one 'C,H'")
-ap.add_argument("--tcexp", type=int, default=0, help="experiment flags for the whole run (ddpm_set_tc_mode(1 | flags << 4)), e.g. 512 = wgrad with (1,3,1) clusters + dY multicast, 1024 = single-CTA wgrad kernel instead of the pair kernel, 2048 = pair kernel with the PDL attribute")
-ap.add_argument("--gnslab", default="1", help="gn: comma list of ddpm_set_gn_slab modes to time (0 streaming, 1 slab, 2 slab without 16-CTA clusters)")
+ap.add_argument("--tcexp", type=int, default=0, help="path-forcing flags for the whole run (ddpm_set_tc_mode(1 | flags << 4)): 32 = conv channel tiles wider than 128, 64 = conv weights streamed instead of resident, 128 = no 32-byte conv epilogue stores, 1024 = single-CTA wgrad kernel instead of the pair kernel")
 ap.add_argument("--shape", default=None, help="restrict conv/wgrad to one 'Cin,Cout,H' (for ncu)")
 args = ap.parse_args()
 only = set(args.only.split(","))
@@ -81,6 +78,7 @@ if args.gnshape:
     c_, h_ = [int(v) for v in args.gnshape.split(",")]
     GN = [(c_, h_, 1)]
 E = engine.Exec(dev, _lib.BF16, True, True, rng=torch.tensor([1, 0], dtype=torch.int64, device=dev))
+_lib.call("ddpm_set_tc_mode", 1 | (args.tcexp << 4), 0)
 
 if "conv" in only:
     for ci, co, hw, cnt, *kk in CONV:
@@ -90,12 +88,8 @@ if "conv" in only:
         x = E.act(B, hw, hw, ci); x.interior().normal_()
         y = E.act(B, hw, hw, co)
         fl = 2.0 * B * hw * hw * co * ci * ks * ks
-        modes = [(1, "")] + ([(1 | (3 << 4), " skipAB"), (1 | (4 << 4), " skipEpi"), (1 | (8 << 4), " skipStores"), (1 | (7 << 4), " skipAB+Epi"), (1 | (32 << 4), " skip(NT/2)")] if args.exp else [])
-        for mode, tag in modes:
-            _lib.lib.ddpm_set_tc_mode(mode, 0)
-            sec = timeit(lambda: engine.conv(E, x, wf, y, ks, 1, ks // 2))
-            report("conv", f"{ci}->{co}@{hw}k{ks}{tag}", sec, flops=fl, cnt=2 * cnt)
-        _lib.lib.ddpm_set_tc_mode(1, 0)
+        sec = timeit(lambda: engine.conv(E, x, wf, y, ks, 1, ks // 2))
+        report("conv", f"{ci}->{co}@{hw}k{ks}", sec, flops=fl, cnt=2 * cnt)
         if args.epi:
             bias = torch.randn(co, device=dev); tb = torch.randn(B, co, device=dev)
             r = E.act(B, hw, hw, co); r.interior().normal_()
@@ -104,15 +98,9 @@ if "conv" in only:
             sec = timeit(lambda: engine.conv(E, x, wf, y, ks, 1, ks // 2, bias=bias, accum=True))
             report("conv", f"{ci}->{co}@{hw}k{ks} skip(+bias+accum)", sec, flops=fl, cnt=2 * cnt)
             del r
-        if args.v1:
-            _lib.lib.ddpm_set_tc_v2(0)
-            sec = timeit(lambda: engine.conv(E, x, wf, y, ks, 1, ks // 2))
-            report("conv", f"{ci}->{co}@{hw}k{ks} skip(v1 kernel)", sec, flops=fl, cnt=2 * cnt)
-            _lib.lib.ddpm_set_tc_v2(1)
         del x, y
 
 if "wgrad" in only:
-    _lib.lib.ddpm_set_tc_mode(1 | (args.tcexp << 4), 0)
     for ci, co, hw, cnt, *kk in CONV:
         w = torch.nn.Parameter(torch.zeros(co, ci, 3, 3, device=dev))
         x = E.act(B, hw, hw, ci); x.interior().normal_()
@@ -126,26 +114,23 @@ if "wgrad" in only:
         del x, dy
 
 if "gn" in only:
-  for slab_mode in [int(v) for v in args.gnslab.split(",")]:
-    _lib.lib.ddpm_set_gn_slab(slab_mode)
-    print(f"--- gn, ddpm_set_gn_slab({slab_mode})", flush=True)
     for c, hw, cnt in GN:
-          gn = torch.nn.GroupNorm(32, c, eps=1e-6).to(dev)
-          x = E.act(B, hw, hw, c); x.interior().normal_()
-          o = E.act(B, hw, hw, c)
-          dy = E.act(B, hw, hw, c); dy.interior().normal_()
-          dx = E.act(B, hw, hw, c)
-          n = B * hw * hw * c
-          fl = n * 2 > (100 << 20)            # flush L2 between reps only when the tensor would not fit anyway
-          st = engine.gn_stats(E, x, 32)
-          report("gn", f"stats {c}@{hw}", timeit(lambda: engine.gn_stats(E, x, 32), flush=fl), nbytes=2 * n, cnt=cnt)
-          report("gn", f"apply+silu {c}@{hw}", timeit(lambda: engine.gn_apply(E, x, st, gn, 1, 0.0, 0, out=o), flush=fl), nbytes=4 * n, cnt=cnt)
-          report("gn", f"FUSED fwd silu+drop {c}@{hw}", timeit(lambda: engine.gn_fwd(E, x, gn, 1, 0.1, 3, out=o), flush=fl), nbytes=4 * n, cnt=cnt)
-          report("gn", f"apply+silu+drop {c}@{hw}", timeit(lambda: engine.gn_apply(E, x, st, gn, 1, 0.1, 3, out=o), flush=fl), nbytes=4 * n, cnt=cnt)
-          report("gn", f"bwd(silu+drop) {c}@{hw}", timeit(lambda: engine.gn_bwd(E, x, st, gn, 1, 0.1, 3, dy, dx, False, dy_scratch=True), flush=fl), nbytes=6 * n, cnt=cnt)
-          report("gn", f"skip bwd accumulate {c}@{hw}", timeit(lambda: engine.gn_bwd(E, x, st, gn, 1, 0.0, 0, dy, dx, True, dy_scratch=True), flush=fl), nbytes=8 * n, cnt=cnt)
-          report("gn", f"skip FUSED fwd silu (eval) {c}@{hw}", timeit(lambda: engine.gn_fwd(E, x, gn, 1, 0.0, 0, out=o), flush=fl), nbytes=4 * n, cnt=cnt)
-          del x, o, dy, dx
+        gn = torch.nn.GroupNorm(32, c, eps=1e-6).to(dev)
+        x = E.act(B, hw, hw, c); x.interior().normal_()
+        o = E.act(B, hw, hw, c)
+        dy = E.act(B, hw, hw, c); dy.interior().normal_()
+        dx = E.act(B, hw, hw, c)
+        n = B * hw * hw * c
+        fl = n * 2 > (100 << 20)            # flush L2 between reps only when the tensor would not fit anyway
+        st = engine.gn_stats(E, x, 32)
+        report("gn", f"stats {c}@{hw}", timeit(lambda: engine.gn_stats(E, x, 32), flush=fl), nbytes=2 * n, cnt=cnt)
+        report("gn", f"apply+silu {c}@{hw}", timeit(lambda: engine.gn_apply(E, x, st, gn, 1, 0.0, 0, out=o), flush=fl), nbytes=4 * n, cnt=cnt)
+        report("gn", f"FUSED fwd silu+drop {c}@{hw}", timeit(lambda: engine.gn_fwd(E, x, gn, 1, 0.1, 3, out=o), flush=fl), nbytes=4 * n, cnt=cnt)
+        report("gn", f"apply+silu+drop {c}@{hw}", timeit(lambda: engine.gn_apply(E, x, st, gn, 1, 0.1, 3, out=o), flush=fl), nbytes=4 * n, cnt=cnt)
+        report("gn", f"bwd(silu+drop) {c}@{hw}", timeit(lambda: engine.gn_bwd(E, x, st, gn, 1, 0.1, 3, dy, dx, False, dy_scratch=True), flush=fl), nbytes=6 * n, cnt=cnt)
+        report("gn", f"skip bwd accumulate {c}@{hw}", timeit(lambda: engine.gn_bwd(E, x, st, gn, 1, 0.0, 0, dy, dx, True, dy_scratch=True), flush=fl), nbytes=8 * n, cnt=cnt)
+        report("gn", f"skip FUSED fwd silu (eval) {c}@{hw}", timeit(lambda: engine.gn_fwd(E, x, gn, 1, 0.0, 0, out=o), flush=fl), nbytes=4 * n, cnt=cnt)
+        del x, o, dy, dx
 
 if "colsum" in only:
     for c, hw, cnt in [(96, 64, 12), (192, 32, 12), (192, 16, 12), (192, 8, 20)]:
