@@ -29,7 +29,7 @@ class ConvArgs(C.Structure):
                 ("KH", C.c_int32), ("KW", C.c_int32), ("stride", C.c_int32), ("pad", C.c_int32),
                 ("mode", C.c_int32), ("a_silu", C.c_int32), ("epi", C.c_int32), ("dtype", C.c_int32),
                 ("prefer_tc", C.c_int32), ("bias_n", C.c_int32), ("in2", Tensor), ("w2", C.c_void_p),
-                ("up_phase", C.c_int32), ("gn_ab", C.c_void_p), ("gn_act", C.c_int32)]
+                ("up_phase", C.c_int32)]
 
 
 class WgradArgs(C.Structure):
@@ -83,7 +83,6 @@ SIGNATURES = {
     "ddpm_nhwc_to_nchw": [_TP, _i, _vp, _i, _i64, _i64, _i64, _i64, _vp],
     "ddpm_sinusoid": [_vp, _i, _i, _i, _vp, _i, _vp],
     "ddpm_gn_stats": [_TP, _i, _i, _vp, _vp],
-    "ddpm_gn_coeffs": [_TP, _i, _i, _vp, _vp, _f, _vp, _vp],
     "ddpm_gn_apply": [_TP, _i, _i, _vp, _vp, _vp, _f, _i, _f, _vp, _u32, _TP, _vp],
     "ddpm_gn_fwd": [_TP, _i, _i, _vp, _vp, _vp, _f, _i, _f, _vp, _u32, _TP, _vp],
     "ddpm_gn_bwd": [_TP, _i, _i, _vp, _vp, _vp, _f, _i, _f, _vp, _u32, _TP, _TP, _i, _vp, _vp, _vp, _vp],
@@ -94,7 +93,6 @@ SIGNATURES = {
     "ddpm_add": [_TP, _TP, _TP, _i, _vp],
     "ddpm_colsum": [_TP, _i, _vp, _vp, _vp],
     "ddpm_conv": [C.POINTER(ConvArgs), _vp],
-    "ddpm_conv_gn_fusable": [C.POINTER(ConvArgs)],
     "ddpm_conv_wgrad": [C.POINTER(WgradArgs), _vp],
     "ddpm_wgrad_workspace_bytes": [C.POINTER(WgradArgs)],
     "ddpm_pack_weights": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _vp],
@@ -113,7 +111,6 @@ SIGNATURES = {
     "ddpm_rng_advance": [_vp, _vp],
     "ddpm_set_force_simt": [_i],
     "ddpm_set_tc_mode": [_i, _i],
-    "ddpm_set_pdl": [_i],
     "ddpm_abi_struct_sizes": [_vp, _i],
 }
 

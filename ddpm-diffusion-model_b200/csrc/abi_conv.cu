@@ -13,12 +13,6 @@ static int g_force_simt = 0;
 extern "C" int ddpm_set_force_simt(int v) { g_force_simt = v; return 0; }
 int ddpm_force_simt_flag() { return g_force_simt; }
 
-extern "C" int ddpm_conv_gn_fusable(const ddpm_conv_args* a) {
-    if (!a || !a->gn_ab || !tensor_ok(&a->in) || !tensor_ok(&a->out) || !a->w) return 0;
-    if (a->in2.ptr && (!tensor_ok(&a->in2) || !a->w2 || a->in2.N != a->out.N || a->in2.H != a->out.H || a->in2.W != a->out.W)) return 0;
-    return (a->prefer_tc && !g_force_simt && a->mode == DDPM_CONV_NORMAL && !a->a_silu && conv_tc_supported(a)) ? 1 : 0;
-}
-
 extern "C" int ddpm_conv(const ddpm_conv_args* a, void* stream) {
     if (!a || !tensor_ok(&a->in) || !tensor_ok(&a->out) || !a->w) return DDPM_E_ARG;
     if (a->dtype != DDPM_F32 && a->dtype != DDPM_BF16) return DDPM_E_ARG;
@@ -40,10 +34,6 @@ extern "C" int ddpm_conv(const ddpm_conv_args* a, void* stream) {
     if (a->res.ptr && (!tensor_ok(&a->res) || a->res.C != a->out.C || a->res.H != a->out.H || a->res.W != a->out.W)) return DDPM_E_ARG;
     if (a->z.ptr && (!tensor_ok(&a->z) || a->z.C != a->out.C || a->z.H != a->out.H || a->z.W != a->out.W)) return DDPM_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
-    if (a->gn_ab) {                      // operand-path GroupNorm exists on the tcgen05 kernel only: never a silent unfused result
-        if (a->mode != DDPM_CONV_NORMAL || !ddpm_conv_gn_fusable(a)) return DDPM_E_ARG;
-        return conv_tc_launch(a, st);
-    }
     if (a->in2.ptr) {
         if (!tensor_ok(&a->in2) || !a->w2 || a->mode != DDPM_CONV_NORMAL || a->stride != 1 || a->a_silu) return DDPM_E_ARG;
         if (a->in2.N != a->out.N || a->in2.H != a->out.H || a->in2.W != a->out.W) return DDPM_E_ARG;

@@ -21,7 +21,6 @@ __device__ __forceinline__ T* tokw(const TV& v, int n, int p, int c) { int y = p
 
 template <typename T>
 __global__ void __launch_bounds__(AT) attn_fwd_kernel(TV qkv, TV out, int heads, int d, float scale, float* lse) {
-    pdl_enter();
     extern __shared__ float sm[];
     const int dp = d + 1;
     float* Ks = sm;                       // [KT][dp]
@@ -110,10 +109,10 @@ extern "C" int ddpm_attn_fwd(const ddpm_tensor* qkv, const ddpm_tensor* out, int
     float scale = 1.0f / sqrtf((float)d);
     if (dtype == DDPM_F32) {
         CUDA_TRY(cudaFuncSetAttribute(attn_fwd_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        CUDA_TRY(launch_pdl(attn_fwd_kernel<float>, grid, dim3(AT), smem, st, TV(*qkv), TV(*out), heads, d, scale, lse));
+        CUDA_TRY(launch_kernel(attn_fwd_kernel<float>, grid, dim3(AT), smem, st, TV(*qkv), TV(*out), heads, d, scale, lse));
     } else if (dtype == DDPM_BF16) {
         CUDA_TRY(cudaFuncSetAttribute(attn_fwd_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        CUDA_TRY(launch_pdl(attn_fwd_kernel<bf16>, grid, dim3(AT), smem, st, TV(*qkv), TV(*out), heads, d, scale, lse));
+        CUDA_TRY(launch_kernel(attn_fwd_kernel<bf16>, grid, dim3(AT), smem, st, TV(*qkv), TV(*out), heads, d, scale, lse));
     } else return DDPM_E_ARG;
     LAUNCH_OK();
     return 0;
@@ -126,7 +125,6 @@ extern "C" int ddpm_attn_fwd(const ddpm_tensor* qkv, const ddpm_tensor* out, int
 template <typename T>
 __global__ void __launch_bounds__(AT) attn_bwd_q_kernel(TV qkv, TV out, TV dout, TV dqkv, int heads, int d, float scale,
                                                         const float* lse, float* Pm, float* dSm) {
-    pdl_enter();
     extern __shared__ float sm[];
     const int dp = d + 1;
     float* Ks = sm; float* Vs = Ks + KT * dp;
@@ -218,7 +216,6 @@ __global__ void __launch_bounds__(AT) attn_bwd_q_kernel(TV qkv, TV out, TV dout,
 template <typename T>
 __global__ void __launch_bounds__(AT) attn_bwd_kv_kernel(TV qkv, TV dout, TV dqkv, int heads, int d, float scale,
                                                          const float* Pm, const float* dSm) {
-    pdl_enter();
     extern __shared__ float sm[];
     const int dp = d + 1;
     float* Qt = sm;                       // [KT queries][dp]
@@ -318,9 +315,9 @@ extern "C" int ddpm_attn_bwd(const ddpm_tensor* qkv, const ddpm_tensor* out, con
 #define GO(T) { \
         CUDA_TRY(cudaFuncSetAttribute(attn_bwd_q_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smq)); \
         CUDA_TRY(cudaFuncSetAttribute(attn_bwd_kv_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smk)); \
-        CUDA_TRY(launch_pdl(attn_bwd_q_kernel<T>, gq, dim3(AT), smq, st, TV(*qkv), TV(*out), TV(*dout), TV(*dqkv), heads, d, scale, (const float*)lse, Pm, dSm)); \
+        CUDA_TRY(launch_kernel(attn_bwd_q_kernel<T>, gq, dim3(AT), smq, st, TV(*qkv), TV(*out), TV(*dout), TV(*dqkv), heads, d, scale, (const float*)lse, Pm, dSm)); \
         LAUNCH_OK(); \
-        CUDA_TRY(launch_pdl(attn_bwd_kv_kernel<T>, gk, dim3(AT), smk, st, TV(*qkv), TV(*dout), TV(*dqkv), heads, d, scale, (const float*)Pm, (const float*)dSm)); \
+        CUDA_TRY(launch_kernel(attn_bwd_kv_kernel<T>, gk, dim3(AT), smk, st, TV(*qkv), TV(*dout), TV(*dqkv), heads, d, scale, (const float*)Pm, (const float*)dSm)); \
         LAUNCH_OK(); }
     if (dtype == DDPM_F32) GO(float) else if (dtype == DDPM_BF16) GO(bf16) else return DDPM_E_ARG;
 #undef GO

@@ -125,7 +125,6 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_fwd_tc_kernel(const __gri
     fence_after();
     const uint32_t tmem_base = *tmem_slot;
     const uint32_t o_col = 256u;
-    pdl_enter();
 
     if (warp == 0) {
         if (lane == 0) {
@@ -302,7 +301,6 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_bwd_dq_tc_kernel(const __
     __syncthreads();
     fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    pdl_enter();
     if (warp == 0) {
         if (lane == 0) {
             mb_expect(bar_in, (uint32_t)(p.kch * (2 * p.tok_t + 2 * p.N) * 32));
@@ -420,7 +418,6 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_bwd_dkv_tc_kernel(const _
     __syncthreads();
     fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    pdl_enter();
     if (warp == 0) {
         if (lane == 0) {
             mb_expect(bar_in, (uint32_t)(p.kch * (2 * p.tok_t + 2 * p.N) * 32));
@@ -558,7 +555,7 @@ int attn_tc_launch(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads, in
         configured = smem;
     }
     dim3 grid((p.N + p.tok_q - 1) / p.tok_q, heads, qkv->N);
-    CUDA_TRY(launch_pdl(attn_fwd_tc_kernel, grid, dim3(ATC_THREADS), smem, st, tmQ, tmK, tmV, p));
+    CUDA_TRY(launch_kernel(attn_fwd_tc_kernel, grid, dim3(ATC_THREADS), smem, st, tmQ, tmK, tmV, p));
     LAUNCH_OK();
     return 0;
 }
@@ -601,7 +598,7 @@ int attn_tc_bwd_launch(const ddpm_tensor* qkv, const ddpm_tensor* out, const ddp
         const size_t smem = (size_t)p.o5 + CH + 8 * 5 + 16 + 1024;
         static size_t configured = 0;
         if (smem > configured) { CUDA_TRY(cudaFuncSetAttribute(attn_bwd_dq_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); configured = smem; }
-        CUDA_TRY(launch_pdl(attn_bwd_dq_tc_kernel, grid, dim3(ATC_THREADS), smem, st, qT, gT, qF32, qF128, p));
+        CUDA_TRY(launch_kernel(attn_bwd_dq_tc_kernel, grid, dim3(ATC_THREADS), smem, st, qT, gT, qF32, qF128, p));
         LAUNCH_OK();
     }
     {   // dkv: K tile, V tile, Q32 -> Q128, dO32 -> dO128, P^T, dS^T
@@ -610,7 +607,7 @@ int attn_tc_bwd_launch(const ddpm_tensor* qkv, const ddpm_tensor* out, const ddp
         const size_t smem = (size_t)p.o5 + CH + 8 * 5 + 16 + 1024;
         static size_t configured = 0;
         if (smem > configured) { CUDA_TRY(cudaFuncSetAttribute(attn_bwd_dkv_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); configured = smem; }
-        CUDA_TRY(launch_pdl(attn_bwd_dkv_tc_kernel, grid, dim3(ATC_THREADS), smem, st, qT, qF32, gF32, qF128, gF128, p));
+        CUDA_TRY(launch_kernel(attn_bwd_dkv_tc_kernel, grid, dim3(ATC_THREADS), smem, st, qT, qF32, gF32, qF128, gF128, p));
         LAUNCH_OK();
     }
     return 0;

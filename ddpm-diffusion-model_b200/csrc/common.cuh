@@ -24,30 +24,10 @@ extern int64_t g_ddpm_launches;  // counted by LAUNCH_OK (host side, single-thre
 
 static inline int ceil_div(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 
-// ---- programmatic dependent launch (PDL) ----------------------------------------------------------------------
-// A step is ~300 short launches; with stream serialisation every launch pays the previous grid's drain plus its own
-// launch latency and prologue (barrier init, TMEM allocation, index math).  Kernels launched through launch_pdl()
-// may start while the previous kernel of the stream is still running; they must execute pdl_wait() before their
-// first access to global memory (it returns once every prerequisite grid has completed and flushed), and call
-// pdl_trigger() to let the NEXT kernel of the stream start its own prologue.  Every kernel that is ever launched
-// this way waits before it exits, so completion stays transitive along the stream.
-extern int g_ddpm_pdl;           // 0 (default since round 2; env DDPM_B200_PDL=1 or ddpm_set_pdl(1) turns it on)
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_enter() { pdl_wait(); pdl_trigger(); }
-static inline void pdl_attr(cudaLaunchAttribute* at, unsigned* n) {
-    if (!g_ddpm_pdl) return;
-    at[*n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[*n].val.programmaticStreamSerializationAllowed = 1;
-    ++*n;
-}
 template <typename... KA, typename... A>
-static inline cudaError_t launch_pdl(void (*kernel)(KA...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, A&&... args) {
+static inline cudaError_t launch_kernel(void (*kernel)(KA...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, A&&... args) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute at[1]; unsigned n = 0;
-    pdl_attr(at, &n);
-    cfg.attrs = at; cfg.numAttrs = n;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KA>(args)...);
 }
 

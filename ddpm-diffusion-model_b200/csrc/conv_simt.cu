@@ -27,7 +27,6 @@ struct ConvP {
 
 template <typename T>
 __global__ void __launch_bounds__(CT) conv_simt_kernel(ConvP p) {
-    pdl_enter();
     __shared__ float As[BK][BM + 4];
     __shared__ float Bs[BK][BN + 4];
     const int tid = threadIdx.x;
@@ -200,7 +199,6 @@ struct LinP {
     int M, N, K, xpitch, opitch, zpitch, a_silu, accum, bias_n, vec;
 };
 __global__ void __launch_bounds__(256) linear_small_kernel(LinP p) {
-    pdl_enter();
     __shared__ float As[2][LBK][LBM + 1];
     __shared__ float Bs[2][LBK][LBN + 1];
     const int tid = threadIdx.x;
@@ -273,7 +271,7 @@ static int linear_small_launch(const ddpm_conv_args* a, cudaStream_t st) {
     p.a_silu = a->a_silu; p.accum = (a->epi & DDPM_EPI_ACCUM) ? 1 : 0; p.bias_n = a->bias_n > 0 ? a->bias_n : a->out.C;
     p.vec = (p.K % 4 == 0) && (p.xpitch % 4 == 0) && al(p.x, 16) && al(p.w, 16);
     dim3 grid(ceil_div(p.M, LBM), ceil_div(p.N, LBN));
-    CUDA_TRY(launch_pdl(linear_small_kernel, grid, dim3(256), 0, st, p));
+    CUDA_TRY(launch_kernel(linear_small_kernel, grid, dim3(256), 0, st, p));
     LAUNCH_OK();
     return 0;
 }
@@ -313,7 +311,6 @@ __device__ __forceinline__ void tile_gemm32(FA fa, FB fb, int Kin, float acc[2][
 
 __global__ void __launch_bounds__(256) linear_grouped_fwd_kernel(const float* __restrict__ x, int M, int K, int xpitch,
                                                                  const ddpm_lin_entry* __restrict__ entries, float* out, int opitch, int a_silu) {
-    pdl_enter();
     __shared__ float As[LBK][LBM + 1];
     __shared__ float Bs[LBK][LBN + 1];
     const ddpm_lin_entry e = entries[blockIdx.z];
@@ -338,7 +335,7 @@ extern "C" int ddpm_linear_grouped_fwd(const float* x, int M, int K, int xpitch,
                                        int max_N, float* out, int out_pitch, int a_silu, void* stream) {
     if (!x || !entries_dev || !out || M <= 0 || K <= 0 || n <= 0 || max_N <= 0) return DDPM_E_ARG;
     dim3 grid(ceil_div(M, LBM), ceil_div(max_N, LBN), n);
-    CUDA_TRY(launch_pdl(linear_grouped_fwd_kernel, grid, dim3(256), 0, (cudaStream_t)stream, x, M, K, xpitch, entries_dev, out, out_pitch, a_silu));
+    CUDA_TRY(launch_kernel(linear_grouped_fwd_kernel, grid, dim3(256), 0, (cudaStream_t)stream, x, M, K, xpitch, entries_dev, out, out_pitch, a_silu));
     LAUNCH_OK();
     return 0;
 }
@@ -348,7 +345,6 @@ extern "C" int ddpm_linear_grouped_fwd(const float* x, int M, int K, int xpitch,
 __global__ void __launch_bounds__(256) time_proj_bwd_kernel(const float* __restrict__ temb, int B, int K, const float* __restrict__ dy,
                                                             int dpitch, int N, const float* __restrict__ w, float* dw, float* db,
                                                             float* dtemb, int accum, int tilesA_n) {
-    pdl_enter();
     __shared__ float As[LBK][LBM + 1];
     __shared__ float Bs[LBK][LBN + 1];
     const int kt = blockIdx.x, r = blockIdx.y;               // K tile; row tile of part A (n) or part B (b)
@@ -395,7 +391,7 @@ extern "C" int ddpm_time_proj_bwd(const float* temb, int B, int K, const float* 
     if (!temb || !dy || !w || !dw || !dtemb || B <= 0 || K <= 0 || N <= 0) return DDPM_E_ARG;
     const int tilesA = ceil_div(N, LBM), tilesB = ceil_div(B, LBM);
     dim3 grid(ceil_div(K, LBN), tilesA + tilesB);
-    CUDA_TRY(launch_pdl(time_proj_bwd_kernel, grid, dim3(256), 0, (cudaStream_t)stream, temb, B, K, dy, dy_pitch, N, w, dw, db, dtemb, accum_dtemb, tilesA));
+    CUDA_TRY(launch_kernel(time_proj_bwd_kernel, grid, dim3(256), 0, (cudaStream_t)stream, temb, B, K, dy, dy_pitch, N, w, dw, db, dtemb, accum_dtemb, tilesA));
     LAUNCH_OK();
     return 0;
 }
@@ -417,8 +413,8 @@ int conv_simt_launch(const ddpm_conv_args* a, cudaStream_t st) {
     p.vecB = (p.Kt % 4 == 0) && al(a->w, 4 * es);
     p.vecO = (a->out.pitch % 4 == 0) && al(a->out.ptr, 4 * es);
     dim3 grid(ceil_div(p.M, BM), ceil_div(p.Cout, BN));
-    if (a->dtype == DDPM_F32) CUDA_TRY(launch_pdl(conv_simt_kernel<float>, grid, dim3(CT), 0, st, p));
-    else CUDA_TRY(launch_pdl(conv_simt_kernel<bf16>, grid, dim3(CT), 0, st, p));
+    if (a->dtype == DDPM_F32) CUDA_TRY(launch_kernel(conv_simt_kernel<float>, grid, dim3(CT), 0, st, p));
+    else CUDA_TRY(launch_kernel(conv_simt_kernel<bf16>, grid, dim3(CT), 0, st, p));
     LAUNCH_OK();
     return 0;
 }
@@ -434,7 +430,6 @@ struct WgP {
 
 template <typename T>
 __global__ void __launch_bounds__(CT) wgrad_simt_kernel(WgP p) {
-    pdl_enter();
     __shared__ float Ys[BK][BM + 4];   // [q][co]
     __shared__ float Xs[BK][BN + 4];   // [q][kf]
     const int tid = threadIdx.x;
@@ -554,8 +549,8 @@ int wgrad_simt_launch(const ddpm_wgrad_args* a, cudaStream_t st) {
     p.qper = ceil_div(ceil_div(p.Q, splits), BK) * BK;
     splits = ceil_div(p.Q, p.qper);
     dim3 grid(ceil_div(p.Cout, BM), ceil_div(p.Kf, BN), splits);
-    if (a->dtype == DDPM_F32) CUDA_TRY(launch_pdl(wgrad_simt_kernel<float>, grid, dim3(CT), 0, st, p));
-    else CUDA_TRY(launch_pdl(wgrad_simt_kernel<bf16>, grid, dim3(CT), 0, st, p));
+    if (a->dtype == DDPM_F32) CUDA_TRY(launch_kernel(wgrad_simt_kernel<float>, grid, dim3(CT), 0, st, p));
+    else CUDA_TRY(launch_kernel(wgrad_simt_kernel<bf16>, grid, dim3(CT), 0, st, p));
     LAUNCH_OK();
     return 0;
 }

@@ -162,10 +162,6 @@ int conv_tc_supported(const ddpm_conv_args* a) {
     if (a->res.ptr && (a->res.halo != 1 || a->res.pitch % 8 || ((uintptr_t)a->res.ptr & 15))) return 0;
     if (pick_nt(out.C) == 0) return 0;
     if (in.W + 2 > 300) return 0;         // patch would not fit the A ring (large images: later round)
-    if (a->gn_ab) {                       // GroupNorm (+SiLU) on the input operand: persistent pair kernel, stride-1 3x3 / 1x1 only
-        if (up || a->stride != 1 || (a->epi & DDPM_EPI_DSILU)) return 0;
-        if (((uintptr_t)a->gn_ab & 15) || a->gn_act < 0 || a->gn_act > 1) return 0;
-    }
     if (a->in2.ptr) {                     // fused 1x1 second operand: persistent pair kernel, 3x3 stride-1 main conv only
         const ddpm_tensor& i2 = a->in2;
         if (a->KH != 3 || a->stride != 1 || (a->epi & DDPM_EPI_DSILU)) return 0;
@@ -212,25 +208,6 @@ __device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
     // to drain (ncu: MEMBAR + ERRBAR = 16 % of the stall samples) for no reason
     asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
 }
-__device__ __forceinline__ void mbar_arrive_xform(uint32_t cluster_addr) {
-    // "this warp's rewrite of its patch rows is done".  The rows live in the arriving CTA's OWN shared memory and are read by
-    // that SM's tensor core; each writer has already executed fence.proxy.async, so the data is in place before the signal
-    // leaves.  A release at cluster scope here compiled to MEMBAR.ALL.GPU + ERRBAR + CGAERRBAR per arrive (and the matching
-    // acquire.cluster wait to CCTL.IVALL in the MMA-issue loop): ncu had the kernel at 3x the unfused time with those.
-    asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ uint32_t lds32u(uint32_t a) {
-    uint32_t v; asm volatile("ld.shared.b32 %0, [%1];" : "=r"(v) : "r"(a)); return v;
-}
-__device__ __forceinline__ void sts32u(uint32_t a, uint32_t v) { asm volatile("st.shared.b32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
-__device__ __forceinline__ uint4 lds128u(uint32_t a) {
-    uint4 v;
-    asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a));
-    return v;
-}
-__device__ __forceinline__ void sts128u(uint32_t a, const uint4& v) {
-    asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(a), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
 __device__ __forceinline__ void tma2_load_2d(void* dst, const CUtensorMap* m, uint32_t bar_cluster_addr, int c0, int c1) {
     asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
                  ::"r"(smem_u32(dst)), "l"(m), "r"(bar_cluster_addr), "r"(c0), "r"(c1) : "memory");
@@ -271,63 +248,6 @@ __device__ __forceinline__ void stg256(void* p, const uint4& lo, const uint4& hi
                  ::"l"(p), "r"(lo.x), "r"(lo.y), "r"(lo.z), "r"(lo.w), "r"(hi.x), "r"(hi.y), "r"(hi.z), "r"(hi.w) : "memory");
 }
 
-// ---- GroupNorm (+SiLU) operand transform of one staged K-chunk (conv_tc2_kernel GNA, warps 10..13) ------------------------
-// A transform warp runs alone on its scheduler, so throughput is ILP: the first version (one packet at a time, a
-// "coefficients changed?" branch per packet) issued one instruction per ~8 cycles and made the convolution 2.3x slower
-// (ncu: stall_wait everywhere, tensor pipe 25 %).  Here NB packets are in flight per thread and the body is branch-free
-// (skip rows are computed and not stored), so the 8 x NB element chains interleave; the floor is the MUFU: 8 tanh per
-// packet = 64 issue cycles per warp.
-__device__ __forceinline__ void gn_ld8(uint32_t a, float* v) {
-    const uint4 x = lds128u(a), y = lds128u(a + 16);
-    v[0] = __uint_as_float(x.x); v[1] = __uint_as_float(x.y); v[2] = __uint_as_float(x.z); v[3] = __uint_as_float(x.w);
-    v[4] = __uint_as_float(y.x); v[5] = __uint_as_float(y.y); v[6] = __uint_as_float(y.z); v[7] = __uint_as_float(y.w);
-}
-template <bool ACT>
-__device__ __forceinline__ uint4 gn_xform_packet(const uint4& q, const float* ca, const float* cb) {
-    uint32_t w[4] = {q.x, q.y, q.z, q.w};
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        float lo = fmaf(__uint_as_float(w[i] << 16), ca[2 * i], cb[2 * i]);
-        float hi = fmaf(__uint_as_float(w[i] & 0xffff0000u), ca[2 * i + 1], cb[2 * i + 1]);
-        if (ACT) { lo = silu_half(lo); hi = silu_half(hi); }
-        const __nv_bfloat162 h2 = __floats2bfloat162_rn(lo, hi);
-        w[i] = *reinterpret_cast<const uint32_t*>(&h2);
-    }
-    return make_uint4(w[0], w[1], w[2], w[3]);
-}
-// abase: the chunk in shared memory; mt_u: row map; tabc: coefficient table + this thread's channel offset; cin4 = Cin * 4
-template <bool ACT, bool SINGLE>
-__device__ __forceinline__ void gn_xform_chunk(uint32_t abase, uint32_t mt_u, uint32_t tabc, uint32_t cin4, int tt, int npk) {
-    constexpr int NB = SINGLE ? 4 : 2;
-    float ca[8], cb[8];
-    if (SINGLE) { gn_ld8(tabc, ca); gn_ld8(tabc + cin4, cb); }
-#pragma unroll 1
-    for (int pk0 = tt; pk0 < npk; pk0 += 128 * NB) {
-        uint32_t m[NB]; uint4 q[NB];
-        float la[SINGLE ? 1 : NB][8], lb[SINGLE ? 1 : NB][8];
-#pragma unroll
-        for (int b = 0; b < NB; ++b) {
-            const int pk = pk0 + 128 * b;
-            const int pkc = pk < npk ? pk : tt;                  // out of range: load something valid, store nothing
-            m[b] = lds32u(mt_u + (uint32_t)(pkc >> 1) * 4u);
-            if (pk >= npk) m[b] = 0xFFFFFFFFu;
-            q[b] = lds128u(abase + (uint32_t)pkc * 16u);
-        }
-        if (!SINGLE) {
-#pragma unroll
-            for (int b = 0; b < NB; ++b) {
-                const uint32_t t = tabc + (m[b] == 0xFFFFFFFFu ? 0u : m[b]);
-                gn_ld8(t, la[b]); gn_ld8(t + cin4, lb[b]);
-            }
-        }
-#pragma unroll
-        for (int b = 0; b < NB; ++b) {
-            const uint4 o = SINGLE ? gn_xform_packet<ACT>(q[b], ca, cb) : gn_xform_packet<ACT>(q[b], la[b], lb[b]);
-            if (m[b] != 0xFFFFFFFFu) sts128u(abase + (uint32_t)(pk0 + 128 * b) * 16u, o);
-        }
-    }
-}
-
 struct Tc2Params {
     TV out, res;
     const float* bias; const float* tbias; int tbias_pitch; int bias_n;
@@ -349,29 +269,16 @@ struct Tc2Params {
     int KCH2;                     // K-chunks of the fused 1x1 second operand (0: none): they follow the 3x3 chunks of every
     int b2_chunk_bytes;           //    item, load their patch through tmA2 / their one-tap weight slab through tmB2 and
                                   //    issue only the centre tap
-    const float* gn_ab;           // GNA kernels: fp32 [N][2][Cin] GroupNorm affine of the input operand (ddpm_conv_args.gn_ab)
-    int gn_act;                   //    1: SiLU after the affine
-    int gn_nimg;                  //    images a CTA's patch can span (rows of the shared-memory coefficient table)
 };
 
 // FUSED2: the 1x1 second operand (ddpm_conv_args.in2).  A template parameter, not a run-time branch: the extra stage kind
 // in the producer and MMA-issue loops cost 3-4 % on EVERY convolution when it was one (A/B of three builds on one box,
 // 96->96@64: 67.9 -> 70.0 us) -- the issue loop is that tight.
-//
-// GNA: GroupNorm (+SiLU) of the INPUT operand inside the convolution (north_star (1): "GroupNorm+SiLU ... fused into the
-// prologue"; attention.py:38-39,61, unet_backbone.py:37-38,43-44,215).  Four more warps (10..13) sit between the TMA producer
-// and the MMA issuer: a stage's activation patch lands on the CTA's own afull[s]; the transform warps rewrite it in place
-// as act(a[n][c] * x + b[n][c]) -- ONCE per K-chunk, because all nine taps of the shift-GEMM read the same staged patch --
-// leave halo / out-of-tensor rows at zero (SiLU(b) != 0: the reference zero-pads the ACTIVATED tensor), make the writes
-// visible to the tensor core's async proxy and arrive on the leader's xfull[s]; the issuer waits for xfull[s] (both CTAs'
-// patches transformed) and full[s] (weights).  Per item the warps stage the coefficient rows of the <= gn_nimg images the
-// patch touches and a row map (table offset, or "skip") in shared memory.  Stages of the fused 1x1 second operand (the
-// block input of conv2 + skip) pass through untransformed.
-template <int MT, int TAPS, bool FUSED2, bool GNA>
-__global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv_tc2_kernel(const __grid_constant__ CUtensorMap tmA,
-                                                                    const __grid_constant__ CUtensorMap tmB,
-                                                                    const __grid_constant__ CUtensorMap tmA2,
-                                                                    const __grid_constant__ CUtensorMap tmB2, Tc2Params p) {
+template <int MT, int TAPS, bool FUSED2>
+__global__ void __launch_bounds__(TC2_THREADS, 1) conv_tc2_kernel(const __grid_constant__ CUtensorMap tmA,
+                                                                  const __grid_constant__ CUtensorMap tmB,
+                                                                  const __grid_constant__ CUtensorMap tmA2,
+                                                                  const __grid_constant__ CUtensorMap tmB2, Tc2Params p) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
     uint8_t* ring = smem;
@@ -379,11 +286,8 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
     uint64_t* bars = (uint64_t*)(bres + (p.b_res ? (size_t)(p.Cin / KC) * p.b_chunk_bytes + (FUSED2 ? (size_t)p.KCH2 * p.b2_chunk_bytes : 0) : 0));
     uint64_t* full = bars;            uint64_t* empty = full + p.S;
     uint64_t* tfull = empty + p.S;    uint64_t* tempty = tfull + 2;
-    uint64_t* afull = tempty + 2;     uint64_t* xfull = afull + (GNA ? p.S : 0);        // GNA only
-    uint32_t* tmem_slot = (uint32_t*)(xfull + (GNA ? p.S : 0));
+    uint32_t* tmem_slot = (uint32_t*)(tempty + 2);
     float* sbias = (float*)(tmem_slot + 4);              // [Cout] bias staged once per CTA (16-byte aligned: the barrier block is)
-    float* gtab = sbias + ((p.Cout + 3) & ~3);           // GNA: [2 buffers][gn_nimg][2][Cin] coefficients of an item's images
-    // GNA: behind the two table buffers, [2][P] row maps (table byte offset of a patch row, ~0u: leave the row as it is)
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t rank = cluster_ctarank();
@@ -406,7 +310,6 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
         }
         for (int i = 0; i < p.S; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
         for (int b = 0; b < 2; ++b) { mbar_init(&tfull[b], 1); mbar_init(&tempty[b], 16); }
-        if (GNA) for (int i = 0; i < p.S; ++i) { mbar_init(&afull[i], 1); mbar_init(&xfull[i], 8); }   // 4 transform warps x 2 CTAs
         fence_barrier_init();
     }
     if (warp == 1) tmem_alloc2(tmem_slot, 512u);
@@ -415,7 +318,6 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
     cluster_sync_all();                                  // peer's barriers are initialised before anyone signals them
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    pdl_enter();                                         // everything above overlapped the previous kernel's tail
     // The bias vector is read by every epilogue trip; as __ldg float4 loads after the accumulator wait it cost ~25 % of the
     // epilogue at 96 channels (measured when the time bias absorbed conv1's bias).  Stage it in shared memory once.
     if (p.bias && warp >= 2 && warp < 10) {
@@ -439,10 +341,8 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
                     const uint32_t fbar = mapa_u32(smem_u32(&full[s]), 0);
                     const bool loadB = !(p.b_res && it != pair);                 // resident weights arrive with the first item only
                     const int bbytes = second ? p.b2_chunk_bytes : p.b_chunk_bytes;
-                    // GNA: the patch lands on this CTA's own afull[s] (the transform warps wait there); full[s] counts weights only
-                    const uint32_t tx = (uint32_t)(2 * nk * ((GNA ? 0 : p.P * 32) + (loadB ? bbytes : 0)));
-                    if (leader) { if (tx) mbar_expect_tx(&full[s], tx); else mbar_arrive(&full[s]); }
-                    if (GNA) mbar_expect_tx(&afull[s], (uint32_t)(nk * p.P * 32));
+                    const uint32_t tx = (uint32_t)(2 * nk * (p.P * 32 + (loadB ? bbytes : 0)));
+                    if (leader) mbar_expect_tx(&full[s], tx);
                     uint8_t* sbase = ring + (size_t)s * p.stage_bytes;
                     const CUtensorMap* mA = second ? &tmA2 : &tmA;
                     const CUtensorMap* mB = second ? &tmB2 : &tmB;
@@ -452,12 +352,8 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
                                       : (second ? bres + (size_t)KCH * p.b_chunk_bytes + (size_t)kc0 * p.b2_chunk_bytes
                                                 : bres + (size_t)(kc0 + k) * p.b_chunk_bytes);
                         const int row0 = Q0 - halo_rows;
-                        if (GNA) {
-                            for (int r = 0; r < p.P; r += p.seg) tma_load_2d(adst + (size_t)r * 32, mA, &afull[s], (kc0 + k) * KC, row0 + r);
-                        } else {
-                            for (int r = 0; r < p.P; r += p.seg)
-                                tma2_load_2d(adst + (size_t)r * 32, mA, fbar, (kc0 + k) * KC, row0 + r);
-                        }
+                        for (int r = 0; r < p.P; r += p.seg)
+                            tma2_load_2d(adst + (size_t)r * 32, mA, fbar, (kc0 + k) * KC, row0 + r);
                         if (loadB) tma2_load_3d(bdst, mB, fbar, (kc0 + k) * KC, nrow0, 0);
                     }
                 }
@@ -490,7 +386,6 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
                 for (int st = 0; st < NST; ++st, ++g) {
                     const uint32_t s = g % (uint32_t)p.S; const uint32_t ph = (g / (uint32_t)p.S) & 1;
                     mbar_wait(&full[s], ph);
-                    if (GNA) mbar_wait(&xfull[s], ph);                  // both CTAs' patches transformed
                     tc_fence_after();
                     uint32_t a_lo = ring_lo + s * stage16;
                     if (FUSED2 && st >= NST - KCH2) {
@@ -528,89 +423,6 @@ __global__ void __launch_bounds__(GNA ? TC2_THREADS + 128 : TC2_THREADS, 1) conv
                 __syncwarp();
             }
         }
-    } else if (GNA && warp >= 10) {
-        // ===================================================================== operand transform (both CTAs)
-        // Thread tt owns the 16-byte packets pk = tt + 128 j of a patch (row pk >> 1): conflict-free LDS/STS.128, and
-        // because rows advance by 64 per j the SWIZZLE_32B chunk bit (row >> 2) & 1 -- hence the eight channels a thread
-        // works on -- is the same for all of its packets, so its coefficients stay in registers across a stage.
-        // The coefficient table and the row map are double buffered: item i+1's are prepared (cp.async for the table) while
-        // item i is being transformed, so one named barrier per item is the only per-item serialisation.
-        const int tt = threadIdx.x - TC2_THREADS;
-        const int HpWp = p.Hp * p.Wp;
-        const int lc8 = ((tt & 1) ^ ((tt >> 3) & 1)) << 3;
-        const uint32_t xbar0 = mapa_u32(smem_u32(&xfull[0]), 0);
-        const int C2 = 2 * p.Cin;
-        // explicit ld/st.shared below: through generic pointers the compiler emitted LD.E / ST.E (address space lost)
-        const uint32_t ring_u = smem_u32(ring);
-        const uint32_t tab_bytes = (uint32_t)(p.gn_nimg * C2 * 4), meta_bytes = (uint32_t)(p.P * 4);
-        const uint32_t gtab_u = smem_u32(gtab), meta_u = gtab_u + 2u * tab_bytes;
-        const uint32_t chunk_stride = (uint32_t)(p.a_chunk_bytes + (p.b_res ? 0 : p.b_chunk_bytes));
-        const uint32_t flag_u = meta_u + 2u * meta_bytes;      // [2] "the item's patch lies inside one image"
-        auto prepare = [&](int it, uint32_t buf) {          // coefficient rows + row map of item `it` into buffer `buf`
-            const int pt = it / p.n_tiles;
-            const int row0 = pt * (2 * tile_rows) + (int)rank * tile_rows - halo_rows;
-            const int qa = max(row0, 0), qb = min(row0 + p.P, p.Qtot) - 1;
-            const int n_first = qa / HpWp;
-            int nimg = 0;
-            if (qb >= qa) {
-                nimg = qb / HpWp - n_first + 1;
-                const float* src = p.gn_ab + (size_t)n_first * C2;
-                const uint32_t dst = gtab_u + buf * tab_bytes;
-                for (int i = tt; i < nimg * (C2 >> 2); i += 128)
-                    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst + (uint32_t)i * 16u), "l"(src + 4 * i) : "memory");
-            }
-            asm volatile("cp.async.commit_group;" ::: "memory");
-            if (tt == 0) sts32u(flag_u + buf * 4u, nimg <= 1 ? 1u : 0u);
-            for (int r = tt; r < p.P; r += 128) {
-                const int Q = row0 + r;
-                uint32_t m = 0xFFFFFFFFu;
-                if (Q >= 0 && Q < p.Qtot) {
-                    const int n = Q / HpWp, rem = Q - n * HpWp, yp = rem / p.Wp, xp = rem - yp * p.Wp;
-                    if (yp >= 1 && yp <= p.H && xp >= 1 && xp <= p.W) m = (uint32_t)((n - n_first) * C2 * 4);
-                }
-                sts32u(meta_u + buf * meta_bytes + (uint32_t)r * 4u, m);
-            }
-            return nimg;
-        };
-        uint32_t g = 0, j = 0;
-        int nimg_cur = 0, nimg_next = 0;
-        if (pair < p.items) nimg_next = prepare(pair, 0u);
-        for (int it = pair; it < p.items; it += npairs, ++j) {
-            const uint32_t buf = j & 1;
-            nimg_cur = nimg_next;
-            asm volatile("cp.async.wait_all;" ::: "memory");
-            if (p.gn_act) {                                      // SiLU through tanh: the affine produces z / 2 -- halve the rows this thread copied
-                const uint32_t dst = gtab_u + buf * tab_bytes;
-                for (int i = tt; i < nimg_cur * (C2 >> 2); i += 128) {
-                    uint4 v = lds128u(dst + (uint32_t)i * 16u);
-                    v.x = __float_as_uint(0.5f * __uint_as_float(v.x)); v.y = __float_as_uint(0.5f * __uint_as_float(v.y));
-                    v.z = __float_as_uint(0.5f * __uint_as_float(v.z)); v.w = __float_as_uint(0.5f * __uint_as_float(v.w));
-                    sts128u(dst + (uint32_t)i * 16u, v);
-                }
-            }
-            asm volatile("bar.sync 2, 128;" ::: "memory");       // item `it`'s table / row map complete; the other buffer is free
-            if (it + npairs < p.items) nimg_next = prepare(it + npairs, buf ^ 1u);
-            const uint32_t tab_u = gtab_u + buf * tab_bytes, mt_u = meta_u + buf * meta_bytes;
-            const bool single = lds32u(flag_u + buf * 4u) != 0u;
-            for (int st = 0; st < NST; ++st, ++g) {
-                const uint32_t s = g % (uint32_t)p.S; const uint32_t ph = (g / (uint32_t)p.S) & 1;
-                mbar_wait(&afull[s], ph);
-                if (!(FUSED2 && st >= NST - KCH2)) {
-                    const int kc0 = st * p.KS, nk = min(p.KS, KCH - kc0);
-                    for (int k = 0; k < nk; ++k) {
-                        const uint32_t abase = ring_u + s * (uint32_t)p.stage_bytes + (uint32_t)k * chunk_stride;
-                        const uint32_t tabc = tab_u + (uint32_t)(((kc0 + k) * KC + lc8) * 4);
-                        const uint32_t cin4 = (uint32_t)p.Cin * 4u;
-                        if (p.gn_act) { if (single) gn_xform_chunk<true, true>(abase, mt_u, tabc, cin4, tt, 2 * p.P); else gn_xform_chunk<true, false>(abase, mt_u, tabc, cin4, tt, 2 * p.P); }
-                        else { if (single) gn_xform_chunk<false, true>(abase, mt_u, tabc, cin4, tt, 2 * p.P); else gn_xform_chunk<false, false>(abase, mt_u, tabc, cin4, tt, 2 * p.P); }
-                    }
-                }
-                fence_proxy_async();                      // generic-proxy writes -> visible to the tensor core (async proxy)
-                __syncwarp();
-                if (lane == 0) mbar_arrive_xform(xbar0 + s * 8u);
-            }
-        }
-        asm volatile("cp.async.wait_all;" ::: "memory");
     } else {
         // ===================================================================== epilogue (both CTAs)
         const int qd = warp & 3;                          // TMEM lane quarter this warp may read (warp id % 4)
@@ -791,13 +603,7 @@ int conv_tc_launch(const ddpm_conv_args* a, cudaStream_t st) {
     p.KS = p.taps > 1 ? 1 : (KCH < 4 ? KCH : 4);
     p.KCH2 = a->in2.ptr ? a->in2.C / KC : 0;                // fused 1x1 second operand (3x3 main conv only: KS == 1)
     p.b2_chunk_bytes = (p.NT / 2) * 32;
-    p.gn_ab = a->gn_ab; p.gn_act = a->gn_act; p.gn_nimg = 0;
-    size_t gn_bytes = 0;
-    if (p.gn_ab) {
-        p.gn_nimg = (p.P + p.Hp * p.Wp - 2) / (p.Hp * p.Wp) + 1;
-        gn_bytes = 2 * ((size_t)p.gn_nimg * 2 * p.Cin * 4 + (size_t)p.P * 4) + 16 + 8 * 2 * 12;   // 2 x (table + row map) + flags + afull / xfull
-    }
-    const int budget = 212 * 1024 - (int)((gn_bytes + 1023) & ~(size_t)1023);
+    const int budget = 212 * 1024;
     p.pix_tiles = ceil_div(p.Qtot, 256 * MT);
     p.items = p.pix_tiles * p.n_tiles;
     int pairs = sm_count() / 2; if (pairs > p.items) pairs = p.items; if (pairs < 1) pairs = 1;
@@ -818,7 +624,7 @@ int conv_tc_launch(const ddpm_conv_args* a, cudaStream_t st) {
     }
     if (p.S < 2) return DDPM_E_ARG;
     size_t smem = (size_t)p.S * p.stage_bytes + (p.b_res ? (size_t)KCH * p.b_chunk_bytes + (size_t)p.KCH2 * p.b2_chunk_bytes : 0) +
-                  8 * (2 * p.S + 4) + 16 + (size_t)p.Cout * 4 + 1024 + gn_bytes + 16;
+                  8 * (2 * p.S + 4) + 16 + (size_t)p.Cout * 4 + 1024 + 16;
 
     CUtensorMap tmA, tmB, tmA2, tmB2;
     if (p.KCH2) {
@@ -842,25 +648,19 @@ int conv_tc_launch(const ddpm_conv_args* a, cudaStream_t st) {
         if (encode(&tmB, (void*)a->w, 3, db, sb, bb, CU_TENSOR_MAP_SWIZZLE_32B)) return 1;
     }
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(2 * pairs); cfg.blockDim = dim3(p.gn_ab ? TC2_THREADS + 128 : TC2_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute at[2]; unsigned nat = 1;
+    cfg.gridDim = dim3(2 * pairs); cfg.blockDim = dim3(TC2_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
+    cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    pdl_attr(at, &nat);
-    cfg.attrs = at; cfg.numAttrs = nat;
-    static size_t configured[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-#define TC2_GO(MTV, TAPSV, F2, GN, SLOT) { \
-        if (smem > configured[SLOT]) { CUDA_TRY(cudaFuncSetAttribute(conv_tc2_kernel<MTV, TAPSV, F2, GN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); configured[SLOT] = smem; } \
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, conv_tc2_kernel<MTV, TAPSV, F2, GN>, tmA, tmB, F2 ? tmA2 : tmA, F2 ? tmB2 : tmB, p)); }
-    if (p.gn_ab) {
-        if (p.KCH2) { if (MT == 2) TC2_GO(2, 9, true, true, 8) else TC2_GO(1, 9, true, true, 9) }
-        else if (MT == 2) { if (p.taps == 9) TC2_GO(2, 9, false, true, 10) else TC2_GO(2, 1, false, true, 11) }
-        else { if (p.taps == 9) TC2_GO(1, 9, false, true, 12) else TC2_GO(1, 1, false, true, 13) }
-    }
-    else if (p.KCH2) { if (MT == 2) TC2_GO(2, 9, true, false, 4) else TC2_GO(1, 9, true, false, 5) }
-    else if (p.taps == 4) { if (MT == 2) TC2_GO(2, 4, false, false, 6) else TC2_GO(1, 4, false, false, 7) }
-    else if (MT == 2) { if (p.taps == 9) TC2_GO(2, 9, false, false, 0) else TC2_GO(2, 1, false, false, 1) }
-    else { if (p.taps == 9) TC2_GO(1, 9, false, false, 2) else TC2_GO(1, 1, false, false, 3) }
+    cfg.attrs = at; cfg.numAttrs = 1;
+    static size_t configured[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+#define TC2_GO(MTV, TAPSV, F2, SLOT) { \
+        if (smem > configured[SLOT]) { CUDA_TRY(cudaFuncSetAttribute(conv_tc2_kernel<MTV, TAPSV, F2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); configured[SLOT] = smem; } \
+        CUDA_TRY(cudaLaunchKernelEx(&cfg, conv_tc2_kernel<MTV, TAPSV, F2>, tmA, tmB, F2 ? tmA2 : tmA, F2 ? tmB2 : tmB, p)); }
+    if (p.KCH2) { if (MT == 2) TC2_GO(2, 9, true, 4) else TC2_GO(1, 9, true, 5) }
+    else if (p.taps == 4) { if (MT == 2) TC2_GO(2, 4, false, 6) else TC2_GO(1, 4, false, 7) }
+    else if (MT == 2) { if (p.taps == 9) TC2_GO(2, 9, false, 0) else TC2_GO(2, 1, false, 1) }
+    else { if (p.taps == 9) TC2_GO(1, 9, false, 2) else TC2_GO(1, 1, false, 3) }
 #undef TC2_GO
     LAUNCH_OK();
     return 0;
@@ -939,7 +739,6 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc_kernel(const __grid_const
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     const uint32_t bias_col = (uint32_t)(p.ntap * p.NT);
-    pdl_enter();
 
     if (warp == 0) {
         if (lane == 0) {
@@ -1095,7 +894,6 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc2_kernel(const __grid_cons
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     const uint32_t bias_col = (uint32_t)(p.ntap * p.NT);
-    pdl_enter();
 
     if (warp == 0) {
         // ===================================================================== TMA producer (both CTAs)
@@ -1198,7 +996,6 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc2_kernel(const __grid_cons
 
 // dw[co][ci][ky][kx] += sum_split ws[split][mtile][ky*n_tiles+ntile][co%128][kx*NT + ci%NT]
 __global__ void wgrad_reduce_kernel(const float* __restrict__ ws, float* __restrict__ dw, int splits, WgTcParams p) {
-    pdl_enter();
     const int gtid = blockIdx.x * blockDim.x + threadIdx.x, gthreads = gridDim.x * blockDim.x;
     const int taps = p.ntap * p.ntap;
     const int total = p.CoutV * taps * p.CinV;
@@ -1249,9 +1046,7 @@ static int wg_pick_nt(int Cin) {
 
 static int wg_pair(const WgTcParams& p) {
     // the pair kernel: an even number of 128-row output-channel tiles (Cout in (128,256], (384,512], ...); ddpm_set_tc_mode
-    // flag 1024 turns it off (A/B against the single-CTA kernel).  It is never given the programmatic-dependent-launch
-    // attribute: launched that way on the MAIN stream it dead-locked the GPU in 4 of 10 CelebA256 bench runs (0 of 6 without
-    // the attribute, 0 of 4 with the single-CTA kernel; mechanism not found -- DESIGN.md section 6.2).
+    // flag 1024 turns it off (A/B against the single-CTA kernel).
     if (g_tc_exp & 1024) return 0;
     // Measured (profiles/r2_kbench_wgrad_pair_vs_single.txt): -9 % on the large Cout = 192 layers, +5 % on 384->192 @ 16 / 8
     // (four ci tiles x few pixels: the halved split count costs more than the smaller patch saves) -> small problems with
@@ -1328,7 +1123,7 @@ int wgrad_tc_launch(const ddpm_wgrad_args* a, cudaStream_t st) {
         }
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3(p.m_tiles, p.ntap * p.n_tiles, splits); cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = smem2; cfg.stream = st;
-        cudaLaunchAttribute at[1];                    // no PDL attribute: see wg_pair()
+        cudaLaunchAttribute at[1];
         at[0].id = cudaLaunchAttributeClusterDimension;
         at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
         cfg.attrs = at; cfg.numAttrs = 1;
@@ -1340,12 +1135,12 @@ int wgrad_tc_launch(const ddpm_wgrad_args* a, cudaStream_t st) {
             CUDA_TRY(cudaFuncSetAttribute(wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             configured = smem;
         }
-        CUDA_TRY(launch_pdl(wgrad_tc_kernel, dim3(splits, p.ntap * p.n_tiles, p.m_tiles), dim3(TC_THREADS), smem, st, tmY, tmA, p));
+        CUDA_TRY(launch_kernel(wgrad_tc_kernel, dim3(splits, p.ntap * p.n_tiles, p.m_tiles), dim3(TC_THREADS), smem, st, tmY, tmA, p));
     }
     LAUNCH_OK();
     int total = p.CoutV * p.ntap * p.ntap * p.CinV;
     int rg = (total + 255) / 256; if (rg > 148 * 8) rg = 148 * 8;
-    CUDA_TRY(launch_pdl(wgrad_reduce_kernel, dim3(rg), dim3(256), 0, st, (const float*)p.ws, a->dw, splits, p));
+    CUDA_TRY(launch_kernel(wgrad_reduce_kernel, dim3(rg), dim3(256), 0, st, (const float*)p.ws, a->dw, splits, p));
     LAUNCH_OK();
     return 0;
 }

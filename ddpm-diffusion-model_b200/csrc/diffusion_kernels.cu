@@ -6,18 +6,10 @@
 //
 // HBM roofline (fp32 tensors): q_sample 12 B/elem, MSE 8 (6 with bf16 pred), DDPM step 16,
 // DDIM step 12 (eta=0) / 16, to_image01 8.
-#include <stdlib.h>
 #include "common.cuh"
 #include <math.h>
 
 int64_t g_ddpm_launches = 0;
-// Programmatic dependent launch is OFF by default since round 2 (DDPM_B200_PDL=1 / ddpm_set_pdl(1) turn it on): measured in one
-// call it is neutral at 64 px (12.10 vs 12.12 ms per train step, DDIM-100 390 vs 392 samples/s) and COSTS 5 % of the CelebA256
-// train step (445 vs 467 img/s) and 25 % of a 256-px sampler evaluation (15.1 vs 12.1 ms) -- early-launched dependents sit on SM
-// resources next to the long-running kernels -- and with it the opt-in pair wgrad kernel dead-locked (DESIGN.md 4.4).
-static int pdl_default() { const char* e = getenv("DDPM_B200_PDL"); return (e && e[0] == '1') ? 1 : 0; }
-int g_ddpm_pdl = pdl_default();
-extern "C" int ddpm_set_pdl(int on) { g_ddpm_pdl = on ? 1 : 0; return 0; }
 extern "C" int ddpm_abi_struct_sizes(int32_t* out, int n) {
     const int32_t v[6] = {(int32_t)sizeof(ddpm_tensor), (int32_t)sizeof(ddpm_conv_args), (int32_t)sizeof(ddpm_lin_entry),
                           (int32_t)sizeof(ddpm_wgrad_args), (int32_t)sizeof(ddpm_pack_entry), (int32_t)sizeof(ddpm_adam_hyper)};
@@ -39,7 +31,7 @@ struct Schedule {
 static uint64_t g_next_id = 1;
 static uint64_t g_const_owner[64] = {0};
 
-extern "C" int ddpm_abi_version(void) { return 1; }
+extern "C" int ddpm_abi_version(void) { return 2; }
 
 extern "C" int ddpm_num_sms(int device, int* out) {
     if (!out) return DDPM_E_ARG;
@@ -463,7 +455,6 @@ extern "C" int ddpm_to_image01(const float* x, float* out, int64_t n, void* stre
 // narrow().copy_() launch per image plus four elementwise passes and a permute before the D2H copy.
 __global__ void image_grid_kernel(const float* __restrict__ x, int N, int C, int H, int W, int xmaps, int pad, int Hg, int Wg,
                                   float* __restrict__ gf, uint8_t* __restrict__ gu) {
-    pdl_enter();
     const int64_t total = (int64_t)Hg * Wg;
     const int ch = H + pad, cw = W + pad;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
@@ -493,7 +484,7 @@ extern "C" int ddpm_image_grid(const float* x01, int N, int C, int H, int W, int
     const int Hg = N == 1 ? H : (H + pad) * ymaps + pad, Wg = N == 1 ? W : (W + pad) * xmaps + pad;
     const int64_t total = (int64_t)Hg * Wg;
     int grid = (int)((total + 255) / 256); if (grid > 148 * 8) grid = 148 * 8;
-    CUDA_TRY(launch_pdl(image_grid_kernel, dim3(grid), dim3(256), 0, (cudaStream_t)stream, x01, N, C, H, W, xmaps, pad, Hg, Wg,
+    CUDA_TRY(launch_kernel(image_grid_kernel, dim3(grid), dim3(256), 0, (cudaStream_t)stream, x01, N, C, H, W, xmaps, pad, Hg, Wg,
                         grid_f32, grid_u8));
     LAUNCH_OK();
     return 0;
@@ -506,7 +497,6 @@ extern "C" int ddpm_image_grid(const float* x01, int N, int C, int H, int W, int
 // coalesced plane writes out); 3 B read + 12 B written per pixel.
 __global__ void batch_from_u8_kernel(const uint8_t* __restrict__ data, const int64_t* __restrict__ idx, int B, int64_t hw,
                                      float* __restrict__ out) {
-    pdl_enter();
     const int64_t total = (int64_t)B * hw;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
         const int b = (int)(i / hw); const int64_t p = i - (int64_t)b * hw;
@@ -523,7 +513,7 @@ extern "C" int ddpm_batch_from_u8(const uint8_t* data, int64_t n_images, const i
     if (!data || !idx || !out || n_images <= 0 || B <= 0 || H <= 0 || W <= 0) return DDPM_E_ARG;
     const int64_t hw = (int64_t)H * W, total = (int64_t)B * hw;
     int grid = (int)((total + 255) / 256); if (grid > 148 * 16) grid = 148 * 16;
-    CUDA_TRY(launch_pdl(batch_from_u8_kernel, dim3(grid), dim3(256), 0, (cudaStream_t)stream, data, idx, B, hw, out));
+    CUDA_TRY(launch_kernel(batch_from_u8_kernel, dim3(grid), dim3(256), 0, (cudaStream_t)stream, data, idx, B, hw, out));
     LAUNCH_OK();
     return 0;
 }
@@ -548,7 +538,6 @@ __global__ void layout_kernel(char* nchw, int64_t sn, int64_t sc, int64_t sh, in
 // tensor, twice per UNet evaluation).
 template <typename TS, typename TD, bool TO_NHWC>
 __global__ void layout_pix_kernel(char* nchw, int64_t sn, int64_t sc, int64_t sh, int64_t sw, TV v, int srcC) {
-    pdl_enter();
     const int64_t total = (int64_t)v.N * v.H * v.W;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
         const int x = (int)(i % v.W); const int64_t r = i / v.W;
@@ -581,7 +570,7 @@ __global__ void layout_pix_kernel(char* nchw, int64_t sn, int64_t sc, int64_t sh
 #define LAYOUT_GO(TS, TD, DIR, PTR, SRCC) { \
         if (v.C <= 32) { \
             const int64_t px = (int64_t)v.N * v.H * v.W; int g = (int)((px + 255) / 256); if (g > 148 * 16) g = 148 * 16; \
-            CUDA_TRY(launch_pdl(layout_pix_kernel<TS, TD, DIR>, dim3(g), dim3(256), 0, st, PTR, sn, sc, sh, sw, v, SRCC)); \
+            CUDA_TRY(launch_kernel(layout_pix_kernel<TS, TD, DIR>, dim3(g), dim3(256), 0, st, PTR, sn, sc, sh, sw, v, SRCC)); \
         } else layout_kernel<TS, TD, DIR><<<grid, 256, 0, st>>>(PTR, sn, sc, sh, sw, v, SRCC); }
 
 extern "C" int ddpm_nchw_to_nhwc(const void* src, int src_dtype, int src_C, int64_t sn, int64_t sc, int64_t sh,

@@ -191,7 +191,6 @@ struct GnP {
     const uint64_t* rng; uint32_t layer;
     const float* gamma; const float* beta;
     double* stats;               // [N][G][2] (sum, sum of squares)
-    float* ab;                   // MODE 3: [N][2][C] affine of the normalisation, z = ab[n][0][c] * x + ab[n][1][c]
     float* dgamma; float* dbeta; // backward: accumulated with atomics (may be NULL)
     float* cs_nc; float* cs_c;   // backward: per-image / total channel sums of the final dx (conv bias and time-bias gradients)
     int accumulate;              // backward: dx += ...
@@ -241,12 +240,10 @@ __device__ __forceinline__ void cta_channel_reduce(float (*part)[NT], const floa
     __syncthreads();
 }
 
-// MODE 0: fused stats + apply; 1: stats only; 2: apply only (stats given); 3: stats -> per-(image, channel) affine
-// coefficients for the convolution that applies GroupNorm (+SiLU) to its own input operand (conv_tc.cu, gn_ab)
+// MODE 0: fused stats + apply; 1: stats only; 2: apply only (stats given)
 template <typename T, int VEC, int MODE>
 __global__ void __launch_bounds__(NT, GN_FWD_OCC) gn_fwd_kernel(GnP a) {
     extern __shared__ __align__(16) unsigned char gsm[];
-    pdl_enter();
     const int C = a.x.C, G = a.G, cpg = C / G, HW = a.x.H * a.x.W;
     constexpr bool FAST_ACT = sizeof(T) == 2;                // bf16 tensors: tanh-based SiLU (common.cuh)
     constexpr int RING = gn_ring_bytes<VEC, 1, GN_PIPE_D_FWD>();
@@ -303,15 +300,6 @@ __global__ void __launch_bounds__(NT, GN_FWD_OCC) gn_fwd_kernel(GnP a) {
         }
         cluster_arrive();                                    // remote reads done; waited for before exit
         __syncthreads();
-        if (MODE == 3 && rank == 0) {
-            float* ab = a.ab + (size_t)n * 2 * C;
-            for (int c = threadIdx.x; c < C; c += NT) {
-                const int g = c / cpg;
-                const float sc = gr[g] * __ldg(a.gamma + c);
-                ab[c] = sc;
-                ab[C + c] = __ldg(a.beta + c) - gm[g] * sc;
-            }
-        }
     } else {
         for (int g = threadIdx.x; g < G; g += NT) {
             const double s = a.stats[((size_t)n * G + g) * 2], q = a.stats[((size_t)n * G + g) * 2 + 1];
@@ -352,7 +340,6 @@ __global__ void __launch_bounds__(NT, GN_FWD_OCC) gn_fwd_kernel(GnP a) {
 template <typename T, int VEC, bool STASH>
 __global__ void __launch_bounds__(NT, STASH ? GN_BWD_OCC : 2) gn_bwd_kernel(GnP a) {
     extern __shared__ __align__(16) unsigned char gsm[];
-    pdl_enter();
     const int C = a.x.C, G = a.G, cpg = C / G, HW = a.x.H * a.x.W;
     constexpr bool FAST_ACT = sizeof(T) == 2;                // bf16 tensors: tanh-based SiLU (common.cuh)
     constexpr int RING = gn_ring_bytes<VEC, 3>();
@@ -536,11 +523,10 @@ static int launch_cluster(K kernel, int grid, int cs, size_t smem, cudaStream_t 
     }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid); cfg.blockDim = dim3(NT); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute at[2]; unsigned nat = 1;
+    cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = cs; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    pdl_attr(at, &nat);
-    cfg.attrs = at; cfg.numAttrs = nat;
+    cfg.attrs = at; cfg.numAttrs = 1;
     cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, p);
     if (e != cudaSuccess) return (int)e;
     LAUNCH_OK();
@@ -555,7 +541,7 @@ static int gn_fill(GnP& p, const ddpm_tensor* x, int groups, const double* stats
     p.thr16 = p_drop > 0.f ? (uint32_t)(p_drop * 65536.0f + 0.5f) : 0u;
     p.keep_scale = p_drop > 0.f ? 1.0f / (1.0f - p_drop) : 1.0f;
     p.rng = rng; p.layer = layer; p.gamma = gamma; p.beta = beta; p.stats = const_cast<double*>(stats);
-    p.ab = nullptr; p.dgamma = p.dbeta = nullptr; p.cs_nc = p.cs_c = nullptr; p.accumulate = 0; p.stash = 0; p.wshift = log2_exact(x->W);
+    p.dgamma = p.dbeta = nullptr; p.cs_nc = p.cs_c = nullptr; p.accumulate = 0; p.stash = 0; p.wshift = log2_exact(x->W);
     return 0;
 }
 
@@ -567,8 +553,8 @@ static int gn_fwd_dispatch(GnP& p, const ddpm_tensor* x, const ddpm_tensor* out,
         int cs = MODE == 2 ? 1 : gn_cluster_size(HW, cvs, x->N); \
         if (MODE == 2) { cs = 1; int want = (HW * cvs) / (NT * 16); while (cs < 8 && cs < want) cs <<= 1; } \
         return launch_cluster(gn_fwd_kernel<T, VEC, MODE>, x->N * cs, cs, sm0 + gn_ring_bytes<VEC, 1, GN_PIPE_D_FWD>(), st, p); }
-    const bool v8 = vec_ok(x, 8, 2) && (MODE == 1 || MODE == 3 || vec_ok(out, 8, 2));
-    const bool v4 = vec_ok(x, 4, 4) && (MODE == 1 || MODE == 3 || vec_ok(out, 4, 4));
+    const bool v8 = vec_ok(x, 8, 2) && (MODE == 1 || vec_ok(out, 8, 2));
+    const bool v4 = vec_ok(x, 4, 4) && (MODE == 1 || vec_ok(out, 4, 4));
     if (dtype == DDPM_BF16) { if (v8) GO(bf16, 8) else GO(bf16, 1) }
     else if (dtype == DDPM_F32) { if (v4) GO(float, 4) else GO(float, 1) }
 #undef GO
@@ -580,14 +566,6 @@ extern "C" int ddpm_gn_stats(const ddpm_tensor* x, int dtype, int groups, double
     GnP p; int rc = gn_fill(p, x, groups, stats, nullptr, nullptr, 0.f, 0, 0.f, nullptr, 0); if (rc) return rc;
     p.o = p.x; p.dy = p.x;
     return gn_fwd_dispatch<1>(p, x, x, dtype, (cudaStream_t)stream);
-}
-
-extern "C" int ddpm_gn_coeffs(const ddpm_tensor* x, int dtype, int groups, const float* gamma, const float* beta, float eps,
-                              float* ab, void* stream) {
-    if (!tensor_ok(x) || !ab || !gamma || !beta || groups <= 0 || x->C % groups) return DDPM_E_ARG;
-    GnP p; int rc = gn_fill(p, x, groups, nullptr, gamma, beta, eps, 0, 0.f, nullptr, 0); if (rc) return rc;
-    p.o = p.x; p.dy = p.x; p.ab = ab;
-    return gn_fwd_dispatch<3>(p, x, x, dtype, (cudaStream_t)stream);
 }
 
 extern "C" int ddpm_gn_apply(const ddpm_tensor* x, int dtype, int groups, const double* stats, const float* gamma,
@@ -655,7 +633,6 @@ extern "C" int ddpm_gn_bwd_colsum(const ddpm_tensor* x, int dtype, int groups, c
 // generic walker over (n, y, x, cv) of the OUTPUT view
 template <typename T, int VEC, typename F>
 __global__ void __launch_bounds__(NT) pix_kernel(int N, int H, int W, int C, F f) {
-    pdl_enter();
     const int cvs = C / VEC;
     const int64_t total = (int64_t)N * H * W * cvs;
     for (int64_t i = (int64_t)blockIdx.x * NT + threadIdx.x; i < total; i += (int64_t)gridDim.x * NT) {
@@ -682,7 +659,7 @@ extern "C" int ddpm_upsample2x(const ddpm_tensor* x, const ddpm_tensor* out, int
     if (!tensor_ok(x) || !tensor_ok(out) || out->H != 2 * x->H || out->W != 2 * x->W || out->C != x->C || out->N != x->N) return DDPM_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
 #define GO(T, VEC) { UpFwd<T, VEC> f{TV(*x), TV(*out)}; int64_t tot = (int64_t)out->N * out->H * out->W * (out->C / VEC); \
-        if (launch_pdl(pix_kernel<T, VEC, decltype(f)>, dim3(pix_grid(tot)), dim3(NT), 0, st, out->N, out->H, out->W, out->C, f) != cudaSuccess) return (int)cudaGetLastError(); }
+        if (launch_kernel(pix_kernel<T, VEC, decltype(f)>, dim3(pix_grid(tot)), dim3(NT), 0, st, out->N, out->H, out->W, out->C, f) != cudaSuccess) return (int)cudaGetLastError(); }
     if (dtype == DDPM_BF16) { if (vec_ok(x, 8, 2) && vec_ok(out, 8, 2)) GO(bf16, 8) else GO(bf16, 1) }
     else if (dtype == DDPM_F32) { if (vec_ok(x, 4, 4) && vec_ok(out, 4, 4)) GO(float, 4) else GO(float, 1) }
     else return DDPM_E_ARG;
@@ -711,7 +688,7 @@ extern "C" int ddpm_upsample2x_bwd(const ddpm_tensor* dy, const ddpm_tensor* dx,
     if (!tensor_ok(dy) || !tensor_ok(dx) || dy->H != 2 * dx->H || dy->W != 2 * dx->W || dy->C != dx->C || dy->N != dx->N) return DDPM_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
 #define GO(T, VEC) { UpBwd<T, VEC> f{TV(*dy), TV(*dx), accumulate}; int64_t tot = (int64_t)dx->N * dx->H * dx->W * (dx->C / VEC); \
-        if (launch_pdl(pix_kernel<T, VEC, decltype(f)>, dim3(pix_grid(tot)), dim3(NT), 0, st, dx->N, dx->H, dx->W, dx->C, f) != cudaSuccess) return (int)cudaGetLastError(); }
+        if (launch_kernel(pix_kernel<T, VEC, decltype(f)>, dim3(pix_grid(tot)), dim3(NT), 0, st, dx->N, dx->H, dx->W, dx->C, f) != cudaSuccess) return (int)cudaGetLastError(); }
     if (dtype == DDPM_BF16) { if (vec_ok(dy, 8, 2) && vec_ok(dx, 8, 2)) GO(bf16, 8) else GO(bf16, 1) }
     else if (dtype == DDPM_F32) { if (vec_ok(dy, 4, 4) && vec_ok(dx, 4, 4)) GO(float, 4) else GO(float, 1) }
     else return DDPM_E_ARG;
@@ -736,7 +713,7 @@ extern "C" int ddpm_zero_upsample2x(const ddpm_tensor* x, const ddpm_tensor* out
     if (!tensor_ok(x) || !tensor_ok(out) || out->H != 2 * x->H || out->W != 2 * x->W || out->C != x->C || out->N != x->N) return DDPM_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
 #define GO(T, VEC) { ZeroUp<T, VEC> f{TV(*x), TV(*out)}; int64_t tot = (int64_t)out->N * out->H * out->W * (out->C / VEC); \
-        if (launch_pdl(pix_kernel<T, VEC, decltype(f)>, dim3(pix_grid(tot)), dim3(NT), 0, st, out->N, out->H, out->W, out->C, f) != cudaSuccess) return (int)cudaGetLastError(); }
+        if (launch_kernel(pix_kernel<T, VEC, decltype(f)>, dim3(pix_grid(tot)), dim3(NT), 0, st, out->N, out->H, out->W, out->C, f) != cudaSuccess) return (int)cudaGetLastError(); }
     if (dtype == DDPM_BF16) { if (vec_ok(x, 8, 2) && vec_ok(out, 8, 2)) GO(bf16, 8) else GO(bf16, 1) }
     else if (dtype == DDPM_F32) { if (vec_ok(x, 4, 4) && vec_ok(out, 4, 4)) GO(float, 4) else GO(float, 1) }
     else return DDPM_E_ARG;
@@ -762,7 +739,7 @@ extern "C" int ddpm_add(const ddpm_tensor* a, const ddpm_tensor* b, const ddpm_t
     if (b->N != out->N || b->H != out->H || b->W != out->W || b->C != out->C) return DDPM_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
 #define GO(T, VEC) { AddOp<T, VEC> f{TV(*a), TV(*b), TV(*out)}; int64_t tot = (int64_t)out->N * out->H * out->W * (out->C / VEC); \
-        if (launch_pdl(pix_kernel<T, VEC, decltype(f)>, dim3(pix_grid(tot)), dim3(NT), 0, st, out->N, out->H, out->W, out->C, f) != cudaSuccess) return (int)cudaGetLastError(); }
+        if (launch_kernel(pix_kernel<T, VEC, decltype(f)>, dim3(pix_grid(tot)), dim3(NT), 0, st, out->N, out->H, out->W, out->C, f) != cudaSuccess) return (int)cudaGetLastError(); }
     if (dtype == DDPM_BF16) { if (vec_ok(a, 8, 2) && vec_ok(b, 8, 2) && vec_ok(out, 8, 2)) GO(bf16, 8) else GO(bf16, 1) }
     else if (dtype == DDPM_F32) { if (vec_ok(a, 4, 4) && vec_ok(b, 4, 4) && vec_ok(out, 4, 4)) GO(float, 4) else GO(float, 1) }
     else return DDPM_E_ARG;
@@ -775,7 +752,6 @@ extern "C" int ddpm_add(const ddpm_tensor* a, const ddpm_tensor* b, const ddpm_t
 template <typename T, int VEC>
 __global__ void __launch_bounds__(NT) colsum_kernel(TV dy, float* out_nc, float* dbias) {
     extern __shared__ float acc[];           // [C]
-    pdl_enter();
     const int n = blockIdx.y, C = dy.C, HW = dy.H * dy.W;
     for (int c = threadIdx.x; c < C; c += NT) acc[c] = 0.f;
     __syncthreads();
@@ -810,7 +786,7 @@ extern "C" int ddpm_colsum(const ddpm_tensor* dy, int dtype, float* out_nc, floa
     int HW = dy->H * dy->W;
 #define GO(T, VEC) { int cvs = dy->C / VEC; if (cvs > NT) return DDPM_E_ARG; int ppi = NT / cvs; \
         dim3 grid(blocks_per_image(dy->N, HW, ppi * 8), dy->N); \
-        if (launch_pdl(colsum_kernel<T, VEC>, grid, dim3(NT), sizeof(float) * dy->C, st, v, out_nc, dbias) != cudaSuccess) return (int)cudaGetLastError(); }
+        if (launch_kernel(colsum_kernel<T, VEC>, grid, dim3(NT), sizeof(float) * dy->C, st, v, out_nc, dbias) != cudaSuccess) return (int)cudaGetLastError(); }
     if (dtype == DDPM_BF16) { if (vec_ok(dy, 8, 2)) GO(bf16, 8) else GO(bf16, 1) }
     else if (dtype == DDPM_F32) { if (vec_ok(dy, 4, 4)) GO(float, 4) else GO(float, 1) }
     else return DDPM_E_ARG;

@@ -324,18 +324,16 @@ def _gptr(p) -> Optional[int]:
 def conv(E: Exec, x: Act, wpack: torch.Tensor, out: Act, k: int, stride: int = 1, pad: int = 0, *,
          bias: Optional[torch.Tensor] = None, tbias: Optional[torch.Tensor] = None, res: Optional[Act] = None,
          z: Optional[Act] = None, accum: bool = False, a_silu: bool = False, mode: int = _lib.CONV_NORMAL,
-         dt: Optional[int] = None, in2: Optional[Act] = None, w2pack: Optional[torch.Tensor] = None, up_phase: int = 0,
-         gn_ab: Optional[torch.Tensor] = None, gn_act: int = 0) -> Act:
+         dt: Optional[int] = None, in2: Optional[Act] = None, w2pack: Optional[torch.Tensor] = None, up_phase: int = 0) -> Act:
     """`in2` / `w2pack`: out = conv(x; w) + conv1x1(in2; w2) in one launch (see ddpm_conv_args.in2).
-    `mode=CONV_UP2X_PHASE`, `up_phase`: one output phase of conv3x3(nearest x2 (x)) from the low-resolution x.
-    `gn_ab` / `gn_act`: GroupNorm (+SiLU) of `x` applied inside the convolution (gn_coeffs; ddpm_conv_args.gn_ab)."""
+    `mode=CONV_UP2X_PHASE`, `up_phase`: one output phase of conv3x3(nearest x2 (x)) from the low-resolution x."""
     dt = x.dt if dt is None else dt
-    a = _conv_args(E, x, wpack, out, k, stride, pad, bias, tbias, res, z, accum, a_silu, mode, dt, in2, w2pack, up_phase, gn_ab, gn_act)
+    a = _conv_args(E, x, wpack, out, k, stride, pad, bias, tbias, res, z, accum, a_silu, mode, dt, in2, w2pack, up_phase)
     _lib.call("ddpm_conv", C.byref(a), E.stream)
     return out
 
 
-def _conv_args(E, x, wpack, out, k, stride, pad, bias, tbias, res, z, accum, a_silu, mode, dt, in2, w2pack, up_phase, gn_ab, gn_act):
+def _conv_args(E, x, wpack, out, k, stride, pad, bias, tbias, res, z, accum, a_silu, mode, dt, in2, w2pack, up_phase):
     a = _lib.ConvArgs()
     a.inp, a.out = x.desc(), out.desc()
     a.w = wpack.data_ptr()
@@ -358,8 +356,6 @@ def _conv_args(E, x, wpack, out, k, stride, pad, bias, tbias, res, z, accum, a_s
     a.dtype = dt
     a.prefer_tc = E.prefer_tc
     a.up_phase = up_phase
-    a.gn_ab = gn_ab.data_ptr() if gn_ab is not None else None
-    a.gn_act = gn_act
     return a
 
 
@@ -403,34 +399,6 @@ def gn_stats(E: Exec, x: Act, groups: int) -> torch.Tensor:
     st = torch.empty((x.N, groups, 2), dtype=torch.float64, device=E.device)
     _lib.call("ddpm_gn_stats", C.byref(x.desc()), x.dt, groups, st.data_ptr(), E.stream)
     return st
-
-
-def fuse_gn_enabled() -> bool:
-    """Opt-in (DDPM_B200_FUSE_GN=1).  Measured on B200 (profiles/r2_gn_operand_fusion.txt): the fused form is bit-identical to
-    the two-launch form but slower -- the transform costs ~7.5 instructions per element on warps that run alone on their
-    scheduler, over a patch that is 1.5x the tile (halo) and is re-transformed per output-channel tile: 96->96@64, B=256:
-    47 + 236 us against 103 + 135 us; DDIM-100 350 against 390 samples/s."""
-    import os
-    return os.environ.get("DDPM_B200_FUSE_GN", "0") == "1"
-
-
-def gn_fusable(E: Exec, x: Act, cout: int, k: int, in2: Optional[Act] = None) -> bool:
-    """GroupNorm (+SiLU) folded into the consuming convolution's operand path (north_star (1); conv_tc.cu GNA kernels): used
-    when nothing needs the normalised activation afterwards -- sampling / evaluation (no gradient, no dropout) on the
-    tensor-core path.  Training keeps the materialised activation: it IS the saved operand of the weight gradient."""
-    if not (E.use_tc and not E.need_grad and not E.training and fuse_gn_enabled()):
-        return False
-    if x.halo != 1 or x.C % 16 or cout % 16 or x.pitch % 8 or x.W + 2 > 300:
-        return False
-    return in2 is None or (in2.halo == 1 and in2.C % 16 == 0 and in2.pitch % 8 == 0)
-
-
-def gn_coeffs(E: Exec, x: Act, gn: torch.nn.GroupNorm) -> torch.Tensor:
-    """Statistics of `x` as the affine z = ab[n][0][c] * x + ab[n][1][c] of the normalisation (fp32 [N][2][C])."""
-    ab = torch.empty((x.N, 2, x.C), dtype=torch.float32, device=E.device)
-    _lib.call("ddpm_gn_coeffs", C.byref(x.desc()), x.dt, gn.num_groups, gn.weight.data_ptr(), gn.bias.data_ptr(),
-              float(gn.eps), ab.data_ptr(), E.stream)
-    return ab
 
 
 def gn_apply(E: Exec, x: Act, st: torch.Tensor, gn: torch.nn.GroupNorm, act: int, p_drop: float, layer: int,
@@ -577,8 +545,6 @@ def resblock_fwd(E: Exec, blk, x: Act, tbias: torch.Tensor, out: Optional[Act] =
     `tbias_has_b1`: the caller's time bias already contains conv1's bias (time_proj_all_fwd)."""
     Cout = blk.out_ch
     p_drop = float(blk.drop.p) if (E.training and isinstance(blk.drop, torch.nn.Dropout)) else 0.0
-    if gn_fusable(E, x, Cout, 3, x):
-        return _resblock_fwd_gn_fused(E, blk, x, tbias, out, tbias_has_b1), None
     a1, st1 = gn_fwd(E, x, blk.norm1, 1, 0.0, 0)
     w1, _ = E.wcache.get(E, blk.conv1.weight, E.dt, E.need_grad)
     h = conv(E, a1, w1, E.act(x.N, x.H, x.W, Cout), 3, 1, 1, bias=None if tbias_has_b1 else blk.conv1.bias, tbias=tbias)
@@ -599,28 +565,6 @@ def resblock_fwd(E: Exec, blk, x: Act, tbias: torch.Tensor, out: Optional[Act] =
         conv(E, a2, w2, out, 3, 1, 1, bias=blk.conv2.bias, res=x)
     saved = (x, st1, a1, h, st2, a2, p_drop, layer) if E.need_grad else None
     return out, saved
-
-
-def _resblock_fwd_gn_fused(E: Exec, blk, x: Act, tbias: torch.Tensor, out: Optional[Act], tbias_has_b1: bool) -> Act:
-    """The same block without materialising silu(gn(.)): two statistics launches, two convolutions."""
-    Cout = blk.out_ch
-    w1, _ = E.wcache.get(E, blk.conv1.weight, E.dt, False)
-    h = conv(E, x, w1, E.act(x.N, x.H, x.W, Cout), 3, 1, 1, bias=None if tbias_has_b1 else blk.conv1.bias, tbias=tbias,
-             gn_ab=gn_coeffs(E, x, blk.norm1), gn_act=1)
-    ab2 = gn_coeffs(E, h, blk.norm2)
-    w2, _ = E.wcache.get(E, blk.conv2.weight, E.dt, False)
-    if out is None:
-        out = E.act(x.N, x.H, x.W, Cout)
-    if isinstance(blk.skip, torch.nn.Conv2d):
-        ws, _ = E.wcache.get(E, blk.skip.weight, E.dt, False)
-        if fuse_skip_enabled() and blk.skip.bias is not None and blk.conv2.bias is not None:
-            conv(E, h, w2, out, 3, 1, 1, bias=blk.conv2.bias.detach() + blk.skip.bias.detach(), in2=x, w2pack=ws, gn_ab=ab2, gn_act=1)
-        else:
-            conv(E, x, ws, out, 1, bias=blk.skip.bias)
-            conv(E, h, w2, out, 3, 1, 1, bias=blk.conv2.bias, accum=True, gn_ab=ab2, gn_act=1)
-    else:
-        conv(E, h, w2, out, 3, 1, 1, bias=blk.conv2.bias, res=x, gn_ab=ab2, gn_act=1)
-    return out
 
 
 def resblock_bwd(E: Exec, blk, saved, dout: Act, dx: Optional[Act] = None, dx_accum: bool = False):
@@ -710,12 +654,8 @@ def attn_fwd(E: Exec, blk, x: Act, out: Optional[Act] = None):
     heads, d = blk.num_heads, blk.head_dim
     inner = heads * d
     wq, _ = E.wcache.get(E, blk.qkv.weight, E.dt, E.need_grad)
-    if gn_fusable(E, x, 3 * inner, 1):
-        a, st = None, None
-        qkv = conv(E, x, wq, E.act(x.N, x.H, x.W, 3 * inner), 1, gn_ab=gn_coeffs(E, x, blk.norm), gn_act=0)
-    else:
-        a, st = gn_fwd(E, x, blk.norm, 0, 0.0, 0)
-        qkv = conv(E, a, wq, E.act(x.N, x.H, x.W, 3 * inner), 1)
+    a, st = gn_fwd(E, x, blk.norm, 0, 0.0, 0)
+    qkv = conv(E, a, wq, E.act(x.N, x.H, x.W, 3 * inner), 1)
     o = E.act(x.N, x.H, x.W, inner)
     lse = E.f32(x.N, heads, x.H * x.W)
     _lib.call("ddpm_attn_fwd", C.byref(qkv.desc()), C.byref(o.desc()), heads, d, lse.data_ptr(), E.dt, E.stream)
@@ -966,13 +906,8 @@ def unet_forward(E: Exec, model, x: torch.Tensor, t: torch.Tensor, out_dtype: to
     # ---- head
     w_out, _ = E.wcache.get(E, model.out_conv.weight, E.dt, G, cout_pad=cpad)
     oc = model.out_conv.out_channels
-    if gn_fusable(E, cur, max(oc, cpad), 3):
-        a, st = None, None
-        y = conv(E, cur, w_out, E.act(B, H, W, max(oc, cpad)), 3, 1, 1, bias=model.out_conv.bias,
-                 gn_ab=gn_coeffs(E, cur, model.out_norm), gn_act=1)
-    else:
-        a, st = gn_fwd(E, cur, model.out_norm, 1, 0.0, 0)
-        y = conv(E, a, w_out, E.act(B, H, W, max(oc, cpad)), 3, 1, 1, bias=model.out_conv.bias)
+    a, st = gn_fwd(E, cur, model.out_norm, 1, 0.0, 0)
+    y = conv(E, a, w_out, E.act(B, H, W, max(oc, cpad)), 3, 1, 1, bias=model.out_conv.bias)
     out = to_nchw(E, y.slice(0, oc) if y.C != oc else y, out_dtype)
     saved = None
     if G:

@@ -113,10 +113,6 @@ int ddpm_sinusoid(const void* t, int t_is_float, int B, int dim, void* out, int 
 /* ---------------- GroupNorm (+SiLU, +dropout): attention.py:38-39, unet_backbone.py:38,43 -- */
 /* stats: double [N][G][2] = (sum, sum of squares) over the group's elements; zeroed by the call. */
 int ddpm_gn_stats(const ddpm_tensor* x, int dtype, int groups, double* stats, void* stream);
-/* Statistics reduced to the affine form of the normalisation: ab[n][0][c] = rstd * gamma[c], ab[n][1][c] = beta[c] -
- * mean * rstd * gamma[c] (fp32 [N][2][C]); consumed by ddpm_conv's gn_ab operand transform (sampling path). */
-int ddpm_gn_coeffs(const ddpm_tensor* x, int dtype, int groups, const float* gamma, const float* beta, float eps,
-                   float* ab, void* stream);
 /* out = drop(act(gn(x))); act: 0 none, 1 SiLU.  rng: device uint64[2] {seed, step} (may be NULL
  * when p_drop == 0); layer_id decorrelates call sites. */
 int ddpm_gn_apply(const ddpm_tensor* x, int dtype, int groups, const double* stats, const float* gamma,
@@ -192,17 +188,8 @@ typedef struct {
     ddpm_tensor in2;
     const void* w2;
     int32_t up_phase;      /* DDPM_CONV_UP2X_PHASE: 2*py + px in 0..3 (ignored otherwise) */
-    /* GroupNorm (+SiLU) applied to the INPUT operand inside the convolution (attention.py:38-39,61; unet_backbone.py:37-38,
-     * 43-44,215): the kernel convolves act(gn_ab[n][0][c] * in[n,y,x,c] + gn_ab[n][1][c]) (act = SiLU when gn_act == 1) -- the
-     * normalised activation never exists in HBM.  gn_ab: fp32 [N][2][in.C] from ddpm_gn_coeffs; the zero halo stays zero
-     * (= zero padding of the ACTIVATED tensor, like the reference) and `in2` is not transformed.  Tensor-core path only
-     * (ddpm_conv_gn_fusable); NULL: none. */
-    const float* gn_ab;
-    int32_t gn_act;
 } ddpm_conv_args;
 int ddpm_conv(const ddpm_conv_args* a, void* stream);
-/* 1 when ddpm_conv would run `a` (with a non-NULL gn_ab) on the fused tensor-core path, else 0 (then ddpm_conv rejects it) */
-int ddpm_conv_gn_fusable(const ddpm_conv_args* a);
 /* test / tuning hooks: force the CUDA-core kernels */
 int ddpm_set_force_simt(int on);
 /* Force tensor-core paths that the planners otherwise pick only for other shapes (tests, A/B measurements).  Bit 0 of
@@ -214,10 +201,6 @@ int ddpm_set_force_simt(int on);
  * (1 restores the default planning).  The flags are read on the host when a call plans its launch; no kernel sees them.
  * Anything else returns DDPM_E_ARG and leaves the setting unchanged. */
 int ddpm_set_tc_mode(int mode, int base_offset);
-/* 1 (env DDPM_B200_PDL=1): kernels are launched with programmatic stream serialisation (griddepcontrol): the prologue of
- * kernel i+1 overlaps the tail of kernel i.  0 (default since round 2): plain stream order -- measured neutral at 64 px and
- * 5-25 % slower at 256 px with it on (DESIGN.md section 6). */
-int ddpm_set_pdl(int on);
 
 /* All time_proj linears of a UNet in one launch (unet_backbone.py:25-27,41): out[m][col0_i + n] =
  * sum_k f(x[m][k]) W_i[n][k] + b_i[n], f = SiLU when a_silu.  `entries_dev` is an array in DEVICE memory. */

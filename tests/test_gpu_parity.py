@@ -218,7 +218,7 @@ def _halo_max(a):
                                    (2, 192, 16, 16), (2, 192, 32, 32), (2, 96, 12, 20),
                                    (2, 128, 128, 128),        # few large images -> clusters of 16 CTAs
                                    (130, 192, 16, 16), (2, 288, 64, 64), (3, 96, 24, 24), (2, 384, 32, 32), (5, 192, 8, 8),
-                                   (2, 32, 4, 4)])
+                                   (2, 32, 4, 4), (7, 384, 16, 16), (4, 512, 16, 16)])
 @pytest.mark.parametrize("act", [0, 1])
 def test_groupnorm_fwd_bwd(pkg, shape, act, dt_name):
     _, _lib, engine = pkg

@@ -26,7 +26,7 @@ def test_abi_exports_every_declared_symbol():
     assert not missing, missing
     # the ctypes table binds exactly the header's functions (+ the test hook ddpm_set_force_simt)
     assert declared <= set(_lib.SIGNATURES), declared - set(_lib.SIGNATURES)
-    assert lib.ddpm_abi_version() == 1
+    assert lib.ddpm_abi_version() == 2
 
 
 def test_tc_mode_accepts_only_the_path_forcing_flags():

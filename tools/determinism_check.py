@@ -1,7 +1,7 @@
 """Run-to-run determinism of one backward pass (diagnostic): same weights, same batch, same seeds, R repetitions;
 reports which parameter gradients differ bitwise between repetitions and by how much relative to the gradient's
 scale.  fp32 atomics (GroupNorm dgamma/dbeta, bias column sums) may reorder; tensor-core paths must not differ.
-    python tools/determinism_check.py [tiny|low]      (env DDPM_B200_PDL / DDPM_B200_WGRAD_OVERLAP select modes)"""
+    python tools/determinism_check.py [tiny|low]      (env DDPM_B200_WGRAD_OVERLAP selects the mode)"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -31,7 +31,7 @@ for r in range(R):
     (loss * 1024.0).backward()
     torch.cuda.synchronize()
     runs.append((float(loss), [p.grad.detach().clone() for p in model.parameters()]))
-print(f"{which}: PDL={os.environ.get('DDPM_B200_PDL', '1')} overlap={os.environ.get('DDPM_B200_WGRAD_OVERLAP', '1')} "
+print(f"{which}: overlap={os.environ.get('DDPM_B200_WGRAD_OVERLAP', '1')} "
       f"losses {[f'{l:.7f}' for l, _ in runs]}")
 bad = {}
 for r in range(1, R):

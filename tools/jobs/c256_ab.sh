@@ -13,7 +13,5 @@ except Exception as e:
 PY
 }
 run base A=1
-run nopdl DDPM_B200_PDL=0
 run nooverlap DDPM_B200_WGRAD_OVERLAP=0
-run nopdl_nooverlap DDPM_B200_PDL=0 DDPM_B200_WGRAD_OVERLAP=0
 run base2 A=1
