@@ -146,49 +146,17 @@ static inline bool tensor_ok(const ddpm_tensor* t) {
            (t->halo == 0 || t->halo == 1);
 }
 
-// Philox4x32-10 counter RNG (dropout masks; recomputed in backward from the same counters)
-__device__ __forceinline__ uint4 philox4(uint32_t k0, uint32_t k1, uint4 c) {
-    const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        uint32_t hi0 = __umulhi(M0, c.x), lo0 = M0 * c.x;
-        uint32_t hi1 = __umulhi(M1, c.z), lo1 = M1 * c.z;
-        c = make_uint4(hi1 ^ c.y ^ k0, lo1, hi0 ^ c.w ^ k1, lo0);
-        k0 += W0; k1 += W1;
-    }
-    return c;
-}
-// keep-bits for VEC consecutive elements starting at `e0` (e0 % VEC == 0 for VEC in {4, 8}): one
-// Philox call per 4 elements; bit i set = keep element e0+i.  Same function in forward and backward.
-template <int VEC>
-__device__ __forceinline__ uint32_t dropout_mask(const uint64_t* rng, uint32_t layer, uint64_t e0, float p) {
-    const uint64_t seed = rng[0], step = rng[1];
-    const uint32_t thr = (uint32_t)(p * 16777216.0f);            // keep iff (w >> 8) >= thr
-    uint32_t m = 0;
-    if (VEC == 1) {
-        uint4 r = philox4((uint32_t)seed, (uint32_t)(seed >> 32),
-                          make_uint4((uint32_t)(e0 >> 2), (uint32_t)(e0 >> 34), (uint32_t)step, layer));
-        uint32_t w = (e0 & 3) == 0 ? r.x : (e0 & 3) == 1 ? r.y : (e0 & 3) == 2 ? r.z : r.w;
-        return (w >> 8) >= thr ? 1u : 0u;
-    }
-#pragma unroll
-    for (int q = 0; q < VEC / 4; ++q) {
-        uint64_t e = (e0 >> 2) + q;
-        uint4 r = philox4((uint32_t)seed, (uint32_t)(seed >> 32),
-                          make_uint4((uint32_t)e, (uint32_t)(e >> 32), (uint32_t)step, layer));
-        m |= ((r.x >> 8) >= thr ? 1u : 0u) << (4 * q);
-        m |= ((r.y >> 8) >= thr ? 1u : 0u) << (4 * q + 1);
-        m |= ((r.z >> 8) >= thr ? 1u : 0u) << (4 * q + 2);
-        m |= ((r.w >> 8) >= thr ? 1u : 0u) << (4 * q + 3);
-    }
-    return m;
-}
 // Dropout keep-bits.  The GroupNorm kernels are instruction-bound on B200 (an SM has ~22 B/clk of HBM
 // bandwidth, i.e. a budget of ~20 instructions per bf16 element), and Philox4x32-10 cost ~12 of them.
-// Parity with ATen's mask is statistical only (SURVEY.md §7), so the mask comes from a counter hash:
-// element e uses 16-bit half (e & 1) of lowbias32((e >> 1) ^ key), key = f(seed, step, layer); keep iff
-// half >= thr16 = round(p * 65536).  ~4 instructions per element; fp32 (VEC 4), bf16 (VEC 8) and scalar paths
-// draw the same mask; forward and backward recompute it from the same (seed, step, layer, index).
+// Parity with ATen's mask is statistical only (SURVEY.md §7), so the mask comes from a counter hash.  Element e
+// belongs to the 32-bit word w = e >> 1 and uses 16-bit half (e & 1) of lowbias32(((w & ~3) ^ key) + (w & 3)),
+// key = dropout_key(seed, step, layer); keep iff half >= thr16 = (uint32_t)(p * 65536 + 0.5).  e is the logical NHWC
+// index ((n*H + y)*W + x)*C + c of the view, wrapped to 32 bits: it does not depend on the pitch, the halo or the
+// channel offset of the buffer.  The hash input is a bijection of w for every key (the low two bits of w are added
+// to a block base whose low bits are key & 3, so no two words share an input), and it is what the bf16 path, which
+// training runs, draws with one XOR per 8-element packet.  ~4 instructions per element; fp32 (VEC 4), bf16 (VEC 8)
+// and scalar paths draw the same mask, so forward and backward may take different paths and still recompute the
+// same mask from (seed, step, layer, index).
 __device__ __forceinline__ uint32_t lowbias32(uint32_t x) {
     x ^= x >> 16; x *= 0x7feb352dU; x ^= x >> 15; x *= 0x846ca68bU; x ^= x >> 16;
     return x;
@@ -202,9 +170,12 @@ __device__ __forceinline__ uint32_t dropout_key(const uint64_t* rng, uint32_t la
     return k;
 }
 // in-place: v[i] = keep_i ? v[i] * scale : 0 for the VEC elements starting at (wrapping 32-bit) index e0
+// (e0 % VEC == 0 for VEC > 1).  For VEC 8 the packet's four words are one aligned block (w0 & 3 == 0), so the block
+// base is w0 ^ key; VEC 4 covers half a block and the scalar path one word, so they add w & 3 themselves.
 template <int VEC>
 __device__ __forceinline__ void dropout_apply(float* v, uint32_t key, uint32_t e0, uint32_t thr16, float scale) {
-    const uint32_t base = (e0 >> 1) ^ key;
+    const uint32_t w0 = e0 >> 1;
+    const uint32_t base = VEC == 8 ? (w0 ^ key) : ((w0 & ~3u) ^ key) + (w0 & 3u);
     if (VEC == 1) {
         const uint32_t h = lowbias32(base);
         v[0] = (((e0 & 1) ? (h >> 16) : (h & 0xffffu)) >= thr16) ? v[0] * scale : 0.f;
@@ -216,28 +187,4 @@ __device__ __forceinline__ void dropout_apply(float* v, uint32_t key, uint32_t e
         v[2 * i] = ((h & 0xffffu) >= thr16) ? v[2 * i] * scale : 0.f;
         v[2 * i + 1] = ((h >> 16) >= thr16) ? v[2 * i + 1] * scale : 0.f;
     }
-}
-template <int VEC>
-__device__ __forceinline__ uint32_t dropout_mask16(uint32_t key, uint64_t e0, uint32_t thr16) {
-    const uint32_t base = ((uint32_t)(e0 >> 1) ^ ((uint32_t)(e0 >> 33) * 0x9E3779B9U)) ^ key;
-    uint32_t m = 0;
-    if (VEC == 1) {
-        const uint32_t h = lowbias32(base);
-        return (((e0 & 1) ? (h >> 16) : (h & 0xffffu)) >= thr16) ? 1u : 0u;
-    }
-#pragma unroll
-    for (int i = 0; i < VEC / 2; ++i) {
-        const uint32_t h = lowbias32(base + (uint32_t)i);      // (e0 >> 1) + i: VEC consecutive elements, e0 % VEC == 0
-        m |= ((h & 0xffffu) >= thr16 ? 1u : 0u) << (2 * i);
-        m |= ((h >> 16) >= thr16 ? 1u : 0u) << (2 * i + 1);
-    }
-    return m;
-}
-// keep-mask for element index `e` (one Philox call covers 4 consecutive elements)
-__device__ __forceinline__ bool dropout_keep(const uint64_t* rng, uint32_t layer, uint64_t e, float p) {
-    uint64_t seed = rng[0], step = rng[1];
-    uint4 r = philox4((uint32_t)seed, (uint32_t)(seed >> 32),
-                      make_uint4((uint32_t)(e >> 2), (uint32_t)(e >> 34), (uint32_t)step, layer));
-    uint32_t w = (e & 3) == 0 ? r.x : (e & 3) == 1 ? r.y : (e & 3) == 2 ? r.z : r.w;
-    return (float)(w >> 8) * (1.0f / 16777216.0f) >= p;
 }

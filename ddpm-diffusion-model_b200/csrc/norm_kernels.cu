@@ -599,11 +599,12 @@ static int gn_bwd_impl(const ddpm_tensor* x, int dtype, int groups, const double
     p.dy = TV(*dy); p.o = TV(*dx); p.accumulate = accumulate; p.dgamma = dgamma; p.dbeta = dbeta;
     p.cs_nc = cs_nc; p.cs_c = cs_c; p.stash = dy_scratch ? 1 : 0;
     cudaStream_t st = (cudaStream_t)stream;
-    if (cs_nc) CUDA_TRY(cudaMemsetAsync(cs_nc, 0, sizeof(float) * x->N * x->C, st));
     const int HW = x->H * x->W, C = x->C;
     const size_t sm0 = sizeof(double) * 2 * C + sizeof(float) * (2 * C + 4 * groups);
+    // colsum_nc is zeroed only once the shape is accepted: a rejected call writes nothing
 #define GO(T, VEC) { int cvs = C / VEC; if (cvs > NT) return DDPM_E_ARG; int cs = gn_cluster_size(HW, cvs, x->N); \
         const size_t sm = sm0 + gn_ring_bytes<VEC, 3>(); \
+        if (cs_nc) CUDA_TRY(cudaMemsetAsync(cs_nc, 0, sizeof(float) * x->N * x->C, st)); \
         if (p.stash) return launch_cluster(gn_bwd_kernel<T, VEC, true>, x->N * cs, cs, sm, st, p); \
         return launch_cluster(gn_bwd_kernel<T, VEC, false>, x->N * cs, cs, sm, st, p); }
     if (dtype == DDPM_BF16) { if (vec_ok(x, 8, 2) && vec_ok(dy, 8, 2) && vec_ok(dx, 8, 2)) GO(bf16, 8) else GO(bf16, 1) }
