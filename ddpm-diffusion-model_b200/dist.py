@@ -62,8 +62,7 @@ class GradSync:
     soon as every span that intersects it is final.  `progress(None)` / `finish()` flush the rest."""
 
     def __init__(self, flat_grad: torch.Tensor, module_spans: dict, bucket_bytes: int = 16 << 20, group=None,
-                 tail_bytes: Optional[int] = None, tail_bucket_bytes: Optional[int] = None):
-        import os
+                 tail_bytes: int = 4 << 20, tail_bucket_bytes: int = 4 << 20):
         self.g = flat_grad
         self.group = group
         self.spans = module_spans
@@ -73,10 +72,6 @@ class GradSync:
         # the overlapped backward than that saves (12.59 vs 12.50 ms per step).  One boundary at 4 MB keeps four launches:
         # [4 MB, ...) goes out while the first encoder level's backward (~1 ms) is still running, only [0, 4 MB)
         # (time MLP, in/out convolutions, first encoder level) is exposed.
-        if tail_bytes is None:
-            tail_bytes = int(os.environ.get("DDPM_B200_DP_TAIL_MB", "4")) << 20
-        if tail_bucket_bytes is None:
-            tail_bucket_bytes = int(os.environ.get("DDPM_B200_DP_TAIL_BUCKET_KB", "4096")) << 10
         self.buckets = make_buckets(flat_grad.numel(), max(1, bucket_bytes // 4), tail_bytes // 4, max(1, tail_bucket_bytes // 4))
         self.cuda = flat_grad.is_cuda
         self.comm = torch.cuda.Stream(flat_grad.device) if self.cuda else None

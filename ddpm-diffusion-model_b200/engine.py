@@ -239,6 +239,7 @@ class Exec:
         self.rng = rng
         self.prefer_tc = 1 if prefer_tc else 0
         self.use_tc = bool(prefer_tc) and dt == _lib.BF16     # tcgen05 kernels (channel padding to 16)
+        self.wgrad_side = self.use_tc                         # ResBlock weight gradients on the side stream (weight_grads)
         self.stream = _lib.stream_for(device)
 
     # ---- allocation helpers
@@ -266,28 +267,22 @@ class Exec:
 _SIDE_STREAMS: Dict[str, "torch.cuda.Stream"] = {}
 
 
-def fuse_skip_enabled() -> bool:
-    import os
-    return os.environ.get("DDPM_B200_FUSE_SKIP", "1") != "0"
-
-
-def overlap_enabled() -> bool:
-    import os
-    return os.environ.get("DDPM_B200_WGRAD_OVERLAP", "1") != "0"
-
-
 def _event_on(stream) -> "torch.cuda.Event":
     ev = torch.cuda.Event()
     ev.record(stream)
     return ev
 
 
-def wgrad_async(E: "Exec", after: "torch.cuda.Event", fn) -> "torch.cuda.Event":
-    """Run `fn` (weight-gradient launches) on the per-device side stream once `after` (a main-stream event) has
-    completed; returns the side-stream event that marks their completion.  The weight gradients are off the
-    critical path of backward (only the optimiser needs them), and the tensor-core wgrad kernel (TMA + MMA, one
-    178 KB CTA per SM) leaves the ALU/LSU and two CTA slots per SM free -- exactly what the issue-bound
-    GroupNorm backward running next on the main stream needs."""
+def weight_grads(E: "Exec", fn) -> Optional["torch.cuda.Event"]:
+    """Run `fn` (weight-gradient launches).  With `E.wgrad_side` they go to the per-device side stream once everything
+    enqueued so far on the main stream has completed, and the side-stream event that marks their completion is returned;
+    otherwise they run inline and the result is None.  The weight gradients are off the critical path of backward (only
+    the optimiser needs them), and the tensor-core wgrad kernel (TMA + MMA, one 178 KB CTA per SM) leaves the ALU/LSU
+    and two CTA slots per SM free -- exactly what the issue-bound GroupNorm backward running next on the main stream
+    needs.  Pass the result to `join` before the main stream overwrites or releases what `fn` reads."""
+    if not E.wgrad_side:
+        fn()
+        return None
     key = str(E.device)
     side = _SIDE_STREAMS.get(key)
     if side is None:
@@ -295,13 +290,19 @@ def wgrad_async(E: "Exec", after: "torch.cuda.Event", fn) -> "torch.cuda.Event":
         # CTAs must be placed first -- GroupNorm CTAs then still fit two per SM next to them, the other order does
         # not (three resident GroupNorm CTAs hold 61 K of the SM's 64 K registers)
         side = _SIDE_STREAMS[key] = torch.cuda.Stream(E.device, priority=-1)
-    side.wait_event(after)
+    side.wait_event(_event_on(torch.cuda.current_stream(E.device)))
     main_handle, E.stream = E.stream, side.cuda_stream
     try:
         fn()
     finally:
         E.stream = main_handle
     return _event_on(side)
+
+
+def join(E: "Exec", ev: Optional["torch.cuda.Event"]) -> None:
+    """Make the main stream wait for the launches behind a `weight_grads` result (nothing to wait for when it is None)."""
+    if ev is not None:
+        torch.cuda.current_stream(E.device).wait_event(ev)
 
 
 def grad_of(p: torch.nn.Parameter) -> Optional[torch.Tensor]:
@@ -554,96 +555,56 @@ def resblock_fwd(E: Exec, blk, x: Act, tbias: torch.Tensor, out: Optional[Act] =
         out = E.act(x.N, x.H, x.W, Cout)
     if isinstance(blk.skip, torch.nn.Conv2d):
         ws, _ = E.wcache.get(E, blk.skip.weight, E.dt, E.need_grad)
-        if fuse_skip_enabled() and blk.skip.bias is not None and blk.conv2.bias is not None:
-            # conv2(a2) + skip(x) as ONE implicit GEMM (K = 9*Cout + Cin): no separate 1x1 launch, no read-modify-write of
-            # `out`; the two biases are summed first (a 96..192-element add)
-            conv(E, a2, w2, out, 3, 1, 1, bias=blk.conv2.bias.detach() + blk.skip.bias.detach(), in2=x, w2pack=ws)
-        else:
-            conv(E, x, ws, out, 1, bias=blk.skip.bias)
-            conv(E, a2, w2, out, 3, 1, 1, bias=blk.conv2.bias, accum=True)
+        # conv2(a2) + skip(x) as ONE implicit GEMM (K = 9*Cout + Cin): no separate 1x1 launch, no read-modify-write of
+        # `out`; the two biases are summed first (a 96..192-element add)
+        bias = blk.conv2.bias
+        if blk.skip.bias is not None:
+            bias = blk.skip.bias if bias is None else bias.detach() + blk.skip.bias.detach()
+        conv(E, a2, w2, out, 3, 1, 1, bias=bias, in2=x, w2pack=ws)
     else:
         conv(E, a2, w2, out, 3, 1, 1, bias=blk.conv2.bias, res=x)
     saved = (x, st1, a1, h, st2, a2, p_drop, layer) if E.need_grad else None
     return out, saved
 
 
-def resblock_bwd(E: Exec, blk, saved, dout: Act, dx: Optional[Act] = None, dx_accum: bool = False):
-    """Returns (dx, dtbias [B][Cout] fp32).  `dout` may be overwritten (it becomes dx when the skip
-    is the identity and no explicit target is given)."""
-    x, st1, a1, h, st2, a2, p_drop, layer = saved
-    has_skip_conv = isinstance(blk.skip, torch.nn.Conv2d)
-    if E.use_tc and overlap_enabled() and getattr(E, "overlap_ok", True):
-        return _resblock_bwd_overlapped(E, blk, saved, dout, dx, dx_accum)
-    # conv2 (+ skip conv) parameter gradients
-    wgrad(E, a2, dout, blk.conv2.weight, 3, 1, 1, bias=blk.conv2.bias)
-    _, w2d = E.wcache.get(E, blk.conv2.weight, E.dt, True)
-    da2 = conv(E, dout, w2d, E.act(x.N, x.H, x.W, blk.out_ch), 3, 1, 1)
-    dtb = E.f32(x.N, blk.out_ch)
-    # in place (dh overwrites da2); the same launch emits d(time bias) and d(conv1.bias)
-    dh = gn_bwd(E, h, st2, blk.norm2, 1, p_drop, layer, da2, da2, False, colsum_nc=dtb, colsum_bias=blk.conv1.bias,
-                dy_scratch=True)
-    wgrad(E, a1, dh, blk.conv1.weight, 3, 1, 1)
-    _, w1d = E.wcache.get(E, blk.conv1.weight, E.dt, True)
-    da1 = conv(E, dh, w1d, E.act(x.N, x.H, x.W, blk.in_ch), 3, 1, 1)
-    if has_skip_conv:
-        wgrad(E, x, dout, blk.skip.weight, 1, bias=blk.skip.bias)
-        _, wsd = E.wcache.get(E, blk.skip.weight, E.dt, True)
-        if dx is None:
-            dx, dx_accum = E.act(x.N, x.H, x.W, blk.in_ch), False
-        conv(E, dout, wsd, dx, 1, accum=dx_accum)
-        gn_bwd(E, x, st1, blk.norm1, 1, 0.0, 0, da1, dx, True, dy_scratch=True)
-    else:
-        if dx is None:
-            dx = gn_bwd(E, x, st1, blk.norm1, 1, 0.0, 0, da1, dout, True, dy_scratch=True)       # dout += gn_bwd -> dx
-        else:
-            gn_bwd(E, x, st1, blk.norm1, 1, 0.0, 0, da1, dx, dx_accum, dy_scratch=True)
-            add(E, dx, dout, dx)
-    return dx, dtb
-
-
-def _resblock_bwd_overlapped(E: Exec, blk, saved, dout: Act, dx: Optional[Act], dx_accum: bool):
-    """Same arithmetic as the serial path; the three weight-gradient launches run on the side stream, each paired
-    with the GroupNorm backward that follows on the main stream:
+def resblock_bwd(E: Exec, blk, saved, dout: Act):
+    """Returns (dx, dtbias [B][Cout] fp32).  `dout` is overwritten (it becomes dx when the skip is the identity).
+    The three weight-gradient launches go through `weight_grads`; on the side stream each is paired with the GroupNorm
+    backward that follows on the main stream:
         main:  dgrad(conv2) | gn_bwd(norm2) | dgrad(conv1) [skip dgrad] | gn_bwd(norm1)
         side:               | wgrad(conv2)[,skip]          |            | wgrad(conv1)
-    Hazards: wgrad(conv2/skip) read `dout`, which gn_bwd(norm1) overwrites -> main waits for them first; wgrad(conv1)
-    reads dh / a1, which go back to the buffer pool when this function returns -> main waits before returning."""
+    Hazards: wgrad(conv2/skip) read `dout`, which gn_bwd(norm1) overwrites -> main joins them first; wgrad(conv1)
+    reads dh / a1, which go back to the buffer pool when this function returns -> main joins it before returning."""
     x, st1, a1, h, st2, a2, p_drop, layer = saved
     has_skip_conv = isinstance(blk.skip, torch.nn.Conv2d)
-    main = torch.cuda.current_stream(E.device)
-    # gradient buffers that do not exist yet are created (zero-filled) on the MAIN stream, before the fork events
+    # gradient buffers that do not exist yet are created (zero-filled) on the MAIN stream, before any fork
     for prm in (blk.conv2.weight, blk.conv2.bias, blk.conv1.weight) + ((blk.skip.weight, blk.skip.bias) if has_skip_conv else ()):
         if prm is not None:
             grad_of(prm)
     _, w2d = E.wcache.get(E, blk.conv2.weight, E.dt, True)
     da2 = conv(E, dout, w2d, E.act(x.N, x.H, x.W, blk.out_ch), 3, 1, 1)
 
-    def side1():
+    def conv2_skip_wgrad():
         wgrad(E, a2, dout, blk.conv2.weight, 3, 1, 1, bias=blk.conv2.bias)
         if has_skip_conv:
             wgrad(E, x, dout, blk.skip.weight, 1, bias=blk.skip.bias)
-    s1 = wgrad_async(E, _event_on(main), side1)
+    s1 = weight_grads(E, conv2_skip_wgrad)
     dtb = E.f32(x.N, blk.out_ch)
+    # in place (dh overwrites da2); the same launch emits d(time bias) and d(conv1.bias)
     dh = gn_bwd(E, h, st2, blk.norm2, 1, p_drop, layer, da2, da2, False, colsum_nc=dtb, colsum_bias=blk.conv1.bias,
                 dy_scratch=True)
     _, w1d = E.wcache.get(E, blk.conv1.weight, E.dt, True)
     da1 = conv(E, dh, w1d, E.act(x.N, x.H, x.W, blk.in_ch), 3, 1, 1)
     if has_skip_conv:
         _, wsd = E.wcache.get(E, blk.skip.weight, E.dt, True)
-        if dx is None:
-            dx, dx_accum = E.act(x.N, x.H, x.W, blk.in_ch), False
-        conv(E, dout, wsd, dx, 1, accum=dx_accum)
-    s2 = wgrad_async(E, _event_on(main), lambda: wgrad(E, a1, dh, blk.conv1.weight, 3, 1, 1))
-    main.wait_event(s1)                                   # dout is about to be overwritten / handed on
+        dx = conv(E, dout, wsd, E.act(x.N, x.H, x.W, blk.in_ch), 1)
+    s2 = weight_grads(E, lambda: wgrad(E, a1, dh, blk.conv1.weight, 3, 1, 1))
+    join(E, s1)                                           # dout is about to be overwritten / handed on
     if has_skip_conv:
         gn_bwd(E, x, st1, blk.norm1, 1, 0.0, 0, da1, dx, True, dy_scratch=True)
     else:
-        if dx is None:
-            dx = gn_bwd(E, x, st1, blk.norm1, 1, 0.0, 0, da1, dout, True, dy_scratch=True)       # dout += gn_bwd -> dx
-        else:
-            gn_bwd(E, x, st1, blk.norm1, 1, 0.0, 0, da1, dx, dx_accum, dy_scratch=True)
-            add(E, dx, dout, dx)
-    main.wait_event(s2)                                   # dh / a1 / a2 are recycled by the caller from here on
+        dx = gn_bwd(E, x, st1, blk.norm1, 1, 0.0, 0, da1, dout, True, dy_scratch=True)           # dout += gn_bwd -> dx
+    join(E, s2)                                           # dh / a1 / a2 are recycled by the caller from here on
     return dx, dtb
 
 
@@ -667,7 +628,8 @@ def attn_fwd(E: Exec, blk, x: Act, out: Optional[Act] = None):
     return out, saved
 
 
-def attn_bwd(E: Exec, blk, saved, dout: Act, dx: Optional[Act] = None, dx_accum: bool = False) -> Act:
+def attn_bwd(E: Exec, blk, saved, dout: Act) -> Act:
+    """Returns dx; `dout` is overwritten (dout += gn_bwd -> dx)."""
     x, st, a, qkv, o, lse = saved
     heads, d = blk.num_heads, blk.head_dim
     inner = heads * d
@@ -684,10 +646,7 @@ def attn_bwd(E: Exec, blk, saved, dout: Act, dx: Optional[Act] = None, dx_accum:
     wgrad(E, a, dqkv, blk.qkv.weight, 1)
     _, wqd = E.wcache.get(E, blk.qkv.weight, E.dt, True)
     da = conv(E, dqkv, wqd, E.act(x.N, x.H, x.W, x.C), 1)
-    if dx is None:
-        return gn_bwd(E, x, st, blk.norm, 0, 0.0, 0, da, dout, True, dy_scratch=True)
-    gn_bwd(E, x, st, blk.norm, 0, 0.0, 0, da, dx, dx_accum, dy_scratch=True)
-    return add(E, dx, dout, dx)
+    return gn_bwd(E, x, st, blk.norm, 0, 0.0, 0, da, dout, True, dy_scratch=True)
 
 
 # ----------------------------------------------------------------------------------------------
@@ -719,11 +678,6 @@ def down_bwd(E: Exec, mod, saved, dout: Act, dx: Optional[Act], dx_accum: bool) 
     return dx
 
 
-def fold_upsample_enabled() -> bool:
-    import os
-    return os.environ.get("DDPM_B200_FOLD_UPSAMPLE", "1") != "0"
-
-
 def up_fwd(E: Exec, mod, x: Act, out: Optional[Act] = None):
     """nearest x2 + conv3x3 (unet_backbone.py:56-64).  On the tensor-core path the up-sampling is folded into the
     convolution: each of the four output phases (2y+py, 2x+px) is a 2x2-tap convolution of the LOW-resolution input with
@@ -732,10 +686,10 @@ def up_fwd(E: Exec, mod, x: Act, out: Optional[Act] = None):
     up-sampled tensor has to exist for the weight / data gradients and folding the forward alone measured no gain
     (12.08 vs 12.02 ms per step), so training keeps the single 3x3 launch."""
     cout = mod.conv.out_channels
-    fold = (E.use_tc and not E.need_grad and fold_upsample_enabled() and x.C % 16 == 0 and cout % 16 == 0
+    fold = (E.use_tc and not E.need_grad and x.C % 16 == 0 and cout % 16 == 0
             and x.W + 2 <= 300 and x.pitch % 8 == 0 and x.halo == 1)
     u = None
-    if E.need_grad or not fold:
+    if not fold:
         u = E.act(x.N, 2 * x.H, 2 * x.W, x.C)
         _lib.call("ddpm_upsample2x", C.byref(x.desc()), C.byref(u.desc()), E.dt, E.stream)
     if out is None:
@@ -750,14 +704,13 @@ def up_fwd(E: Exec, mod, x: Act, out: Optional[Act] = None):
     return out, (u if E.need_grad else None)
 
 
-def up_bwd(E: Exec, mod, saved, dout: Act, dx: Optional[Act] = None, dx_accum: bool = False) -> Act:
+def up_bwd(E: Exec, mod, saved, dout: Act) -> Act:
     u = saved
     wgrad(E, u, dout, mod.conv.weight, 3, 1, 1, bias=mod.conv.bias)
     _, wd = E.wcache.get(E, mod.conv.weight, E.dt, True)
     du = conv(E, dout, wd, E.act(u.N, u.H, u.W, u.C), 3, 1, 1)
-    if dx is None:
-        dx, dx_accum = E.act(u.N, u.H // 2, u.W // 2, u.C), False
-    _lib.call("ddpm_upsample2x_bwd", C.byref(du.desc()), C.byref(dx.desc()), E.dt, 1 if dx_accum else 0, E.stream)
+    dx = E.act(u.N, u.H // 2, u.W // 2, u.C)
+    _lib.call("ddpm_upsample2x_bwd", C.byref(du.desc()), C.byref(dx.desc()), E.dt, 0, E.stream)
     return dx
 
 
@@ -928,7 +881,8 @@ def unet_backward(E: Exec, model, saved, dy: torch.Tensor, need_dx: bool, progre
     B = saved["xshape"][0]
     # The weight-gradient side stream pays when kernels are short (64 px, B=128: 12.10 vs 12.21 ms per step); with the long
     # kernels of the 256-px model it only adds contention (CelebA256, B=32: 474 vs 486 img/s over five runs each).
-    E.overlap_ok = B * saved["xshape"][2] * saved["xshape"][3] <= (1 << 20)
+    if B * saved["xshape"][2] * saved["xshape"][3] > (1 << 20):
+        E.wgrad_side = False
     rbs = saved["rbs"]
     dtemb: Optional[torch.Tensor] = None
     temb = saved["temb"]

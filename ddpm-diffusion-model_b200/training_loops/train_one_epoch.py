@@ -195,7 +195,6 @@ def _staged_batches(dataloader, dev, max_batches):
         st = _COPY_STREAMS[key] = {"stream": torch.cuda.Stream(dev), "ring": {}}
     cs, rings = st["stream"], st["ring"]
     it = iter(dataloader)
-    ahead = os.environ.get("DDPM_B200_PREFETCH", "1") != "0"
 
     def stage(i):
         if (max_batches is not None) and (i >= max_batches):
@@ -204,7 +203,7 @@ def _staged_batches(dataloader, dev, max_batches):
             x, y = next(it)
         except StopIteration:
             return None
-        if ahead and isinstance(x, torch.Tensor) and x.device.type == "cpu" and x.is_pinned():
+        if isinstance(x, torch.Tensor) and x.device.type == "cpu" and x.is_pinned():
             rk = (tuple(x.shape), x.dtype)
             ring = rings.get(rk)
             if ring is None:
@@ -286,7 +285,7 @@ class _GraphStep:
             return t
         POOL.get = _recording_get
         try:
-            with torch.cuda.graph(g, capture_error_mode=os.environ.get("DDPM_B200_GRAPH_CAPTURE_MODE", "global")):
+            with torch.cuda.graph(g, capture_error_mode="global"):
                 whole()
         finally:
             del POOL.get                                  # back to the class method
@@ -384,11 +383,10 @@ def train_one_epoch(model, diffusion, dataloader, optimizer, *, scaler=None, ema
 
     loss_sum = torch.zeros((), dtype=torch.float32, device=dev)
     _TRACE.reset()
-    # one-graph-per-step path (see _GraphStep): only when a step is a pure function of device state
-    # (data parallel: the bucketed NCCL all-reduces are captured with the step -- every rank captures at the same step, the
-    # collectives replay in the same order; DDPM_B200_TRAIN_GRAPH_DP=0 keeps multi-process runs eager)
-    dp_graph = world == 1 or os.environ.get("DDPM_B200_TRAIN_GRAPH_DP", "0") == "1"
-    graph_ok = (_graph_enabled() and dp_graph and grad_accum_steps == 1 and fused.fusable and on_oom == "skip"
+    # one-graph-per-step path (see _GraphStep): only when a step is a pure function of device state, and only in a single
+    # process -- capturing the bucketed NCCL all-reduces with the step hung on 2 GPUs (DESIGN §6.3), so multi-process runs
+    # stay eager
+    graph_ok = (_graph_enabled() and world == 1 and grad_accum_steps == 1 and fused.fusable and on_oom == "skip"
                 and not ((base_lr is not None) and (warmup_steps is not None) and (warmup_steps > 0) and global_step < warmup_steps)
                 and not getattr(model, "_ddpm_train_graph_failed", False) and _pure_step(model, diffusion))
     gcache = getattr(model, "_ddpm_train_graphs", None)   # key -> {"key", "warm", "gs"}; a few configurations stay captured
@@ -550,8 +548,6 @@ def train_one_epoch(model, diffusion, dataloader, optimizer, *, scaler=None, ema
         x = loss = None                                   # noqa: F841  (drop the last iteration's tensors)
 
         def _body(xs):
-            if sync is not None:
-                sync.begin()
             tt = diffusion.sample_timesteps(Bc, device=dev)
             with autocast_ctx(device="cuda", enabled=bool(use_autocast), dtype="bf16"):
                 ls = diffusion.loss_simple(model, xs, tt)
@@ -559,8 +555,6 @@ def train_one_epoch(model, diffusion, dataloader, optimizer, *, scaler=None, ema
                 scaler.scale(ls).backward()
             else:
                 ls.backward()
-            if sync is not None:
-                sync.finish()
             fused.run(scaler if use_scaler else None, use_scaler, grad_clip, ema)
             return ls.detach().float()
         try:

@@ -340,11 +340,12 @@ def test_grad_norm_diagnostic_uses_the_scale_of_its_own_step():
 
 
 @pytest.mark.parametrize("case", [(2, 32, 32, 8, 8), (3, 192, 192, 16, 16), (2, 192, 192, 32, 32), (1, 128, 128, 128, 128), (5, 64, 64, 4, 4)])
-def test_upsample_folded_into_the_conv_gather(case, monkeypatch):
+def test_upsample_folded_into_the_conv_gather(case):
     """Upsample = nearest x2 + conv3x3 (unet_backbone.py:56-64) on the tensor-core path: four 2x2-tap phase convolutions
     of the LOW-resolution input with pre-summed weights (DDPM_CONV_UP2X_PHASE) against (i) ATen fp32 on the bf16-rounded
-    input and (ii) the materialising path (up-sample kernel + 3x3 convolution).  The phase weights are summed in fp32 and
-    rounded once, the reference rounds each of the nine weights: bf16 tolerance 1e-2."""
+    input and (ii) the materialising path (up-sample kernel + 3x3 convolution), which runs whenever gradients are needed.
+    The phase weights are summed in fp32 and rounded once, the reference rounds each of the nine weights: bf16 tolerance
+    1e-2."""
     from ddpm_diffusion_model_b200 import _lib, engine
     from ddpm_diffusion_model_b200.model.unet_backbone import Upsample
     import torch.nn.functional as F
@@ -362,9 +363,11 @@ def test_upsample_folded_into_the_conv_gather(case, monkeypatch):
     torch.cuda.synchronize()
     assert _lib.launch_count(reset=True) == 5                                   # the weight pack (first use) + four phase launches
     assert saved is None
-    monkeypatch.setenv("DDPM_B200_FOLD_UPSAMPLE", "0")
-    out2, _ = engine.up_fwd(E, mod, x, None)
+    # with gradients the materialising path runs (backward needs the up-sampled tensor anyway; measured: no gain from folding)
+    Eg = engine.Exec(dev(), _lib.BF16, True, True)
+    out2, u = engine.up_fwd(Eg, mod, x, None)
     torch.cuda.synchronize()
+    assert u is not None
     xr = x.interior().float().permute(0, 3, 1, 2)
     ref = F.conv2d(F.interpolate(xr, scale_factor=2, mode="nearest"), mod.conv.weight.detach().bfloat16().float(), mod.conv.bias, padding=1)
     got = out.interior().float().permute(0, 3, 1, 2)
@@ -374,11 +377,45 @@ def test_upsample_folded_into_the_conv_gather(case, monkeypatch):
     full = wide.buf.t.float()
     assert float(full[..., :16].abs().max()) == 0 and float(full[..., 16 + Co:].abs().max()) == 0
     assert float(full[:, 0].abs().max() + full[:, -1].abs().max() + full[:, :, 0].abs().max() + full[:, :, -1].abs().max()) == 0
-    # with gradients the materialising path runs (backward needs the up-sampled tensor anyway; measured: no gain from folding)
-    Eg = engine.Exec(dev(), _lib.BF16, True, True)
-    monkeypatch.setenv("DDPM_B200_FOLD_UPSAMPLE", "1")
-    out3, u = engine.up_fwd(Eg, mod, x, None)
-    assert u is not None and rel(out3.interior().float(), out.interior().float()) < 1e-2
+
+
+@pytest.mark.parametrize("cin,cout", [(64, 96), (96, 96)])
+def test_resblock_backward_inline_and_side_stream_schedules_agree(cin, cout):
+    """engine.resblock_bwd with its weight gradients inline on the main stream and on the side stream (Exec.wgrad_side),
+    bf16, dropout on, skip convolution and identity skip.  Tensor-core weight gradients are bit-stable; the fp32-atomic
+    GroupNorm and bias gradients and the time-bias column sum may reorder."""
+    from ddpm_diffusion_model_b200 import _lib, engine
+    from ddpm_diffusion_model_b200.model.unet_backbone import ResBlock
+    torch.manual_seed(4)
+    N, H, W, tdim = 4, 32, 32, 128
+    blk = ResBlock(cin, cout, tdim, dropout=0.1).to(dev()).train()
+    x = torch.randn(N, cin, H, W, device=dev())
+    tb = torch.randn(N, cout, device=dev())
+    dy = torch.randn(N, cout, H, W, device=dev())
+    rng = torch.tensor([7, 1], dtype=torch.int64, device=dev())
+    assert engine.Exec(dev(), _lib.BF16, True, True).wgrad_side                 # the default for bf16
+    res = {}
+    for side in (False, True):
+        for p in blk.parameters():
+            p.grad = None
+        E = engine.Exec(dev(), _lib.BF16, True, True, rng=rng)
+        E.wgrad_side = side
+        _, sv = engine.resblock_fwd(E, blk, engine.to_nhwc(E, x), tb, None, 1)
+        dx, dtb = engine.resblock_bwd(E, blk, sv, engine.to_nhwc(E, dy))
+        torch.cuda.synchronize()
+        res[side] = (dx.interior().float(), dtb.clone(),
+                     {k: p.grad.clone() for k, p in blk.named_parameters() if p.grad is not None})
+    (dx0, dtb0, g0), (dx1, dtb1, g1) = res[False], res[True]
+    assert rel(dx1, dx0) <= 1e-6, rel(dx1, dx0)
+    assert rel(dtb1, dtb0) <= 1e-6, rel(dtb1, dtb0)
+    expect = {"conv1.weight", "conv1.bias", "conv2.weight", "conv2.bias", "norm1.weight", "norm1.bias", "norm2.weight",
+              "norm2.bias"} | ({"skip.weight", "skip.bias"} if cin != cout else set())
+    assert set(g0) == set(g1) == expect
+    for k in expect:
+        if k in ("conv1.weight", "conv2.weight", "skip.weight"):
+            assert torch.equal(g1[k], g0[k]), k
+        else:
+            assert rel(g1[k], g0[k]) <= 1e-6, (k, rel(g1[k], g0[k]))
 
 
 def test_train_one_epoch_stages_pinned_host_batches_ahead_without_changing_results():

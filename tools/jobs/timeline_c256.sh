@@ -3,6 +3,5 @@ cd "$(dirname "$0")/../.."
 mkdir -p gpurun_out
 python tools/step_timeline.py 32 4 celeba256 > gpurun_out/r2_step_timeline_celeba256.txt 2>&1
 head -30 gpurun_out/r2_step_timeline_celeba256.txt
-DDPM_B200_WGRAD_OVERLAP=0 python tools/step_timeline.py 32 4 celeba256 2>&1 | head -3
 python tools/step_timeline.py 128 6 low64 > gpurun_out/r2_step_timeline_low64.txt 2>&1
 head -12 gpurun_out/r2_step_timeline_low64.txt
