@@ -101,7 +101,7 @@ extern "C" int ddpm_attn_fwd(const ddpm_tensor* qkv, const ddpm_tensor* out, int
     if (!tensor_ok(qkv) || !tensor_ok(out) || !lse || heads <= 0 || d <= 0 || d > DMAX) return DDPM_E_ARG;
     if (qkv->C != 3 * heads * d || out->C != heads * d || out->N != qkv->N || out->H != qkv->H || out->W != qkv->W) return DDPM_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
-    // tcgen05 forward for the UNet's shapes (<= 256 tokens, head_dim 32 / 64, bf16); everything else on the CUDA cores
+    // tcgen05 forward for bf16, head_dim 32 / 64 / 128, W <= 128; everything else on the CUDA cores
     if (!ddpm_force_simt_flag() && attn_tc_supported(qkv, out, heads, d, dtype)) return attn_tc_launch(qkv, out, heads, d, lse, st);
     int N = qkv->H * qkv->W;
     dim3 grid(ceil_div(N, 4 * QPW), heads, qkv->N);
@@ -302,10 +302,16 @@ extern "C" int ddpm_attn_bwd(const ddpm_tensor* qkv, const ddpm_tensor* out, con
     if (!tensor_ok(qkv) || !tensor_ok(out) || !tensor_ok(dout) || !tensor_ok(dqkv) || !lse || !scratch) return DDPM_E_ARG;
     if (heads <= 0 || d <= 0 || d > DMAX || qkv->C != 3 * heads * d || dqkv->C != qkv->C || out->C != heads * d || dout->C != out->C) return DDPM_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
-    // tcgen05 backward with P recomputed from lse (no N x N scratch) for the UNet's shapes; CUDA cores otherwise
-    if (!ddpm_force_simt_flag() && attn_tc_supported(qkv, out, heads, d, dtype) && attn_tc_supported(dqkv, dout, heads, d, dtype) &&
-        dout->halo == qkv->halo)
+    // tcgen05 backward with P recomputed from lse (no N x N scratch) whenever qkv / out are eligible; CUDA cores otherwise.
+    // ddpm_attn_bwd_scratch_floats sizes the scratch from qkv / out alone, so dout / dqkv that the tensor-core kernels cannot
+    // take are rejected rather than sent to the CUDA-core kernels, which would write N x N matrices into that scratch.
+    if (!ddpm_force_simt_flag() && attn_tc_supported(qkv, out, heads, d, dtype)) {
+        if (!attn_tc_supported(dqkv, dout, heads, d, dtype) || dout->halo != qkv->halo) return DDPM_E_ARG;
+        const ddpm_tensor* same[3] = {out, dout, dqkv};
+        for (const ddpm_tensor* t : same)
+            if (t->N != qkv->N || t->H != qkv->H || t->W != qkv->W) return DDPM_E_ARG;
         return attn_tc_bwd_launch(qkv, out, dout, lse, dqkv, heads, d, scratch, st);
+    }
     int N = qkv->H * qkv->W;
     float* Pm = scratch; float* dSm = scratch + (size_t)qkv->N * heads * N * N;
     float scale = 1.0f / sqrtf((float)d);

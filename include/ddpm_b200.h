@@ -260,13 +260,16 @@ int ddpm_pack_weights_batched(const ddpm_pack_entry* entries_dev, int n, void* s
  * the four permute+contiguous copies (:63-65,72) disappear.  lse: fp32 [N][heads][H*W]. */
 int ddpm_attn_fwd(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads, int d, float* lse,
                   int dtype, void* stream);
-/* scratch: fp32 [N][heads][HW][HW] * 2 (P and dS) */
+/* scratch: ddpm_attn_bwd_scratch_floats(qkv, out, ...) fp32 elements.  When qkv / out take the tensor-core kernels, dout
+ * and dqkv must too (same geometry, 16-byte aligned, pitch a multiple of 8) and dout->halo must equal qkv->halo;
+ * otherwise the call returns DDPM_E_ARG and writes nothing. */
 int ddpm_attn_bwd(const ddpm_tensor* qkv, const ddpm_tensor* out, const ddpm_tensor* dout,
                   const float* lse, const ddpm_tensor* dqkv, int heads, int d, float* scratch,
                   int dtype, void* stream);
-/* fp32 elements of `scratch` ddpm_attn_bwd needs for this problem: N*N-sized P and dS matrices for the CUDA-core kernels,
- * one value per (image, head, query) for the tensor-core kernels (bf16, <= 256 tokens, head_dim 32 / 64), which recompute
- * P from the forward's log-sum-exp. */
+/* fp32 elements of `scratch` ddpm_attn_bwd needs for this problem, from qkv / out alone: N*N-sized P and dS matrices
+ * ([N][heads][HW][HW] * 2) for the CUDA-core kernels, one value per (image, head, query) for the tensor-core kernels
+ * (bf16, head_dim 32 / 64 / 128, W <= 128, any H; 16-byte aligned, pitch a multiple of 8), which recompute P from the
+ * forward's log-sum-exp. */
 int64_t ddpm_attn_bwd_scratch_floats(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads, int d, int dtype);
 
 /* ---------------- optimiser-side parameter pass -------------------------------------------- */
