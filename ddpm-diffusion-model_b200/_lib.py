@@ -10,7 +10,7 @@ import os
 
 from . import build as _build
 
-F32, BF16 = 0, 1
+F32, BF16, F16 = 0, 1, 2
 CLAMP_X0, DYN_THRESH = 1, 2
 CONV_NORMAL, CONV_TRANSPOSED, CONV_UP2X_PHASE = 0, 1, 2
 EPI_ACCUM, EPI_DSILU = 1, 2

@@ -1,5 +1,5 @@
 // ddpm_conv / ddpm_conv_wgrad: argument validation and dispatch between the tcgen05 tensor-core
-// kernels (conv_tc.cu, bf16) and the CUDA-core kernels (conv_simt.cu, fp32 + every odd shape).
+// kernels (conv_tc.cu, bf16 / fp16) and the CUDA-core kernels (conv_simt.cu, fp32 + every odd shape).
 #include "common.cuh"
 
 int conv_simt_launch(const ddpm_conv_args* a, cudaStream_t st);
@@ -15,7 +15,7 @@ int ddpm_force_simt_flag() { return g_force_simt; }
 
 extern "C" int ddpm_conv(const ddpm_conv_args* a, void* stream) {
     if (!a || !tensor_ok(&a->in) || !tensor_ok(&a->out) || !a->w) return DDPM_E_ARG;
-    if (a->dtype != DDPM_F32 && a->dtype != DDPM_BF16) return DDPM_E_ARG;
+    if (a->dtype != DDPM_F32 && a->dtype != DDPM_BF16 && a->dtype != DDPM_F16) return DDPM_E_ARG;
     if (a->KH <= 0 || a->KW <= 0 || a->stride <= 0 || a->pad < 0) return DDPM_E_ARG;
     if (a->in.N != a->out.N) return DDPM_E_ARG;
     if (a->mode == DDPM_CONV_NORMAL) {
@@ -53,7 +53,7 @@ extern "C" int ddpm_conv(const ddpm_conv_args* a, void* stream) {
 
 extern "C" int ddpm_conv_wgrad(const ddpm_wgrad_args* a, void* stream) {
     if (!a || !tensor_ok(&a->act) || !tensor_ok(&a->dy) || !a->dw) return DDPM_E_ARG;
-    if (a->dtype != DDPM_F32 && a->dtype != DDPM_BF16) return DDPM_E_ARG;
+    if (a->dtype != DDPM_F32 && a->dtype != DDPM_BF16 && a->dtype != DDPM_F16) return DDPM_E_ARG;
     if (a->KH <= 0 || a->KW <= 0 || a->stride <= 0 || a->pad < 0 || a->act.N != a->dy.N) return DDPM_E_ARG;
     if (a->dy.H != (a->act.H + 2 * a->pad - a->KH) / a->stride + 1) return DDPM_E_ARG;
     if (a->dy.W != (a->act.W + 2 * a->pad - a->KW) / a->stride + 1) return DDPM_E_ARG;

@@ -94,15 +94,15 @@ __global__ void __launch_bounds__(AT) attn_fwd_kernel(TV qkv, TV out, int heads,
 }
 
 int attn_tc_supported(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads, int d, int dtype);      // attn_tc.cu
-int attn_tc_launch(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads, int d, float* lse, cudaStream_t st);
+int attn_tc_launch(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads, int d, float* lse, int dtype, cudaStream_t st);
 int ddpm_force_simt_flag();
 extern "C" int ddpm_attn_fwd(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads, int d, float* lse,
                              int dtype, void* stream) {
     if (!tensor_ok(qkv) || !tensor_ok(out) || !lse || heads <= 0 || d <= 0 || d > DMAX) return DDPM_E_ARG;
     if (qkv->C != 3 * heads * d || out->C != heads * d || out->N != qkv->N || out->H != qkv->H || out->W != qkv->W) return DDPM_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
-    // tcgen05 forward for bf16, head_dim 32 / 64 / 128, W <= 128; everything else on the CUDA cores
-    if (!ddpm_force_simt_flag() && attn_tc_supported(qkv, out, heads, d, dtype)) return attn_tc_launch(qkv, out, heads, d, lse, st);
+    // tcgen05 forward for bf16 / fp16, head_dim 32 / 64 / 128, W <= 128; everything else on the CUDA cores
+    if (!ddpm_force_simt_flag() && attn_tc_supported(qkv, out, heads, d, dtype)) return attn_tc_launch(qkv, out, heads, d, lse, dtype, st);
     int N = qkv->H * qkv->W;
     dim3 grid(ceil_div(N, 4 * QPW), heads, qkv->N);
     size_t smem = sizeof(float) * (2 * KT * (d + 1) + 4 * d + 4 * KT);
@@ -113,6 +113,9 @@ extern "C" int ddpm_attn_fwd(const ddpm_tensor* qkv, const ddpm_tensor* out, int
     } else if (dtype == DDPM_BF16) {
         CUDA_TRY(cudaFuncSetAttribute(attn_fwd_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         CUDA_TRY(launch_kernel(attn_fwd_kernel<bf16>, grid, dim3(AT), smem, st, TV(*qkv), TV(*out), heads, d, scale, lse));
+    } else if (dtype == DDPM_F16) {
+        CUDA_TRY(cudaFuncSetAttribute(attn_fwd_kernel<f16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        CUDA_TRY(launch_kernel(attn_fwd_kernel<f16>, grid, dim3(AT), smem, st, TV(*qkv), TV(*out), heads, d, scale, lse));
     } else return DDPM_E_ARG;
     LAUNCH_OK();
     return 0;
@@ -286,7 +289,7 @@ __global__ void __launch_bounds__(AT) attn_bwd_kv_kernel(TV qkv, TV dout, TV dqk
 
 int64_t attn_tc_bwd_scratch_floats(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads, int d, int dtype);      // attn_tc.cu
 int attn_tc_bwd_launch(const ddpm_tensor* qkv, const ddpm_tensor* out, const ddpm_tensor* dout, const float* lse,
-                       const ddpm_tensor* dqkv, int heads, int d, float* scratch, cudaStream_t st);
+                       const ddpm_tensor* dqkv, int heads, int d, float* scratch, int dtype, cudaStream_t st);
 extern "C" int64_t ddpm_attn_bwd_scratch_floats(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads, int d, int dtype) {
     if (!tensor_ok(qkv) || !tensor_ok(out) || heads <= 0 || d <= 0) return 0;
     const int64_t N = (int64_t)qkv->H * qkv->W;
@@ -310,7 +313,7 @@ extern "C" int ddpm_attn_bwd(const ddpm_tensor* qkv, const ddpm_tensor* out, con
         const ddpm_tensor* same[3] = {out, dout, dqkv};
         for (const ddpm_tensor* t : same)
             if (t->N != qkv->N || t->H != qkv->H || t->W != qkv->W) return DDPM_E_ARG;
-        return attn_tc_bwd_launch(qkv, out, dout, lse, dqkv, heads, d, scratch, st);
+        return attn_tc_bwd_launch(qkv, out, dout, lse, dqkv, heads, d, scratch, dtype, st);
     }
     int N = qkv->H * qkv->W;
     float* Pm = scratch; float* dSm = scratch + (size_t)qkv->N * heads * N * N;
@@ -325,7 +328,7 @@ extern "C" int ddpm_attn_bwd(const ddpm_tensor* qkv, const ddpm_tensor* out, con
         LAUNCH_OK(); \
         CUDA_TRY(launch_kernel(attn_bwd_kv_kernel<T>, gk, dim3(AT), smk, st, TV(*qkv), TV(*dout), TV(*dqkv), heads, d, scale, (const float*)Pm, (const float*)dSm)); \
         LAUNCH_OK(); }
-    if (dtype == DDPM_F32) GO(float) else if (dtype == DDPM_BF16) GO(bf16) else return DDPM_E_ARG;
+    if (dtype == DDPM_F32) GO(float) else if (dtype == DDPM_BF16) GO(bf16) else if (dtype == DDPM_F16) GO(f16) else return DDPM_E_ARG;
 #undef GO
     return 0;
 }

@@ -1,4 +1,5 @@
-// tcgen05 / TMEM spatial self-attention (attention.py:56-74), bf16, head_dim 32 / 64 / 128, any H x W with W <= 128.
+// tcgen05 / TMEM spatial self-attention (attention.py:56-74), bf16 or fp16 (a template parameter, format from Fmt16),
+// head_dim 32 / 64 / 128, any H x W with W <= 128.
 // Tiles are R = floor(128 / W) whole image rows (<= 128 tokens); a tile may be ragged (R*W < 128) and the last one partial.
 // Q, K, V (and dO) arrive by TMA straight out of the NHWC `qkv` tensor (4-D maps over (channel, x, y, image): the halo
 // pixels are not in the box, the permute + contiguous copies of attention.py:63-65 never exist).
@@ -7,7 +8,7 @@
 //   S_j = Q K_j^T  tcgen05.mma, M = 128 queries, N = the key tile padded to 16, K = head_dim; Q and K as 16-channel K-major
 //                  chunks (SWIZZLE_32B); S double-buffered in tensor memory (columns 0 / 128) so S_{j+1} is computed while
 //                  the softmax warps work on S_j; K / V double-buffered in shared memory
-//   P_j            128 threads, one query row each: running max m and sum l, P_j = exp(S_j - m) as bf16 K-major chunks
+//   P_j            128 threads, one query row each: running max m and sum l, P_j = exp(S_j - m) as 16-bit K-major chunks
 //   O += P_j V_j   B = V read MN-major (head_dim contiguous, 64-channel SWIZZLE_128B boxes; head_dim 128 = two boxes and two
 //                  N = 64 halves) into TMEM columns 256..; the softmax threads fold it into fp32 registers,
 //                  o = o * exp(m_old - m_new) + P_j V_j, and store o / l and lse = m * scale + log l.
@@ -21,8 +22,8 @@
 #include <cudaTypedefs.h>
 #include <math.h>
 
-extern int ddpm_encode_tiled_bf16(CUtensorMap* m, void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-                                  const uint32_t* box, int swizzle_bytes);      // conv_tc.cu
+extern int ddpm_encode_tiled16(CUtensorMap* m, CUtensorMapDataType type, void* base, int rank, const uint64_t* dims,
+                               const uint64_t* strides_bytes, const uint32_t* box, int swizzle_bytes);      // conv_tc.cu
 
 namespace {
 
@@ -58,7 +59,7 @@ __device__ __forceinline__ void tm_alloc(uint32_t* dst_smem, uint32_t ncols) {
 __device__ __forceinline__ void tm_dealloc(uint32_t taddr, uint32_t ncols) {
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
-__device__ __forceinline__ void mma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
+__device__ __forceinline__ void mma_f16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
         "setp.ne.b32 p, %4, 0;\n\t"
@@ -87,35 +88,35 @@ __device__ __forceinline__ uint64_t mdesc(uint32_t saddr, uint32_t lbo_bytes, ui
     d |= (uint64_t)(layout & 7) << 61;
     return d;
 }
-// instruction descriptors: bf16 x bf16 -> fp32, M = 128.  S-type: both operands K-major, N = n.  O-type: B MN-major, N = 64.
-__device__ __forceinline__ uint32_t idesc_kk(int n) { return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((128u >> 4) << 24); }
-__device__ __forceinline__ uint32_t idesc_mn64() { return (1u << 4) | (1u << 7) | (1u << 10) | (1u << 16) | ((64u >> 3) << 17) | ((128u >> 4) << 24); }
+// instruction descriptors: 16-bit x 16-bit -> fp32, M = 128.  S-type: both operands K-major, N = n.  O-type: B MN-major, N = 64.
+template <typename T> __device__ __forceinline__ uint32_t idesc_kk(int n) { return (1u << 4) | Fmt16<T>::idesc_ab | ((uint32_t)(n >> 3) << 17) | ((128u >> 4) << 24); }
+template <typename T> __device__ __forceinline__ uint32_t idesc_mn64() { return (1u << 4) | Fmt16<T>::idesc_ab | (1u << 16) | ((64u >> 3) << 17) | ((128u >> 4) << 24); }
 // K-major operand (SWIZZLE_32B, layout 6): 16-channel chunk kc of `rows` rows of 32 B, SBO = 256 B per 8-row group
 __device__ __forceinline__ uint64_t kdesc(const uint8_t* base, int kc, int rows) { return mdesc(s32(base) + (uint32_t)(kc * rows * 32), 16u, 256u, 6u); }
 // MN-major operand (SWIZZLE_128B, layout 2): 64-channel box nb of `rows` rows of 128 B, K-step kc = 16 rows
 __device__ __forceinline__ uint64_t ndesc(const uint8_t* base, int nb, int kc, int rows) {
     return mdesc(s32(base) + (uint32_t)(nb * rows * 128 + kc * 16 * 128), (uint32_t)(rows * 128), 1024u, 2u);
 }
-__device__ __forceinline__ void store_chunk_sw32(uint32_t row_addr, uint32_t sw, const float* e) {
+template <typename T> __device__ __forceinline__ void store_chunk_sw32(uint32_t row_addr, uint32_t sw, const float* e) {
     uint4 lo, hi;
-    __nv_bfloat162* pl = reinterpret_cast<__nv_bfloat162*>(&lo);
-    __nv_bfloat162* ph = reinterpret_cast<__nv_bfloat162*>(&hi);
+    typename Fmt16<T>::T2* pl = reinterpret_cast<typename Fmt16<T>::T2*>(&lo);
+    typename Fmt16<T>::T2* ph = reinterpret_cast<typename Fmt16<T>::T2*>(&hi);
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-        pl[i] = __floats2bfloat162_rn(e[2 * i], e[2 * i + 1]);
-        ph[i] = __floats2bfloat162_rn(e[8 + 2 * i], e[8 + 2 * i + 1]);
+        pl[i] = Fmt16<T>::from_f2(e[2 * i], e[2 * i + 1]);
+        ph[i] = Fmt16<T>::from_f2(e[8 + 2 * i], e[8 + 2 * i + 1]);
     }
     asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(row_addr + (0u ^ sw)), "r"(lo.x), "r"(lo.y), "r"(lo.z), "r"(lo.w) : "memory");
     asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(row_addr + (16u ^ sw)), "r"(hi.x), "r"(hi.y), "r"(hi.z), "r"(hi.w) : "memory");
 }
-__device__ __forceinline__ void store_row16(bf16* dst, const uint32_t* r, float mul) {
+template <typename T> __device__ __forceinline__ void store_row16(T* dst, const uint32_t* r, float mul) {
     uint4 lo, hi;
-    __nv_bfloat162* pl = reinterpret_cast<__nv_bfloat162*>(&lo);
-    __nv_bfloat162* ph = reinterpret_cast<__nv_bfloat162*>(&hi);
+    typename Fmt16<T>::T2* pl = reinterpret_cast<typename Fmt16<T>::T2*>(&lo);
+    typename Fmt16<T>::T2* ph = reinterpret_cast<typename Fmt16<T>::T2*>(&hi);
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-        pl[i] = __floats2bfloat162_rn(__uint_as_float(r[2 * i]) * mul, __uint_as_float(r[2 * i + 1]) * mul);
-        ph[i] = __floats2bfloat162_rn(__uint_as_float(r[8 + 2 * i]) * mul, __uint_as_float(r[8 + 2 * i + 1]) * mul);
+        pl[i] = Fmt16<T>::from_f2(__uint_as_float(r[2 * i]) * mul, __uint_as_float(r[2 * i + 1]) * mul);
+        ph[i] = Fmt16<T>::from_f2(__uint_as_float(r[8 + 2 * i]) * mul, __uint_as_float(r[8 + 2 * i + 1]) * mul);
     }
     *reinterpret_cast<uint4*>(dst) = lo;
     *reinterpret_cast<uint4*>(dst + 8) = hi;
@@ -146,7 +147,7 @@ struct AtcP {
     int zero_v;                      // ragged key tile: zero the V stages once
 };
 
-template <int D>
+template <typename T, int D>
 __global__ void __launch_bounds__(ATC_THREADS, 1) attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ,
                                                                       const __grid_constant__ CUtensorMap tmK,
                                                                       const __grid_constant__ CUtensorMap tmV, AtcP p) {
@@ -197,7 +198,7 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_fwd_tc_kernel(const __gri
         }
     } else if (warp == 1) {
         if (lane == 0) {
-            const uint32_t idesc1 = idesc_kk(g.NKp), idesc2 = idesc_mn64();
+            const uint32_t idesc1 = idesc_kk<T>(g.NKp), idesc2 = idesc_mn64<T>();
             mb_wait(bar_q, 0);
             // iteration j issues S_j, then P_{j-1} V_{j-1}: the tensor core computes the next scores while the softmax
             // warps exponentiate the current ones
@@ -209,7 +210,7 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_fwd_tc_kernel(const __gri
                     fence_after();
                     const uint8_t* kb = Ks + (size_t)s * p.kst;
                     for (int kc = 0; kc < KCH; ++kc)
-                        mma_bf16(tmem_base + (uint32_t)(j & 1) * 128u, kdesc(Qs, kc, 128), kdesc(kb, kc, g.NKp), idesc1, kc > 0 ? 1u : 0u);
+                        mma_f16(tmem_base + (uint32_t)(j & 1) * 128u, kdesc(Qs, kc, 128), kdesc(kb, kc, g.NKp), idesc1, kc > 0 ? 1u : 0u);
                     mma_commit(bar_s + (j & 1));
                 }
                 if (j >= 1) {
@@ -219,7 +220,7 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_fwd_tc_kernel(const __gri
                     const uint8_t* vb = Vs + (size_t)s * p.vst;
                     for (int nb = 0; nb < NVB; ++nb)
                         for (int kc = 0; kc < g.NKp / 16; ++kc)
-                            mma_bf16(tmem_base + o_col + (uint32_t)nb * 64u, kdesc(Ps, kc, 128), ndesc(vb, nb, kc, g.NKp), idesc2, kc > 0 ? 1u : 0u);
+                            mma_f16(tmem_base + o_col + (uint32_t)nb * 64u, kdesc(Ps, kc, 128), ndesc(vb, nb, kc, g.NKp), idesc2, kc > 0 ? 1u : 0u);
                     mma_commit(bar_o);
                     mma_commit(empty + s);
                 }
@@ -282,7 +283,7 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_fwd_tc_kernel(const __gri
                     e[i] = valid && c0 + i < kv ? exp2f(fmaf(__uint_as_float(r[i]), p.scale_log2e, -mb)) : 0.f;
                     sum += e[i];
                 }
-                store_chunk_sw32(prow + (uint32_t)(c0 >> 4) * 4096u, sw, e);
+                store_chunk_sw32<T>(prow + (uint32_t)(c0 >> 4) * 4096u, sw, e);
             }
             l = fmaf(l, corr, sum);
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");      // generic-proxy writes of P -> visible to the tensor core
@@ -297,14 +298,14 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_fwd_tc_kernel(const __gri
             const float inv = valid ? 1.0f / l : 0.f;
             const int qq = valid ? q : 0;
             const int y = qq / g.W, x = qq - y * g.W;
-            bf16* orow = p.out.at<bf16>(b, y, x, h * D);
+            T* orow = p.out.at<T>(b, y, x, h * D);
             if (valid) {
 #pragma unroll
                 for (int c0 = 0; c0 < D; c0 += 8) {
                     uint4 v;
-                    __nv_bfloat162* pv = reinterpret_cast<__nv_bfloat162*>(&v);
+                    typename Fmt16<T>::T2* pv = reinterpret_cast<typename Fmt16<T>::T2*>(&v);
 #pragma unroll
-                    for (int i = 0; i < 4; ++i) pv[i] = __floats2bfloat162_rn(o[c0 + 2 * i] * inv, o[c0 + 2 * i + 1] * inv);
+                    for (int i = 0; i < 4; ++i) pv[i] = Fmt16<T>::from_f2(o[c0 + 2 * i] * inv, o[c0 + 2 * i + 1] * inv);
                     *reinterpret_cast<uint4*>(orow + c0) = v;
                 }
                 p.lse[((size_t)b * p.heads + h) * g.N + q] = m * p.scale + logf(l);
@@ -321,10 +322,10 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_fwd_tc_kernel(const __gri
 // Backward, recomputing P from lse (no N x N scratch): two kernels with "natural" operand orientations only.
 //
 //   dq kernel, one CTA per (image, head, query tile), a loop over key tiles j:   S = Q K_j^T,  dP = dO V_j^T  (TMEM),
-//       threads (one query row each): D = dO . O,  P = exp(S*scale - lse),  dS = P * (dP - D)  -> bf16 K-major chunks,
+//       threads (one query row each): D = dO . O,  P = exp(S*scale - lse),  dS = P * (dP - D)  -> 16-bit K-major chunks,
 //       dQ += dS K_j (B = K read MN-major) in TMEM -> * scale -> dqkv[q-channels];  D is also written out for the second kernel.
 //   dkv kernel, one CTA per (image, head, key tile), a loop over query tiles i:   S^T = K Q_i^T,  dP^T = V dO_i^T,
-//       threads (one key row each): P^T and dS^T from the tile's lse / D (staged in shared memory) -> two bf16 K-major
+//       threads (one key row each): P^T and dS^T from the tile's lse / D (staged in shared memory) -> two 16-bit K-major
 //       chunk buffers, dV += P^T dO_i, dK += dS^T Q_i (B = dO / Q read MN-major, loaded into the buffers of the K-major
 //       copies once S^T and dP^T are complete) -> dqkv[v-channels], * scale -> dqkv[k-channels].
 // TMEM: S at 0, dP at `col_dp`, the accumulators at `col_acc` (after the all-keys tile of N <= 256, over S).
@@ -342,6 +343,7 @@ struct AtbP {
 
 // regions: o0 Q [kch][128][32], o1 dO [kch][128][32], o2 stages of {K32 [kch][NKp][32], V32 [kch][NKp][32], K128 [nvb][NKp][128]},
 //          o5 dS [NKp/16][128][32]
+template <typename T>
 __global__ void __launch_bounds__(ATC_THREADS, 1) attn_bwd_dq_tc_kernel(const __grid_constant__ CUtensorMap tmQt, const __grid_constant__ CUtensorMap tmGt,
                                                                          const __grid_constant__ CUtensorMap tmF32, const __grid_constant__ CUtensorMap tmF128,
                                                                          AtbP p) {
@@ -395,7 +397,7 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_bwd_dq_tc_kernel(const __
         }
     } else if (warp == 1) {
         if (lane == 0) {
-            const uint32_t idesc1 = idesc_kk(g.NKp), idesc2 = idesc_mn64();
+            const uint32_t idesc1 = idesc_kk<T>(g.NKp), idesc2 = idesc_mn64<T>();
             mb_wait(bar_in, 0);
             for (int j = 0; j < g.nit; ++j) {
                 const int s = j % p.nst;
@@ -403,16 +405,16 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_bwd_dq_tc_kernel(const __
                 mb_wait(full + s, (j / p.nst) & 1);
                 fence_after();
                 for (int kc = 0; kc < p.kch; ++kc)
-                    mma_bf16(tmem_base, kdesc(Qs, kc, 128), kdesc(st, kc, g.NKp), idesc1, kc > 0 ? 1u : 0u);
+                    mma_f16(tmem_base, kdesc(Qs, kc, 128), kdesc(st, kc, g.NKp), idesc1, kc > 0 ? 1u : 0u);
                 for (int kc = 0; kc < p.kch; ++kc)
-                    mma_bf16(tmem_base + p.col_dp, kdesc(Gs, kc, 128), kdesc(st + kbytes, kc, g.NKp), idesc1, kc > 0 ? 1u : 0u);
+                    mma_f16(tmem_base + p.col_dp, kdesc(Gs, kc, 128), kdesc(st + kbytes, kc, g.NKp), idesc1, kc > 0 ? 1u : 0u);
                 mma_commit(bar_s);
                 mb_wait(full_mn + s, (j / p.nst) & 1);
                 mb_wait(bar_ds, j & 1);              // dS_j written, S_j / dP_j read: their TMEM columns are free again
                 fence_after();
                 for (int nb = 0; nb < p.nvb; ++nb)
                     for (int kc = 0; kc < g.NKp / 16; ++kc)
-                        mma_bf16(tmem_base + p.col_acc + (uint32_t)nb * 64u, kdesc(Ss, kc, 128), ndesc(st + 2 * kbytes, nb, kc, g.NKp), idesc2,
+                        mma_f16(tmem_base + p.col_acc + (uint32_t)nb * 64u, kdesc(Ss, kc, 128), ndesc(st + 2 * kbytes, nb, kc, g.NKp), idesc2,
                                  (j > 0 || kc > 0) ? 1u : 0u);
                 mma_commit(empty + s);
             }
@@ -424,17 +426,17 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_bwd_dq_tc_kernel(const __
         const bool valid = row < g.T && q < g.N;
         const int qq = valid ? q : 0;
         const int y = qq / g.W, x = qq - y * g.W;
-        // D = dO . O for this query (bf16 token rows of `dout` / `out`), lse of the forward
+        // D = dO . O for this query (16-bit token rows of `dout` / `out`), lse of the forward
         float D = 0.f, L = 0.f;
         if (valid) {
-            const bf16* go = p.dout.at<bf16>(b, y, x, h * p.d);
-            const bf16* oo = p.out.at<bf16>(b, y, x, h * p.d);
+            const T* go = p.dout.at<T>(b, y, x, h * p.d);
+            const T* oo = p.out.at<T>(b, y, x, h * p.d);
             for (int c = 0; c < p.d; c += 8) {
                 const uint4 a = *reinterpret_cast<const uint4*>(go + c), o = *reinterpret_cast<const uint4*>(oo + c);
-                const __nv_bfloat162* ha = reinterpret_cast<const __nv_bfloat162*>(&a);
-                const __nv_bfloat162* ho = reinterpret_cast<const __nv_bfloat162*>(&o);
+                const typename Fmt16<T>::T2* ha = reinterpret_cast<const typename Fmt16<T>::T2*>(&a);
+                const typename Fmt16<T>::T2* ho = reinterpret_cast<const typename Fmt16<T>::T2*>(&o);
 #pragma unroll
-                for (int i = 0; i < 4; ++i) { const float2 fa = __bfloat1622float2(ha[i]), fo = __bfloat1622float2(ho[i]); D = fmaf(fa.x, fo.x, fmaf(fa.y, fo.y, D)); }
+                for (int i = 0; i < 4; ++i) { const float2 fa = Fmt16<T>::to_f2(ha[i]), fo = Fmt16<T>::to_f2(ho[i]); D = fmaf(fa.x, fo.x, fmaf(fa.y, fo.y, D)); }
             }
             L = p.lse[((size_t)b * p.heads + h) * g.N + q];
             p.Dbuf[((size_t)b * p.heads + h) * g.N + q] = D;
@@ -457,7 +459,7 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_bwd_dq_tc_kernel(const __
                     const float pij = exp2f(fmaf(__uint_as_float(rs[i]), p.scale_log2e, -Lb));
                     e[i] = valid && c0 + i < kv ? pij * (__uint_as_float(rp[i]) - D) : 0.f;
                 }
-                store_chunk_sw32(srow + (uint32_t)(c0 >> 4) * 4096u, sw, e);
+                store_chunk_sw32<T>(srow + (uint32_t)(c0 >> 4) * 4096u, sw, e);
             }
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             fence_before();
@@ -465,12 +467,12 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_bwd_dq_tc_kernel(const __
         }
         mb_wait(bar_o, 0);
         fence_after();
-        bf16* drow = p.dqkv.at<bf16>(b, y, x, h * p.d);
+        T* drow = p.dqkv.at<T>(b, y, x, h * p.d);
         for (int c0 = 0; c0 < p.d; c0 += 16) {
             uint32_t r[16];
             tm_ld16(lane_addr + p.col_acc + (uint32_t)c0, r);
             tm_ld_wait();
-            if (valid) store_row16(drow + c0, r, p.scale);
+            if (valid) store_row16<T>(drow + c0, r, p.scale);
         }
         fence_before();
     }
@@ -481,6 +483,7 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_bwd_dq_tc_kernel(const __
 // regions: o0 K tile [kch][128][32], o1 V tile [kch][128][32], o2 Q32 [kch][NKp][32] then Q128 [nvb][NKp][128],
 //          o3 dO32 then dO128 likewise, o4 P^T [NKp/16][128][32], o5 dS^T likewise, o6 the query tile's lse / D [2][NKp]
 //          (inside the dead K tile when there is a single query tile)
+template <typename T>
 __global__ void __launch_bounds__(ATC_THREADS, 1) attn_bwd_dkv_tc_kernel(const __grid_constant__ CUtensorMap tmKt, const __grid_constant__ CUtensorMap tmQ32,
                                                                           const __grid_constant__ CUtensorMap tmG32, const __grid_constant__ CUtensorMap tmQ128,
                                                                           const __grid_constant__ CUtensorMap tmG128, AtbP p) {
@@ -535,27 +538,27 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_bwd_dkv_tc_kernel(const _
         }
     } else if (warp == 1) {
         if (lane == 0) {
-            const uint32_t idesc1 = idesc_kk(g.NKp), idesc2 = idesc_mn64();
+            const uint32_t idesc1 = idesc_kk<T>(g.NKp), idesc2 = idesc_mn64<T>();
             const uint32_t col_dv = p.col_acc, col_dk = p.col_acc + (uint32_t)p.nvb * 64u;
             mb_wait(bar_kv, 0);
             for (int i = 0; i < g.nit; ++i) {
                 mb_wait(bar_in, i & 1);
                 fence_after();
                 for (int kc = 0; kc < p.kch; ++kc)
-                    mma_bf16(tmem_base, kdesc(Kt, kc, 128), kdesc(Qr, kc, g.NKp), idesc1, kc > 0 ? 1u : 0u);
+                    mma_f16(tmem_base, kdesc(Kt, kc, 128), kdesc(Qr, kc, g.NKp), idesc1, kc > 0 ? 1u : 0u);
                 for (int kc = 0; kc < p.kch; ++kc)
-                    mma_bf16(tmem_base + p.col_dp, kdesc(Vt, kc, 128), kdesc(Gr, kc, g.NKp), idesc1, kc > 0 ? 1u : 0u);
+                    mma_f16(tmem_base + p.col_dp, kdesc(Vt, kc, 128), kdesc(Gr, kc, g.NKp), idesc1, kc > 0 ? 1u : 0u);
                 mma_commit(bar_s);
                 mb_wait(bar_in2, i & 1);
                 mb_wait(bar_p, i & 1);
                 fence_after();
                 for (int nb = 0; nb < p.nvb; ++nb)
                     for (int kc = 0; kc < g.NKp / 16; ++kc)        // dV += P^T dO
-                        mma_bf16(tmem_base + col_dv + (uint32_t)nb * 64u, kdesc(Pt, kc, 128), ndesc(Gr, nb, kc, g.NKp), idesc2,
+                        mma_f16(tmem_base + col_dv + (uint32_t)nb * 64u, kdesc(Pt, kc, 128), ndesc(Gr, nb, kc, g.NKp), idesc2,
                                  (i > 0 || kc > 0) ? 1u : 0u);
                 for (int nb = 0; nb < p.nvb; ++nb)
                     for (int kc = 0; kc < g.NKp / 16; ++kc)        // dK += dS^T Q
-                        mma_bf16(tmem_base + col_dk + (uint32_t)nb * 64u, kdesc(St, kc, 128), ndesc(Qr, nb, kc, g.NKp), idesc2,
+                        mma_f16(tmem_base + col_dk + (uint32_t)nb * 64u, kdesc(St, kc, 128), ndesc(Qr, nb, kc, g.NKp), idesc2,
                                  (i > 0 || kc > 0) ? 1u : 0u);
                 mma_commit(bar_free);
             }
@@ -596,8 +599,8 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_bwd_dkv_tc_kernel(const _
                     e[k] = pij;
                     f[k] = ok ? pij * (__uint_as_float(rp[k]) - Ds[c0 + k]) : 0.f;
                 }
-                store_chunk_sw32(prow + (uint32_t)(c0 >> 4) * 4096u, sw, e);
-                store_chunk_sw32(srow + (uint32_t)(c0 >> 4) * 4096u, sw, f);
+                store_chunk_sw32<T>(prow + (uint32_t)(c0 >> 4) * 4096u, sw, e);
+                store_chunk_sw32<T>(srow + (uint32_t)(c0 >> 4) * 4096u, sw, f);
             }
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             fence_before();
@@ -605,14 +608,14 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) attn_bwd_dkv_tc_kernel(const _
         }
         mb_wait(bar_o, 0);
         fence_after();
-        bf16* krow = p.dqkv.at<bf16>(b, y, x, p.inner + h * p.d);
-        bf16* vrow = p.dqkv.at<bf16>(b, y, x, 2 * p.inner + h * p.d);
+        T* krow = p.dqkv.at<T>(b, y, x, p.inner + h * p.d);
+        T* vrow = p.dqkv.at<T>(b, y, x, 2 * p.inner + h * p.d);
         for (int c0 = 0; c0 < p.d; c0 += 16) {
             uint32_t rv[16], rk[16];
             tm_ld16(lane_addr + p.col_acc + (uint32_t)c0, rv);
             tm_ld16(lane_addr + p.col_acc + (uint32_t)p.nvb * 64u + (uint32_t)c0, rk);
             tm_ld_wait();
-            if (valid) { store_row16(vrow + c0, rv, 1.0f); store_row16(krow + c0, rk, p.scale); }
+            if (valid) { store_row16<T>(vrow + c0, rv, 1.0f); store_row16<T>(krow + c0, rk, p.scale); }
         }
         fence_before();
     }
@@ -642,10 +645,10 @@ static int atc_smem_attr(const void* kernel, size_t smem) {
     return (int)cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
 }
 
-// bf16; head_dim 32 / 64 / 128 (V, dO, Q are read as 64-channel boxes: with head_dim 32 the upper 32 output columns are
+// bf16 / fp16; head_dim 32 / 64 / 128 (V, dO, Q are read as 64-channel boxes: with head_dim 32 the upper 32 output columns are
 // the next head's and are ignored); W <= 128 so that a tile holds at least one whole image row.
 int attn_tc_supported(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads, int d, int dtype) {
-    if (dtype != DDPM_BF16 || (d != 32 && d != 64 && d != 128)) return 0;
+    if ((dtype != DDPM_BF16 && dtype != DDPM_F16) || (d != 32 && d != 64 && d != 128)) return 0;
     if (qkv->W > 128) return 0;
     if (qkv->halo != 1 && qkv->halo != 0) return 0;
     if (qkv->pitch % 8 || out->pitch % 8 || ((uintptr_t)qkv->ptr & 15) || ((uintptr_t)out->ptr & 15)) return 0;
@@ -653,18 +656,19 @@ int attn_tc_supported(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads,
     return 1;
 }
 
-// 4-D tensor map over (channel, x, y, image) of one NHWC bf16 tensor, halo excluded: boxes of `channels` x W x `rows`,
+// 4-D tensor map over (channel, x, y, image) of one NHWC 16-bit tensor, halo excluded: boxes of `channels` x W x `rows`,
 // 16 channels SWIZZLE_32B (K-major operands), 64 channels SWIZZLE_128B (MN-major operands)
+template <typename T>
 static int atc_map(const ddpm_tensor* t, int channels, int rows, CUtensorMap* m) {
     const int Hp = t->H + 2 * t->halo, Wp = t->W + 2 * t->halo;
     char* base = (char*)t->ptr + ((size_t)t->halo * Wp + t->halo) * t->pitch * 2;
     const uint64_t dims[4] = {(uint64_t)t->C, (uint64_t)t->W, (uint64_t)t->H, (uint64_t)t->N};
     const uint64_t strides[3] = {(uint64_t)t->pitch * 2, (uint64_t)Wp * t->pitch * 2, (uint64_t)Hp * Wp * t->pitch * 2};
     const uint32_t box[4] = {(uint32_t)channels, (uint32_t)t->W, (uint32_t)rows, 1u};
-    return ddpm_encode_tiled_bf16(m, base, 4, dims, strides, box, channels == 16 ? 32 : 128);
+    return ddpm_encode_tiled16(m, Fmt16<T>::tma_type, base, 4, dims, strides, box, channels == 16 ? 32 : 128);
 }
 
-template <int D>
+template <typename T, int D>
 static int attn_fwd_tc_launch(const ddpm_tensor* qkv, AtcP& p, cudaStream_t st) {
     const AtGeo& g = p.g;
     constexpr int KCH = D / 16, NVB = (D + 63) / 64;
@@ -679,25 +683,32 @@ static int attn_fwd_tc_launch(const ddpm_tensor* qkv, AtcP& p, cudaStream_t st) 
     p.zero_v = g.NK != g.NKp;
     const size_t smem = (size_t)p.bar_off + 8 * 11 + 16 + 1024;
     CUtensorMap tmQ, tmK, tmV;
-    int rc = atc_map(qkv, 16, g.R, &tmQ); if (rc) return rc;
-    rc = atc_map(qkv, 16, g.KR, &tmK); if (rc) return rc;
-    rc = atc_map(qkv, 64, g.KR, &tmV); if (rc) return rc;
+    int rc = atc_map<T>(qkv, 16, g.R, &tmQ); if (rc) return rc;
+    rc = atc_map<T>(qkv, 16, g.KR, &tmK); if (rc) return rc;
+    rc = atc_map<T>(qkv, 64, g.KR, &tmV); if (rc) return rc;
     static size_t configured = 0;
-    if (smem > configured) { rc = atc_smem_attr((const void*)attn_fwd_tc_kernel<D>, smem); if (rc) return rc; configured = smem; }
+    if (smem > configured) { rc = atc_smem_attr((const void*)attn_fwd_tc_kernel<T, D>, smem); if (rc) return rc; configured = smem; }
     dim3 grid((qkv->H + g.R - 1) / g.R, p.heads, qkv->N);
-    CUDA_TRY(launch_kernel(attn_fwd_tc_kernel<D>, grid, dim3(ATC_THREADS), smem, st, tmQ, tmK, tmV, p));
+    CUDA_TRY(launch_kernel(attn_fwd_tc_kernel<T, D>, grid, dim3(ATC_THREADS), smem, st, tmQ, tmK, tmV, p));
     LAUNCH_OK();
     return 0;
 }
 
-int attn_tc_launch(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads, int d, float* lse, cudaStream_t st) {
+template <typename T>
+static int attn_tc_launch_t(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads, int d, float* lse, cudaStream_t st) {
     AtcP p;
     p.out = TV(*out); p.lse = lse; p.heads = heads; p.inner = heads * d;
     p.g = atc_geo(qkv, d);
     p.scale = 1.0f / sqrtf((float)d); p.scale_log2e = p.scale * 1.4426950408889634f;
-    if (d == 32) return attn_fwd_tc_launch<32>(qkv, p, st);
-    if (d == 64) return attn_fwd_tc_launch<64>(qkv, p, st);
-    return attn_fwd_tc_launch<128>(qkv, p, st);
+    if (d == 32) return attn_fwd_tc_launch<T, 32>(qkv, p, st);
+    if (d == 64) return attn_fwd_tc_launch<T, 64>(qkv, p, st);
+    return attn_fwd_tc_launch<T, 128>(qkv, p, st);
+}
+
+int attn_tc_launch(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads, int d, float* lse, int dtype, cudaStream_t st) {
+    if (dtype == DDPM_BF16) return attn_tc_launch_t<bf16>(qkv, out, heads, d, lse, st);
+    if (dtype == DDPM_F16) return attn_tc_launch_t<f16>(qkv, out, heads, d, lse, st);
+    return DDPM_E_ARG;
 }
 
 // floats of scratch the tensor-core backward needs (D = dO . O per query) -- 0 when the shape is not eligible
@@ -706,8 +717,9 @@ int64_t attn_tc_bwd_scratch_floats(const ddpm_tensor* qkv, const ddpm_tensor* ou
     return (int64_t)qkv->N * heads * qkv->H * qkv->W;
 }
 
-int attn_tc_bwd_launch(const ddpm_tensor* qkv, const ddpm_tensor* out, const ddpm_tensor* dout, const float* lse,
-                       const ddpm_tensor* dqkv, int heads, int d, float* scratch, cudaStream_t st) {
+template <typename T>
+static int attn_tc_bwd_launch_t(const ddpm_tensor* qkv, const ddpm_tensor* out, const ddpm_tensor* dout, const float* lse,
+                                const ddpm_tensor* dqkv, int heads, int d, float* scratch, cudaStream_t st) {
     AtbP p;
     p.out = TV(*out); p.dout = TV(*dout); p.dqkv = TV(*dqkv); p.lse = lse; p.Dbuf = scratch;
     p.heads = heads; p.d = d; p.inner = heads * d; p.kch = d / 16; p.nvb = (d + 63) / 64;
@@ -720,9 +732,9 @@ int attn_tc_bwd_launch(const ddpm_tensor* qkv, const ddpm_tensor* out, const ddp
     const bool ragged = g.NK != g.NKp;
     const int A1 = p.kch * 4096, K32 = p.kch * g.NKp * 32, M128 = p.nvb * g.NKp * 128, CH = (g.NKp / 16) * 4096;
     CUtensorMap qT, qF32, qF128, gT, gF32, gF128;
-    int rc = atc_map(qkv, 16, g.R, &qT); if (rc) return rc;
-    if ((rc = atc_map(qkv, 16, g.KR, &qF32)) || (rc = atc_map(qkv, 64, g.KR, &qF128))) return rc;
-    if ((rc = atc_map(dout, 16, g.R, &gT)) || (rc = atc_map(dout, 16, g.KR, &gF32)) || (rc = atc_map(dout, 64, g.KR, &gF128))) return rc;
+    int rc = atc_map<T>(qkv, 16, g.R, &qT); if (rc) return rc;
+    if ((rc = atc_map<T>(qkv, 16, g.KR, &qF32)) || (rc = atc_map<T>(qkv, 64, g.KR, &qF128))) return rc;
+    if ((rc = atc_map<T>(dout, 16, g.R, &gT)) || (rc = atc_map<T>(dout, 16, g.KR, &gF32)) || (rc = atc_map<T>(dout, 64, g.KR, &gF128))) return rc;
     dim3 grid((qkv->H + g.R - 1) / g.R, heads, qkv->N);
     {   // dq: Q, dO, stages of {K32, V32, K128}, dS
         p.sst = (2 * K32 + M128 + 1023) & ~1023;
@@ -733,8 +745,8 @@ int attn_tc_bwd_launch(const ddpm_tensor* qkv, const ddpm_tensor* out, const ddp
         p.zero_off = p.o2; p.zero_bytes = ragged ? p.nst * p.sst : 0;
         const size_t smem = (size_t)p.bar_off + 8 * 10 + 16 + 1024;
         static size_t configured = 0;
-        if (smem > configured) { rc = atc_smem_attr((const void*)attn_bwd_dq_tc_kernel, smem); if (rc) return rc; configured = smem; }
-        CUDA_TRY(launch_kernel(attn_bwd_dq_tc_kernel, grid, dim3(ATC_THREADS), smem, st, qT, gT, qF32, qF128, p));
+        if (smem > configured) { rc = atc_smem_attr((const void*)attn_bwd_dq_tc_kernel<T>, smem); if (rc) return rc; configured = smem; }
+        CUDA_TRY(launch_kernel(attn_bwd_dq_tc_kernel<T>, grid, dim3(ATC_THREADS), smem, st, qT, gT, qF32, qF128, p));
         LAUNCH_OK();
     }
     {   // dkv: K tile, V tile, Q32 -> Q128, dO32 -> dO128, P^T, dS^T, lse / D of the query tile
@@ -745,9 +757,16 @@ int attn_tc_bwd_launch(const ddpm_tensor* qkv, const ddpm_tensor* out, const ddp
         p.zero_off = p.o2; p.zero_bytes = ragged ? 2 * RB : 0;
         const size_t smem = (size_t)p.bar_off + 8 * 7 + 16 + 1024;
         static size_t configured = 0;
-        if (smem > configured) { rc = atc_smem_attr((const void*)attn_bwd_dkv_tc_kernel, smem); if (rc) return rc; configured = smem; }
-        CUDA_TRY(launch_kernel(attn_bwd_dkv_tc_kernel, grid, dim3(ATC_THREADS), smem, st, qT, qF32, gF32, qF128, gF128, p));
+        if (smem > configured) { rc = atc_smem_attr((const void*)attn_bwd_dkv_tc_kernel<T>, smem); if (rc) return rc; configured = smem; }
+        CUDA_TRY(launch_kernel(attn_bwd_dkv_tc_kernel<T>, grid, dim3(ATC_THREADS), smem, st, qT, qF32, gF32, qF128, gF128, p));
         LAUNCH_OK();
     }
     return 0;
+}
+
+int attn_tc_bwd_launch(const ddpm_tensor* qkv, const ddpm_tensor* out, const ddpm_tensor* dout, const float* lse,
+                       const ddpm_tensor* dqkv, int heads, int d, float* scratch, int dtype, cudaStream_t st) {
+    if (dtype == DDPM_BF16) return attn_tc_bwd_launch_t<bf16>(qkv, out, dout, lse, dqkv, heads, d, scratch, st);
+    if (dtype == DDPM_F16) return attn_tc_bwd_launch_t<f16>(qkv, out, dout, lse, dqkv, heads, d, scratch, st);
+    return DDPM_E_ARG;
 }

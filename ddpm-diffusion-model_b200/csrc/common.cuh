@@ -1,11 +1,55 @@
 // Shared device/host helpers for libddpm_b200 (sm_100a only).
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
+#include <type_traits>
 #include "../../include/ddpm_b200.h"
 
 typedef __nv_bfloat16 bf16;
+typedef __half f16;
+
+// The two 16-bit activation formats (DDPM_BF16, DDPM_F16): everything a kernel needs to know about one.  Kernels take the
+// element type as a template parameter and read the format from here.  fp32 -> 16-bit conversions round to nearest; for
+// fp16 that gives +-inf beyond 65504 (IEEE, no saturation), which is what a GradScaler relies on to detect overflow.
+template <typename T> struct Fmt16;
+template <> struct Fmt16<bf16> {
+    typedef __nv_bfloat162 T2;
+    static constexpr CUtensorMapDataType tma_type = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    static constexpr uint32_t idesc_ab = (1u << 7) | (1u << 10);   // tcgen05.mma kind::f16: A and B format BF16 (bits 7-9, 10-12)
+    static constexpr uint16_t one = 0x3F80;                         // 1.0
+    __device__ __forceinline__ static float to_f(bf16 h) { return __bfloat162float(h); }
+    __device__ __forceinline__ static bf16 from_f(float v) { return __float2bfloat16_rn(v); }
+    __device__ __forceinline__ static float2 to_f2(T2 h) { return __bfloat1622float2(h); }
+    __device__ __forceinline__ static T2 from_f2(float a, float b) { return __floats2bfloat162_rn(a, b); }
+    // the two elements of a 32-bit word in one integer instruction each (a bf16 is the upper half of an fp32)
+    __device__ __forceinline__ static void unpack(uint32_t w, float& lo, float& hi) {
+        lo = __uint_as_float(w << 16); hi = __uint_as_float(w & 0xffff0000u);
+    }
+};
+template <> struct Fmt16<f16> {
+    typedef __half2 T2;
+    static constexpr CUtensorMapDataType tma_type = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+    static constexpr uint32_t idesc_ab = 0u;                        // A and B format F16
+    static constexpr uint16_t one = 0x3C00;
+    __device__ __forceinline__ static float to_f(f16 h) { return __half2float(h); }
+    __device__ __forceinline__ static f16 from_f(float v) { return __float2half_rn(v); }
+    __device__ __forceinline__ static float2 to_f2(T2 h) { return __half22float2(h); }
+    __device__ __forceinline__ static T2 from_f2(float a, float b) { return __floats2half2_rn(a, b); }
+    __device__ __forceinline__ static void unpack(uint32_t w, float& lo, float& hi) {
+        const float2 f = __half22float2(*reinterpret_cast<const T2*>(&w));
+        lo = f.x; hi = f.y;
+    }
+};
+// 2-wide access through a 32-bit word (the element pair of a uint2 / uint4 lane)
+template <typename T> __device__ __forceinline__ float2 unpack2(const uint32_t& w) {
+    return Fmt16<T>::to_f2(*reinterpret_cast<const typename Fmt16<T>::T2*>(&w));
+}
+template <typename T> __device__ __forceinline__ void pack2(uint32_t& w, float a, float b) {
+    *reinterpret_cast<typename Fmt16<T>::T2*>(&w) = Fmt16<T>::from_f2(a, b);
+}
 
 extern int64_t g_ddpm_launches;  // counted by LAUNCH_OK (host side, single-threaded use)
 
@@ -37,14 +81,37 @@ template <> struct Cvt<float> {
     __device__ __forceinline__ static void st(float* p, float v) { *p = v; }
 };
 template <> struct Cvt<bf16> {
-    __device__ __forceinline__ static float ld(const bf16* p) { return __bfloat162float(*p); }
-    __device__ __forceinline__ static void st(bf16* p, float v) { *p = __float2bfloat16_rn(v); }
+    __device__ __forceinline__ static float ld(const bf16* p) { return Fmt16<bf16>::to_f(*p); }
+    __device__ __forceinline__ static void st(bf16* p, float v) { *p = Fmt16<bf16>::from_f(v); }
+};
+template <> struct Cvt<f16> {
+    __device__ __forceinline__ static float ld(const f16* p) { return Fmt16<f16>::to_f(*p); }
+    __device__ __forceinline__ static void st(f16* p, float v) { *p = Fmt16<f16>::from_f(v); }
 };
 template <typename T> __device__ __forceinline__ float ldf(const T* p) { return Cvt<T>::ld(p); }
 template <typename T> __device__ __forceinline__ void stf(T* p, float v) { Cvt<T>::st(p, v); }
 
-// 8-element (bf16) / 4-element (fp32) 16-byte vectors of activations
-template <typename T> struct Vec16;
+// 8-element (bf16 / fp16) / 4-element (fp32) 16-byte vectors of activations
+template <typename T> struct Vec16 {
+    static constexpr int N = 8;
+    float v[8];
+    __device__ __forceinline__ void load(const T* p) {
+        uint4 t = *reinterpret_cast<const uint4*>(p);
+        const typename Fmt16<T>::T2* h = reinterpret_cast<const typename Fmt16<T>::T2*>(&t);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            float2 f = Fmt16<T>::to_f2(h[i]);
+            v[2 * i] = f.x; v[2 * i + 1] = f.y;
+        }
+    }
+    __device__ __forceinline__ void store(T* p) const {
+        uint4 t;
+        typename Fmt16<T>::T2* h = reinterpret_cast<typename Fmt16<T>::T2*>(&t);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) h[i] = Fmt16<T>::from_f2(v[2 * i], v[2 * i + 1]);
+        *reinterpret_cast<uint4*>(p) = t;
+    }
+};
 template <> struct Vec16<float> {
     static constexpr int N = 4;
     float v[4];
@@ -54,26 +121,6 @@ template <> struct Vec16<float> {
     }
     __device__ __forceinline__ void store(float* p) const {
         *reinterpret_cast<float4*>(p) = make_float4(v[0], v[1], v[2], v[3]);
-    }
-};
-template <> struct Vec16<bf16> {
-    static constexpr int N = 8;
-    float v[8];
-    __device__ __forceinline__ void load(const bf16* p) {
-        uint4 t = *reinterpret_cast<const uint4*>(p);
-        const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&t);
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            float2 f = __bfloat1622float2(h[i]);
-            v[2 * i] = f.x; v[2 * i + 1] = f.y;
-        }
-    }
-    __device__ __forceinline__ void store(bf16* p) const {
-        uint4 t;
-        __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(&t);
-#pragma unroll
-        for (int i = 0; i < 4; ++i) h[i] = __floats2bfloat162_rn(v[2 * i], v[2 * i + 1]);
-        *reinterpret_cast<uint4*>(p) = t;
     }
 };
 
@@ -92,7 +139,9 @@ __device__ __forceinline__ float dsilu_f(float z) {
 // bf16 activation paths: SiLU through ONE MUFU (tanh.approx, relative error 2^-11) instead of ex2 + rcp:
 //   with h = z/2:  silu(z) = h + h*tanh(h);   silu'(z) = s + s*h*(1 - tanh(h)),  s = 0.5 + 0.5*tanh(h)
 // 3 (forward) / 6 (derivative) instructions including the affine that produces h, against 6 / 9.  Absolute error
-// <= |z| * 2.5e-4 -- below the bf16 resolution of the tensors these kernels write; the fp32 kernels keep silu_f.
+// <= |z| * 2.5e-4 -- below the bf16 resolution of the tensors these kernels write; the fp32 kernels keep silu_f, and so do
+// the fp16 ones: fp16 has 3 more significant bits, and where SiLU cancels (silu(-3) = -0.14, silu(-6) = -0.015) that bound
+// is ~5 and ~200 fp16 ulps of the result.
 __device__ __forceinline__ float tanh_approx(float x) { float y; asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float silu_half(float h) { return fmaf(h, tanh_approx(h), h); }
 __device__ __forceinline__ float dsilu_half(float h) {

@@ -71,13 +71,13 @@ __global__ void __launch_bounds__(CT) conv_simt_kernel(ConvP p) {
                     }
                     if (ok) {
                         const T* src = p.in.at<T>(an, iy, ix, ci);
-                        if (sizeof(T) == 4) {
+                        if constexpr (sizeof(T) == 4) {
                             float4 t = *reinterpret_cast<const float4*>(src);
                             av[0] = t.x; av[1] = t.y; av[2] = t.z; av[3] = t.w;
                         } else {
                             uint2 t = *reinterpret_cast<const uint2*>(src);
-                            float2 a = __bfloat1622float2(*reinterpret_cast<__nv_bfloat162*>(&t.x));
-                            float2 b = __bfloat1622float2(*reinterpret_cast<__nv_bfloat162*>(&t.y));
+                            float2 a = unpack2<T>(t.x);
+                            float2 b = unpack2<T>(t.y);
                             av[0] = a.x; av[1] = a.y; av[2] = b.x; av[3] = b.y;
                         }
                     }
@@ -114,13 +114,13 @@ __global__ void __launch_bounds__(CT) conv_simt_kernel(ConvP p) {
             const int k = k0 + akq;
             if (bcol_ok && k < p.Kt) {
                 if (p.vecB) {
-                    if (sizeof(T) == 4) {
+                    if constexpr (sizeof(T) == 4) {
                         float4 t = *reinterpret_cast<const float4*>(wrow + k);
                         bv[0] = t.x; bv[1] = t.y; bv[2] = t.z; bv[3] = t.w;
                     } else {
                         uint2 t = *reinterpret_cast<const uint2*>(wrow + k);
-                        float2 a = __bfloat1622float2(*reinterpret_cast<__nv_bfloat162*>(&t.x));
-                        float2 b = __bfloat1622float2(*reinterpret_cast<__nv_bfloat162*>(&t.y));
+                        float2 a = unpack2<T>(t.x);
+                        float2 b = unpack2<T>(t.y);
                         bv[0] = a.x; bv[1] = a.y; bv[2] = b.x; bv[3] = b.y;
                     }
                 } else {
@@ -170,11 +170,11 @@ __global__ void __launch_bounds__(CT) conv_simt_kernel(ConvP p) {
         }
         T* dst = p.out.at<T>(n, oy, ox, co0);
         if (p.vecO && co0 + 3 < p.Cout) {
-            if (sizeof(T) == 4) *reinterpret_cast<float4*>(dst) = make_float4(v[0], v[1], v[2], v[3]);
+            if constexpr (sizeof(T) == 4) *reinterpret_cast<float4*>(dst) = make_float4(v[0], v[1], v[2], v[3]);
             else {
                 uint2 t;
-                *reinterpret_cast<__nv_bfloat162*>(&t.x) = __floats2bfloat162_rn(v[0], v[1]);
-                *reinterpret_cast<__nv_bfloat162*>(&t.y) = __floats2bfloat162_rn(v[2], v[3]);
+                pack2<T>(t.x, v[0], v[1]);
+                pack2<T>(t.y, v[2], v[3]);
                 *reinterpret_cast<uint2*>(dst) = t;
             }
         } else {
@@ -414,7 +414,9 @@ int conv_simt_launch(const ddpm_conv_args* a, cudaStream_t st) {
     p.vecO = (a->out.pitch % 4 == 0) && al(a->out.ptr, 4 * es);
     dim3 grid(ceil_div(p.M, BM), ceil_div(p.Cout, BN));
     if (a->dtype == DDPM_F32) CUDA_TRY(launch_kernel(conv_simt_kernel<float>, grid, dim3(CT), 0, st, p));
-    else CUDA_TRY(launch_kernel(conv_simt_kernel<bf16>, grid, dim3(CT), 0, st, p));
+    else if (a->dtype == DDPM_BF16) CUDA_TRY(launch_kernel(conv_simt_kernel<bf16>, grid, dim3(CT), 0, st, p));
+    else if (a->dtype == DDPM_F16) CUDA_TRY(launch_kernel(conv_simt_kernel<f16>, grid, dim3(CT), 0, st, p));
+    else return DDPM_E_ARG;
     LAUNCH_OK();
     return 0;
 }
@@ -460,11 +462,11 @@ __global__ void __launch_bounds__(CT) wgrad_simt_kernel(WgP p) {
             if (co0 + l4 < p.Cout) {
                 const T* src = p.dy.at<T>(n, oy, ox, co0 + l4);
                 if (p.vecY && co0 + l4 + 3 < p.Cout) {
-                    if (sizeof(T) == 4) { float4 t = *reinterpret_cast<const float4*>(src); yv[0] = t.x; yv[1] = t.y; yv[2] = t.z; yv[3] = t.w; }
+                    if constexpr (sizeof(T) == 4) { float4 t = *reinterpret_cast<const float4*>(src); yv[0] = t.x; yv[1] = t.y; yv[2] = t.z; yv[3] = t.w; }
                     else {
                         uint2 t = *reinterpret_cast<const uint2*>(src);
-                        float2 a = __bfloat1622float2(*reinterpret_cast<__nv_bfloat162*>(&t.x));
-                        float2 b = __bfloat1622float2(*reinterpret_cast<__nv_bfloat162*>(&t.y));
+                        float2 a = unpack2<T>(t.x);
+                        float2 b = unpack2<T>(t.y);
                         yv[0] = a.x; yv[1] = a.y; yv[2] = b.x; yv[3] = b.y;
                     }
                 } else {
@@ -478,11 +480,11 @@ __global__ void __launch_bounds__(CT) wgrad_simt_kernel(WgP p) {
                 int iy = oy * p.stride + ky - p.pad, ix = ox * p.stride + kx - p.pad;
                 if (iy >= 0 && iy < p.act.H && ix >= 0 && ix < p.act.W) {
                     const T* src = p.act.at<T>(n, iy, ix, ci[0]);
-                    if (sizeof(T) == 4) { float4 t = *reinterpret_cast<const float4*>(src); xv[0] = t.x; xv[1] = t.y; xv[2] = t.z; xv[3] = t.w; }
+                    if constexpr (sizeof(T) == 4) { float4 t = *reinterpret_cast<const float4*>(src); xv[0] = t.x; xv[1] = t.y; xv[2] = t.z; xv[3] = t.w; }
                     else {
                         uint2 t = *reinterpret_cast<const uint2*>(src);
-                        float2 a = __bfloat1622float2(*reinterpret_cast<__nv_bfloat162*>(&t.x));
-                        float2 b = __bfloat1622float2(*reinterpret_cast<__nv_bfloat162*>(&t.y));
+                        float2 a = unpack2<T>(t.x);
+                        float2 b = unpack2<T>(t.y);
                         xv[0] = a.x; xv[1] = a.y; xv[2] = b.x; xv[3] = b.y;
                     }
                 }
@@ -550,7 +552,9 @@ int wgrad_simt_launch(const ddpm_wgrad_args* a, cudaStream_t st) {
     splits = ceil_div(p.Q, p.qper);
     dim3 grid(ceil_div(p.Cout, BM), ceil_div(p.Kf, BN), splits);
     if (a->dtype == DDPM_F32) CUDA_TRY(launch_kernel(wgrad_simt_kernel<float>, grid, dim3(CT), 0, st, p));
-    else CUDA_TRY(launch_kernel(wgrad_simt_kernel<bf16>, grid, dim3(CT), 0, st, p));
+    else if (a->dtype == DDPM_BF16) CUDA_TRY(launch_kernel(wgrad_simt_kernel<bf16>, grid, dim3(CT), 0, st, p));
+    else if (a->dtype == DDPM_F16) CUDA_TRY(launch_kernel(wgrad_simt_kernel<f16>, grid, dim3(CT), 0, st, p));
+    else return DDPM_E_ARG;
     LAUNCH_OK();
     return 0;
 }

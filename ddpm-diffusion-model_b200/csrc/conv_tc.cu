@@ -1,4 +1,6 @@
-// tcgen05 / TMEM implicit-GEMM convolution for sm_100a (bf16 in, fp32 accumulate in tensor memory).
+// tcgen05 / TMEM implicit-GEMM convolution for sm_100a (bf16 or fp16 in, fp32 accumulate in tensor memory).  The element
+// type is a template parameter of every kernel here; its format (TMA type, instruction-descriptor bits, packing, 1.0) comes
+// from Fmt16 (common.cuh).
 //
 // "Shift-GEMM" over the padded NHWC layout.  Activations carry a zero halo, so with
 // Q = (n*Hp + yp)*Wp + xp the padded-linear pixel index, a 3x3/s1/p1 convolution is
@@ -14,11 +16,10 @@
 // for fprop and, with flipped/transposed weights, dgrad.
 #include "common.cuh"
 #include <cuda.h>
-#include <type_traits>
 #include <cudaTypedefs.h>
 
 #define TC_THREADS 192
-#define KC 16                 // channels per K-chunk (one UMMA K step for bf16)
+#define KC 16                 // channels per K-chunk (one UMMA K step for 16-bit operands)
 
 static int sm_count();
 // path-forcing flags of ddpm_set_tc_mode (mode >> 4, see ddpm_b200.h), read by the launch planners below
@@ -69,7 +70,7 @@ __device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t ncols) {
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
+__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
         "setp.ne.b32 p, %4, 0;\n\t"
@@ -120,24 +121,24 @@ static int get_encode() {
     return 0;
 }
 
-static int encode(CUtensorMap* m, void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
+static int encode(CUtensorMap* m, CUtensorMapDataType type, void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
                   const uint32_t* box, CUtensorMapSwizzle sw) {
     cuuint64_t gd[5]; cuuint64_t gs[4]; cuuint32_t bx[5]; cuuint32_t es[5];
     for (int i = 0; i < rank; ++i) { gd[i] = dims[i]; bx[i] = box[i]; es[i] = 1; }
     for (int i = 0; i < rank - 1; ++i) gs[i] = strides_bytes[i];
-    CUresult r = g_encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, base, gd, gs, bx, es,
+    CUresult r = g_encode(m, type, (cuuint32_t)rank, base, gd, gs, bx, es,
                           CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     return r == CUDA_SUCCESS ? 0 : 1;   // cudaErrorInvalidValue
 }
 
-// shared with attn_tc.cu: bf16 tiled tensor map, swizzle_bytes in {0, 32, 64, 128}
-int ddpm_encode_tiled_bf16(CUtensorMap* m, void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-                           const uint32_t* box, int swizzle_bytes) {
+// shared with attn_tc.cu: tiled tensor map of 16-bit elements, swizzle_bytes in {0, 32, 64, 128}
+int ddpm_encode_tiled16(CUtensorMap* m, CUtensorMapDataType type, void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
+                        const uint32_t* box, int swizzle_bytes) {
     int rc = get_encode(); if (rc) return rc;
     const CUtensorMapSwizzle sw = swizzle_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : swizzle_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B
                                 : swizzle_bytes == 32 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_NONE;
-    return encode(m, base, rank, dims, strides_bytes, box, sw);
+    return encode(m, type, base, rank, dims, strides_bytes, box, sw);
 }
 
 static int pick_nt(int Cout) {
@@ -148,7 +149,7 @@ static int pick_nt(int Cout) {
 
 int conv_tc_supported(const ddpm_conv_args* a) {
     const bool up = a->mode == DDPM_CONV_UP2X_PHASE;
-    if (a->dtype != DDPM_BF16 || (a->mode != DDPM_CONV_NORMAL && !up) || a->a_silu || a->z.ptr) return 0;
+    if ((a->dtype != DDPM_BF16 && a->dtype != DDPM_F16) || (a->mode != DDPM_CONV_NORMAL && !up) || a->a_silu || a->z.ptr) return 0;
     if (up) { if (a->KH != 2 || a->KW != 2 || a->stride != 1 || a->res.ptr || a->in2.ptr || (a->epi & DDPM_EPI_ACCUM)) return 0; }
     else if (!((a->KH == 3 && a->KW == 3 && a->pad == 1) || (a->KH == 1 && a->KW == 1 && a->pad == 0))) return 0;
     const ddpm_tensor &in = a->in, &out = a->out;
@@ -223,7 +224,7 @@ __device__ __forceinline__ void tmem_alloc2(uint32_t* dst_smem, uint32_t ncols) 
 __device__ __forceinline__ void tmem_dealloc2(uint32_t taddr, uint32_t ncols) {
     asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
-__device__ __forceinline__ void umma2_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
+__device__ __forceinline__ void umma2_f16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
         "setp.ne.b32 p, %4, 0;\n\t"
@@ -274,11 +275,10 @@ struct Tc2Params {
 // FUSED2: the 1x1 second operand (ddpm_conv_args.in2).  A template parameter, not a run-time branch: the extra stage kind
 // in the producer and MMA-issue loops cost 3-4 % on EVERY convolution when it was one (A/B of three builds on one box,
 // 96->96@64: 67.9 -> 70.0 us) -- the issue loop is that tight.
-template <int MT, int TAPS, bool FUSED2>
-__global__ void __launch_bounds__(TC2_THREADS, 1) conv_tc2_kernel(const __grid_constant__ CUtensorMap tmA,
-                                                                  const __grid_constant__ CUtensorMap tmB,
-                                                                  const __grid_constant__ CUtensorMap tmA2,
-                                                                  const __grid_constant__ CUtensorMap tmB2, Tc2Params p) {
+// The element type T is a parameter of the body; the kernels below are its two entry points (bf16 keeps its name).
+template <typename T, int MT, int TAPS, bool FUSED2>
+__device__ __forceinline__ void conv_tc2(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmA2,
+                                         const CUtensorMap& tmB2, Tc2Params p) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
     uint8_t* ring = smem;
@@ -365,7 +365,7 @@ __global__ void __launch_bounds__(TC2_THREADS, 1) conv_tc2_kernel(const __grid_c
         // one elected lane issues the tcgen05 instructions
         if (leader) {
             const bool el = elect_one();
-            const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(p.NT >> 3) << 17) | ((256u >> 4) << 24);
+            const uint32_t idesc = (1u << 4) | Fmt16<T>::idesc_ab | ((uint32_t)(p.NT >> 3) << 17) | ((256u >> 4) << 24);
             const uint32_t hi = desc_hi(256u, 6u);                       // SBO 256 B, SWIZZLE_32B
             uint32_t tapoff[TAPS];                                       // A row shift of each tap, in 16-byte units
 #pragma unroll
@@ -396,7 +396,7 @@ __global__ void __launch_bounds__(TC2_THREADS, 1) conv_tc2_kernel(const __grid_c
 #pragma unroll
                         for (int mt = 0; mt < MT; ++mt) {
                             const uint64_t adesc = desc_pack(a_lo + tapoff[TAPS / 2] + (uint32_t)(mt * 256), hi);
-                            if (el) umma2_bf16(dbase + (uint32_t)(mt * p.NT), adesc, bdesc, idesc, 1u);
+                            if (el) umma2_f16(dbase + (uint32_t)(mt * p.NT), adesc, bdesc, idesc, 1u);
                         }
                         if (el) umma2_commit_mc(&empty[s]);
                         __syncwarp();
@@ -411,7 +411,7 @@ __global__ void __launch_bounds__(TC2_THREADS, 1) conv_tc2_kernel(const __grid_c
 #pragma unroll
                             for (int mt = 0; mt < MT; ++mt) {
                                 const uint64_t adesc = desc_pack(a_lo + tapoff[tap] + (uint32_t)(mt * 256), hi);
-                                if (el) umma2_bf16(dbase + (uint32_t)(mt * p.NT), adesc, bdesc, idesc, tap == 0 ? acc : 1u);
+                                if (el) umma2_f16(dbase + (uint32_t)(mt * p.NT), adesc, bdesc, idesc, tap == 0 ? acc : 1u);
                             }
                         }
                         acc = 1;
@@ -441,7 +441,7 @@ __global__ void __launch_bounds__(TC2_THREADS, 1) conv_tc2_kernel(const __grid_c
             // Row addressing for this item is done BEFORE waiting for the accumulators, and the residual / accumulate
             // rows are prefetched into L2 while the MMAs are still running: the epilogue was latency-bound on
             // those reads (96->96@64: 75 us plain vs 140 us with a residual).
-            bf16* orow_a[MT]; const bf16* rrow_a[MT]; const float* tb_a[MT];
+            T* orow_a[MT]; const T* rrow_a[MT]; const float* tb_a[MT];
 #pragma unroll
             for (int mt = 0; mt < MT; ++mt) {
                 const int Q = Q0 + mt * 128 + qd * 32 + lane;
@@ -454,10 +454,10 @@ __global__ void __launch_bounds__(TC2_THREADS, 1) conv_tc2_kernel(const __grid_c
                     if (p.sub) { valid = valid && ((y | x) & 1) == 0; y >>= 1; x >>= 1; }
                     if (p.up) { y = 2 * y + p.py; x = 2 * x + p.px; }
                 }
-                orow_a[mt] = valid ? p.out.at<bf16>(n, y, x, n0) : nullptr;
-                rrow_a[mt] = (valid && p.has_res) ? p.res.at<bf16>(n, y, x, n0) : nullptr;
+                orow_a[mt] = valid ? p.out.at<T>(n, y, x, n0) : nullptr;
+                rrow_a[mt] = (valid && p.has_res) ? p.res.at<T>(n, y, x, n0) : nullptr;
                 tb_a[mt] = (valid && p.tbias) ? p.tbias + (size_t)n * p.tbias_pitch + n0 : nullptr;
-                const bf16* pf = rrow_a[mt] ? rrow_a[mt] : ((p.accum && valid) ? orow_a[mt] : nullptr);
+                const T* pf = rrow_a[mt] ? rrow_a[mt] : ((p.accum && valid) ? orow_a[mt] : nullptr);
                 if (pf) {
                     for (int c = blk_lo << 4; c < (blk_hi << 4); c += 64)
                         asm volatile("prefetch.global.L2 [%0];" ::"l"(pf + c));
@@ -468,7 +468,7 @@ __global__ void __launch_bounds__(TC2_THREADS, 1) conv_tc2_kernel(const __grid_c
             const uint32_t dbase = tmem_base + buf * (uint32_t)cols_per_buf;
 #pragma unroll
             for (int mt = 0; mt < MT; ++mt) {
-                bf16* orow = orow_a[mt]; const bf16* rrow = rrow_a[mt]; const float* tb = tb_a[mt];
+                T* orow = orow_a[mt]; const T* rrow = rrow_a[mt]; const float* tb = tb_a[mt];
                 const bool valid = orow != nullptr;
                 // (staging the tile in shared memory to emit full 128-byte lines per store instruction was measured
                 // SLOWER -- 153 vs 117 us at 96->96@64: the kernel is bound by L2 traffic, not store coalescing)
@@ -522,30 +522,30 @@ __global__ void __launch_bounds__(TC2_THREADS, 1) conv_tc2_kernel(const __grid_c
                                 }
                             }
                             if (rrow) {
-                                const __nv_bfloat162* ha = reinterpret_cast<const __nv_bfloat162*>(&rr[q][0]);
-                                const __nv_bfloat162* hb = reinterpret_cast<const __nv_bfloat162*>(&rr[q][1]);
+                                const typename Fmt16<T>::T2* ha = reinterpret_cast<const typename Fmt16<T>::T2*>(&rr[q][0]);
+                                const typename Fmt16<T>::T2* hb = reinterpret_cast<const typename Fmt16<T>::T2*>(&rr[q][1]);
 #pragma unroll
                                 for (int i = 0; i < 4; ++i) {
-                                    float2 fa = __bfloat1622float2(ha[i]), fb = __bfloat1622float2(hb[i]);
+                                    float2 fa = Fmt16<T>::to_f2(ha[i]), fb = Fmt16<T>::to_f2(hb[i]);
                                     v[2 * i] += fa.x; v[2 * i + 1] += fa.y; v[8 + 2 * i] += fb.x; v[8 + 2 * i + 1] += fb.y;
                                 }
                             }
                             if (p.accum) {
-                                const __nv_bfloat162* ha = reinterpret_cast<const __nv_bfloat162*>(&ra[q][0]);
-                                const __nv_bfloat162* hb = reinterpret_cast<const __nv_bfloat162*>(&ra[q][1]);
+                                const typename Fmt16<T>::T2* ha = reinterpret_cast<const typename Fmt16<T>::T2*>(&ra[q][0]);
+                                const typename Fmt16<T>::T2* hb = reinterpret_cast<const typename Fmt16<T>::T2*>(&ra[q][1]);
 #pragma unroll
                                 for (int i = 0; i < 4; ++i) {
-                                    float2 fa = __bfloat1622float2(ha[i]), fb = __bfloat1622float2(hb[i]);
+                                    float2 fa = Fmt16<T>::to_f2(ha[i]), fb = Fmt16<T>::to_f2(hb[i]);
                                     v[2 * i] += fa.x; v[2 * i + 1] += fa.y; v[8 + 2 * i] += fb.x; v[8 + 2 * i + 1] += fb.y;
                                 }
                             }
                             uint4 o0, o1;
-                            __nv_bfloat162* h0 = reinterpret_cast<__nv_bfloat162*>(&o0);
-                            __nv_bfloat162* h1 = reinterpret_cast<__nv_bfloat162*>(&o1);
+                            typename Fmt16<T>::T2* h0 = reinterpret_cast<typename Fmt16<T>::T2*>(&o0);
+                            typename Fmt16<T>::T2* h1 = reinterpret_cast<typename Fmt16<T>::T2*>(&o1);
 #pragma unroll
                             for (int i = 0; i < 4; ++i) {
-                                h0[i] = __floats2bfloat162_rn(v[2 * i], v[2 * i + 1]);
-                                h1[i] = __floats2bfloat162_rn(v[8 + 2 * i], v[8 + 2 * i + 1]);
+                                h0[i] = Fmt16<T>::from_f2(v[2 * i], v[2 * i + 1]);
+                                h1[i] = Fmt16<T>::from_f2(v[8 + 2 * i], v[8 + 2 * i + 1]);
                             }
                             if (p.v256) stg256(orow + c, o0, o1);
                             else { *reinterpret_cast<uint4*>(orow + c) = o0; *reinterpret_cast<uint4*>(orow + c + 8) = o1; }
@@ -564,8 +564,18 @@ __global__ void __launch_bounds__(TC2_THREADS, 1) conv_tc2_kernel(const __grid_c
     if (warp == 1) { tc_fence_after(); tmem_dealloc2(tmem_base, 512u); }
 }
 
-int conv_tc_launch(const ddpm_conv_args* a, cudaStream_t st) {
-    int rc = get_encode(); if (rc) return rc;
+#define CONV_TC2_ENTRY(NAME, T) \
+    template <int MT, int TAPS, bool FUSED2> \
+    __global__ void __launch_bounds__(TC2_THREADS, 1) NAME(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, \
+                                                           const __grid_constant__ CUtensorMap tmA2, const __grid_constant__ CUtensorMap tmB2, \
+                                                           Tc2Params p) { conv_tc2<T, MT, TAPS, FUSED2>(tmA, tmB, tmA2, tmB2, p); }
+CONV_TC2_ENTRY(conv_tc2_kernel, bf16)
+CONV_TC2_ENTRY(conv_tc2_f16_kernel, f16)
+#undef CONV_TC2_ENTRY
+
+template <typename T>
+static int conv_tc_launch_t(const ddpm_conv_args* a, cudaStream_t st) {
+    constexpr CUtensorMapDataType TM = Fmt16<T>::tma_type;
     Tc2Params p;
     p.out = TV(a->out);
     p.has_res = a->res.ptr != nullptr; p.res = p.has_res ? TV(a->res) : TV(a->out);
@@ -630,22 +640,22 @@ int conv_tc_launch(const ddpm_conv_args* a, cudaStream_t st) {
     if (p.KCH2) {
         uint64_t da[2] = {(uint64_t)a->in2.C, (uint64_t)p.Qtot}; uint64_t sa[1] = {(uint64_t)a->in2.pitch * 2};
         uint32_t ba[2] = {KC, (uint32_t)p.seg};
-        if (encode(&tmA2, a->in2.ptr, 2, da, sa, ba, CU_TENSOR_MAP_SWIZZLE_32B)) return 1;
+        if (encode(&tmA2, TM, a->in2.ptr, 2, da, sa, ba, CU_TENSOR_MAP_SWIZZLE_32B)) return 1;
         // 1x1 weights [Cout][1][Cin2] viewed as (c, n, tap = 1)
         uint64_t db[3] = {(uint64_t)a->in2.C, (uint64_t)p.Cout, 1};
         uint64_t sb[2] = {(uint64_t)a->in2.C * 2, (uint64_t)p.Cout * a->in2.C * 2};
         uint32_t bb[3] = {KC, (uint32_t)(p.NT / 2), 1};
-        if (encode(&tmB2, (void*)a->w2, 3, db, sb, bb, CU_TENSOR_MAP_SWIZZLE_32B)) return 1;
+        if (encode(&tmB2, TM, (void*)a->w2, 3, db, sb, bb, CU_TENSOR_MAP_SWIZZLE_32B)) return 1;
     }
     {
         uint64_t da[2] = {(uint64_t)p.Cin, (uint64_t)p.Qtot}; uint64_t sa[1] = {(uint64_t)a->in.pitch * 2};
         uint32_t ba[2] = {KC, (uint32_t)p.seg};
-        if (encode(&tmA, a->in.ptr, 2, da, sa, ba, CU_TENSOR_MAP_SWIZZLE_32B)) return 1;
+        if (encode(&tmA, TM, a->in.ptr, 2, da, sa, ba, CU_TENSOR_MAP_SWIZZLE_32B)) return 1;
         // weights [Cout][taps][Cin] viewed as (c, n, tap): one box brings all taps of NT/2 rows -> smem [tap][n][16 ch]
         uint64_t db[3] = {(uint64_t)p.Cin, (uint64_t)p.Cout, (uint64_t)p.taps};
         uint64_t sb[2] = {(uint64_t)p.taps * p.Cin * 2, (uint64_t)p.Cin * 2};
         uint32_t bb[3] = {KC, (uint32_t)(p.NT / 2), (uint32_t)p.taps};
-        if (encode(&tmB, (void*)a->w, 3, db, sb, bb, CU_TENSOR_MAP_SWIZZLE_32B)) return 1;
+        if (encode(&tmB, TM, (void*)a->w, 3, db, sb, bb, CU_TENSOR_MAP_SWIZZLE_32B)) return 1;
     }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(2 * pairs); cfg.blockDim = dim3(TC2_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
@@ -655,8 +665,9 @@ int conv_tc_launch(const ddpm_conv_args* a, cudaStream_t st) {
     cfg.attrs = at; cfg.numAttrs = 1;
     static size_t configured[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 #define TC2_GO(MTV, TAPSV, F2, SLOT) { \
-        if (smem > configured[SLOT]) { CUDA_TRY(cudaFuncSetAttribute(conv_tc2_kernel<MTV, TAPSV, F2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); configured[SLOT] = smem; } \
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, conv_tc2_kernel<MTV, TAPSV, F2>, tmA, tmB, F2 ? tmA2 : tmA, F2 ? tmB2 : tmB, p)); }
+        auto* kern = std::is_same<T, f16>::value ? conv_tc2_f16_kernel<MTV, TAPSV, F2> : conv_tc2_kernel<MTV, TAPSV, F2>; \
+        if (smem > configured[SLOT]) { CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); configured[SLOT] = smem; } \
+        CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, tmA, tmB, F2 ? tmA2 : tmA, F2 ? tmB2 : tmB, p)); }
     if (p.KCH2) { if (MT == 2) TC2_GO(2, 9, true, 4) else TC2_GO(1, 9, true, 5) }
     else if (p.taps == 4) { if (MT == 2) TC2_GO(2, 4, false, 6) else TC2_GO(1, 4, false, 7) }
     else if (MT == 2) { if (p.taps == 9) TC2_GO(2, 9, false, 0) else TC2_GO(2, 1, false, 1) }
@@ -664,6 +675,13 @@ int conv_tc_launch(const ddpm_conv_args* a, cudaStream_t st) {
 #undef TC2_GO
     LAUNCH_OK();
     return 0;
+}
+
+int conv_tc_launch(const ddpm_conv_args* a, cudaStream_t st) {
+    int rc = get_encode(); if (rc) return rc;
+    if (a->dtype == DDPM_BF16) return conv_tc_launch_t<bf16>(a, st);
+    if (a->dtype == DDPM_F16) return conv_tc_launch_t<f16>(a, st);
+    return DDPM_E_ARG;
 }
 
 // ================================================================================================
@@ -698,11 +716,11 @@ struct WgTcParams {
     float* dbias;               // fp32 [CoutV], accumulated by the reduce kernel
 };
 
-__global__ void __launch_bounds__(TC_THREADS) wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmY,
-                                                               const __grid_constant__ CUtensorMap tmA, WgTcParams p) {
+template <typename T>
+__device__ __forceinline__ void wgrad_tc(const CUtensorMap& tmY, const CUtensorMap& tmA, WgTcParams p) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    uint8_t* ones = smem + (size_t)WG_STAGES * p.stage_bytes;            // [16 px][64 ch] of bf16 1.0 (2 KB, 1024-aligned)
+    uint8_t* ones = smem + (size_t)WG_STAGES * p.stage_bytes;            // [16 px][64 ch] of 1.0 (2 KB, 1024-aligned)
     uint64_t* full = (uint64_t*)(ones + 2048);
     uint64_t* empty = full + WG_STAGES;
     uint64_t* acc_full = empty + WG_STAGES;
@@ -731,7 +749,7 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc_kernel(const __grid_const
     }
     if (warp == 1) tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols);
     if (do_bias && warp >= 2) {
-        for (int i = threadIdx.x - 64; i < 2048 / 4; i += TC_THREADS - 64) reinterpret_cast<uint32_t*>(ones)[i] = 0x3F803F80u;
+        for (int i = threadIdx.x - 64; i < 2048 / 4; i += TC_THREADS - 64) reinterpret_cast<uint32_t*>(ones)[i] = (uint32_t)Fmt16<T>::one * 0x10001u;
         fence_proxy_async();                             // generic-proxy writes -> visible to the tensor core's async proxy
     }
     tc_fence_before();
@@ -759,14 +777,14 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc_kernel(const __grid_const
         {   // whole warp, warp-uniform control flow; one elected lane issues tcgen05 instructions
             const bool el = elect_one();
             // a_major = b_major = MN (bits 15, 16); M = 128; N = NT
-            const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) |
+            const uint32_t idesc = (1u << 4) | Fmt16<T>::idesc_ab | (1u << 15) | (1u << 16) |
                                    ((uint32_t)(p.NT >> 3) << 17) | ((128u >> 4) << 24);
             const uint32_t hi = desc_hi(1024u, 2u);                      // SBO 1024 B, SWIZZLE_128B
             const uint32_t y_lo0 = desc_lo(smem_u32(smem), (uint32_t)(WG_KQ * 128));
             const uint32_t a_lo0 = desc_lo(smem_u32(smem) + (uint32_t)y_bytes, (uint32_t)(WG_ROWS * 128));
             const uint32_t stage16 = (uint32_t)(p.stage_bytes >> 4);
             const bool three = p.ntap == 3;
-            const uint32_t idesc_b = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) | ((16u >> 3) << 17) | ((128u >> 4) << 24);
+            const uint32_t idesc_b = (1u << 4) | Fmt16<T>::idesc_ab | (1u << 15) | (1u << 16) | ((16u >> 3) << 17) | ((128u >> 4) << 24);
             const uint64_t ones_desc = desc_pack(desc_lo(smem_u32(ones), 2048u), hi);
             // two copies of the loop: a predicated-off bias MMA in the common loop cost 11 % (measured A/B)
             auto run = [&](auto with_bias, auto with_three) {
@@ -781,13 +799,13 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc_kernel(const __grid_const
 #pragma unroll
                     for (int ks = 0; ks < WG_KQ / 16; ++ks) {
                         const uint64_t ydesc = desc_pack(y_lo + (uint32_t)(ks * 16 * 128 / 16), hi);
-                        if (el) umma_bf16(tmem_base, ydesc, desc_pack(a_lo + (uint32_t)((ks * 16) * 8), hi), idesc, ks == 0 ? acc : 1u);
+                        if (el) umma_f16(tmem_base, ydesc, desc_pack(a_lo + (uint32_t)((ks * 16) * 8), hi), idesc, ks == 0 ? acc : 1u);
                         if (THREE && el) {
-                            umma_bf16(tmem_base + (uint32_t)p.NT, ydesc, desc_pack(a_lo + (uint32_t)((ks * 16 + 1) * 8), hi), idesc, ks == 0 ? acc : 1u);
-                            umma_bf16(tmem_base + (uint32_t)(2 * p.NT), ydesc, desc_pack(a_lo + (uint32_t)((ks * 16 + 2) * 8), hi), idesc, ks == 0 ? acc : 1u);
+                            umma_f16(tmem_base + (uint32_t)p.NT, ydesc, desc_pack(a_lo + (uint32_t)((ks * 16 + 1) * 8), hi), idesc, ks == 0 ? acc : 1u);
+                            umma_f16(tmem_base + (uint32_t)(2 * p.NT), ydesc, desc_pack(a_lo + (uint32_t)((ks * 16 + 2) * 8), hi), idesc, ks == 0 ? acc : 1u);
                         }
                         if (BIAS) {
-                            if (kmod == grp) { if (el) umma_bf16(tmem_base + bias_col, ydesc, ones_desc, idesc_b, accb); accb = 1; }
+                            if (kmod == grp) { if (el) umma_f16(tmem_base + bias_col, ydesc, ones_desc, idesc_b, accb); accb = 1; }
                             if (++kmod == ngrp) kmod = 0;
                         }
                     }
@@ -852,11 +870,11 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc_kernel(const __grid_const
 // The epilogue, the workspace layout and the reduce kernel are those of the single-CTA kernel.
 // ================================================================================================
 #define WG2_STAGES 6
-__global__ void __launch_bounds__(TC_THREADS) wgrad_tc2_kernel(const __grid_constant__ CUtensorMap tmY,
-                                                                const __grid_constant__ CUtensorMap tmA, WgTcParams p) {
+template <typename T>
+__device__ __forceinline__ void wgrad_tc2(const CUtensorMap& tmY, const CUtensorMap& tmA, WgTcParams p) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    uint8_t* ones = smem + (size_t)WG2_STAGES * p.stage_bytes;           // [16 px][64 ch] of bf16 1.0 (2 KB, 1024-aligned)
+    uint8_t* ones = smem + (size_t)WG2_STAGES * p.stage_bytes;           // [16 px][64 ch] of 1.0 (2 KB, 1024-aligned)
     uint64_t* full = (uint64_t*)(ones + 2048);
     uint64_t* empty = full + WG2_STAGES;
     uint64_t* acc_full = empty + WG2_STAGES;
@@ -885,7 +903,7 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc2_kernel(const __grid_cons
     }
     if (warp == 1) tmem_alloc2(tmem_slot, (uint32_t)p.tmem_cols);
     if (do_bias && warp >= 2) {
-        for (int i = threadIdx.x - 64; i < 2048 / 4; i += TC_THREADS - 64) reinterpret_cast<uint32_t*>(ones)[i] = 0x3F803F80u;
+        for (int i = threadIdx.x - 64; i < 2048 / 4; i += TC_THREADS - 64) reinterpret_cast<uint32_t*>(ones)[i] = (uint32_t)Fmt16<T>::one * 0x10001u;
         fence_proxy_async();
     }
     tc_fence_before();
@@ -916,14 +934,14 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc2_kernel(const __grid_cons
         if (leader) {
             const bool el = elect_one();
             // a_major = b_major = MN (bits 15, 16); M = 256 over the pair; N = NT (each CTA holds NT/2 patch channels)
-            const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) |
+            const uint32_t idesc = (1u << 4) | Fmt16<T>::idesc_ab | (1u << 15) | (1u << 16) |
                                    ((uint32_t)(p.NT >> 3) << 17) | ((256u >> 4) << 24);
             const uint32_t hi = desc_hi(1024u, 2u);                      // SBO 1024 B, SWIZZLE_128B
             const uint32_t y_lo0 = desc_lo(smem_u32(smem), (uint32_t)(WG_KQ * 128));
             const uint32_t a_lo0 = desc_lo(smem_u32(smem) + (uint32_t)y_bytes, (uint32_t)(WG_ROWS * 128));
             const uint32_t stage16 = (uint32_t)(p.stage_bytes >> 4);
             const bool three = p.ntap == 3;
-            const uint32_t idesc_b = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) | ((16u >> 3) << 17) | ((256u >> 4) << 24);
+            const uint32_t idesc_b = (1u << 4) | Fmt16<T>::idesc_ab | (1u << 15) | (1u << 16) | ((16u >> 3) << 17) | ((256u >> 4) << 24);
             const uint64_t ones_desc = desc_pack(desc_lo(smem_u32(ones), 2048u), hi);
             auto run = [&](auto with_bias, auto with_three) {
                 constexpr bool BIAS = decltype(with_bias)::value, THREE = decltype(with_three)::value;
@@ -937,13 +955,13 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc2_kernel(const __grid_cons
 #pragma unroll
                     for (int ks = 0; ks < WG_KQ / 16; ++ks) {
                         const uint64_t ydesc = desc_pack(y_lo + (uint32_t)(ks * 16 * 128 / 16), hi);
-                        if (el) umma2_bf16(tmem_base, ydesc, desc_pack(a_lo + (uint32_t)((ks * 16) * 8), hi), idesc, ks == 0 ? acc : 1u);
+                        if (el) umma2_f16(tmem_base, ydesc, desc_pack(a_lo + (uint32_t)((ks * 16) * 8), hi), idesc, ks == 0 ? acc : 1u);
                         if (THREE && el) {
-                            umma2_bf16(tmem_base + (uint32_t)p.NT, ydesc, desc_pack(a_lo + (uint32_t)((ks * 16 + 1) * 8), hi), idesc, ks == 0 ? acc : 1u);
-                            umma2_bf16(tmem_base + (uint32_t)(2 * p.NT), ydesc, desc_pack(a_lo + (uint32_t)((ks * 16 + 2) * 8), hi), idesc, ks == 0 ? acc : 1u);
+                            umma2_f16(tmem_base + (uint32_t)p.NT, ydesc, desc_pack(a_lo + (uint32_t)((ks * 16 + 1) * 8), hi), idesc, ks == 0 ? acc : 1u);
+                            umma2_f16(tmem_base + (uint32_t)(2 * p.NT), ydesc, desc_pack(a_lo + (uint32_t)((ks * 16 + 2) * 8), hi), idesc, ks == 0 ? acc : 1u);
                         }
                         if (BIAS) {
-                            if (kmod == grp) { if (el) umma2_bf16(tmem_base + bias_col, ydesc, ones_desc, idesc_b, accb); accb = 1; }
+                            if (kmod == grp) { if (el) umma2_f16(tmem_base + bias_col, ydesc, ones_desc, idesc_b, accb); accb = 1; }
                             if (++kmod == ngrp) kmod = 0;
                         }
                     }
@@ -993,6 +1011,16 @@ __global__ void __launch_bounds__(TC_THREADS) wgrad_tc2_kernel(const __grid_cons
     cluster_sync_all();                                  // nobody exits (or frees TMEM) while the pair is still working
     if (warp == 1) { tc_fence_after(); tmem_dealloc2(tmem_base, (uint32_t)p.tmem_cols); }
 }
+
+// entry points of the two weight-gradient bodies per element type (bf16 keeps its names)
+#define WGRAD_TC_ENTRY(NAME, BODY, T) \
+    __global__ void __launch_bounds__(TC_THREADS) NAME(const __grid_constant__ CUtensorMap tmY, const __grid_constant__ CUtensorMap tmA, \
+                                                       WgTcParams p) { BODY<T>(tmY, tmA, p); }
+WGRAD_TC_ENTRY(wgrad_tc_kernel, wgrad_tc, bf16)
+WGRAD_TC_ENTRY(wgrad_tc_f16_kernel, wgrad_tc, f16)
+WGRAD_TC_ENTRY(wgrad_tc2_kernel, wgrad_tc2, bf16)
+WGRAD_TC_ENTRY(wgrad_tc2_f16_kernel, wgrad_tc2, f16)
+#undef WGRAD_TC_ENTRY
 
 // dw[co][ci][ky][kx] += sum_split ws[split][mtile][ky*n_tiles+ntile][co%128][kx*NT + ci%NT]
 __global__ void wgrad_reduce_kernel(const float* __restrict__ ws, float* __restrict__ dw, int splits, WgTcParams p) {
@@ -1083,7 +1111,7 @@ extern "C" int64_t ddpm_wgrad_workspace_bytes(const ddpm_wgrad_args* a) {
 }
 
 int wgrad_tc_supported(const ddpm_wgrad_args* a) {
-    if (a->dtype != DDPM_BF16 || a->stride != 1 || a->a_silu) return 0;
+    if ((a->dtype != DDPM_BF16 && a->dtype != DDPM_F16) || a->stride != 1 || a->a_silu) return 0;
     if (!((a->KH == 3 && a->KW == 3 && a->pad == 1) || (a->KH == 1 && a->KW == 1 && a->pad == 0))) return 0;
     const ddpm_tensor &x = a->act, &y = a->dy;
     if (x.halo != 1 || y.halo != 1 || x.H != y.H || x.W != y.W || x.N != y.N) return 0;
@@ -1094,8 +1122,9 @@ int wgrad_tc_supported(const ddpm_wgrad_args* a) {
     return 1;
 }
 
-int wgrad_tc_launch(const ddpm_wgrad_args* a, cudaStream_t st) {
-    int rc = get_encode(); if (rc) return rc;
+template <typename T>
+static int wgrad_tc_launch_t(const ddpm_wgrad_args* a, cudaStream_t st) {
+    constexpr CUtensorMapDataType TM = Fmt16<T>::tma_type;
     WgTcParams p; int splits; wg_plan(a, &p, &splits);
     const int64_t main_bytes = (int64_t)splits * p.m_tiles * p.ntap * p.n_tiles * 128 * p.ntap * p.NT * 4;
     int64_t need = main_bytes + (int64_t)splits * p.ntap * p.n_tiles * p.m_tiles * 128 * 4;
@@ -1107,18 +1136,21 @@ int wgrad_tc_launch(const ddpm_wgrad_args* a, cudaStream_t st) {
     {
         uint64_t d[2] = {(uint64_t)p.Cout, (uint64_t)p.Qtot}; uint64_t s[1] = {(uint64_t)a->dy.pitch * 2};
         uint32_t b[2] = {64, WG_KQ};
-        if (encode(&tmY, a->dy.ptr, 2, d, s, b, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
+        if (encode(&tmY, TM, a->dy.ptr, 2, d, s, b, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
     }
     {
         uint64_t d[2] = {(uint64_t)p.Cin, (uint64_t)p.Qtot}; uint64_t s[1] = {(uint64_t)a->act.pitch * 2};
         uint32_t b[2] = {64, WG_ROWS};
-        if (encode(&tmA, a->act.ptr, 2, d, s, b, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
+        if (encode(&tmA, TM, a->act.ptr, 2, d, s, b, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
     }
+    constexpr bool H = std::is_same<T, f16>::value;
+    auto* kern2 = H ? wgrad_tc2_f16_kernel : wgrad_tc2_kernel;
+    auto* kern1 = H ? wgrad_tc_f16_kernel : wgrad_tc_kernel;
     if (wg_pair(p)) {
         const size_t smem2 = (size_t)WG2_STAGES * p.stage_bytes + 2048 + 8 * (2 * WG2_STAGES + 1) + 16 + 1024;
         static size_t configured2 = 0;
         if (smem2 > configured2) {
-            CUDA_TRY(cudaFuncSetAttribute(wgrad_tc2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
+            CUDA_TRY(cudaFuncSetAttribute(kern2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
             configured2 = smem2;
         }
         cudaLaunchConfig_t cfg = {};
@@ -1127,15 +1159,15 @@ int wgrad_tc_launch(const ddpm_wgrad_args* a, cudaStream_t st) {
         at[0].id = cudaLaunchAttributeClusterDimension;
         at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
         cfg.attrs = at; cfg.numAttrs = 1;
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, wgrad_tc2_kernel, tmY, tmA, p));
+        CUDA_TRY(cudaLaunchKernelEx(&cfg, kern2, tmY, tmA, p));
     } else {
         const size_t smem = (size_t)WG_STAGES * p.stage_bytes + 2048 + 8 * (2 * WG_STAGES + 1) + 16 + 1024;
         static size_t configured = 0;
         if (smem > configured) {
-            CUDA_TRY(cudaFuncSetAttribute(wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            CUDA_TRY(cudaFuncSetAttribute(kern1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             configured = smem;
         }
-        CUDA_TRY(launch_kernel(wgrad_tc_kernel, dim3(splits, p.ntap * p.n_tiles, p.m_tiles), dim3(TC_THREADS), smem, st, tmY, tmA, p));
+        CUDA_TRY(launch_kernel(kern1, dim3(splits, p.ntap * p.n_tiles, p.m_tiles), dim3(TC_THREADS), smem, st, tmY, tmA, p));
     }
     LAUNCH_OK();
     int total = p.CoutV * p.ntap * p.ntap * p.CinV;
@@ -1143,4 +1175,11 @@ int wgrad_tc_launch(const ddpm_wgrad_args* a, cudaStream_t st) {
     CUDA_TRY(launch_kernel(wgrad_reduce_kernel, dim3(rg), dim3(256), 0, st, (const float*)p.ws, a->dw, splits, p));
     LAUNCH_OK();
     return 0;
+}
+
+int wgrad_tc_launch(const ddpm_wgrad_args* a, cudaStream_t st) {
+    int rc = get_encode(); if (rc) return rc;
+    if (a->dtype == DDPM_BF16) return wgrad_tc_launch_t<bf16>(a, st);
+    if (a->dtype == DDPM_F16) return wgrad_tc_launch_t<f16>(a, st);
+    return DDPM_E_ARG;
 }

@@ -84,25 +84,23 @@ __device__ __forceinline__ int clamp_t(int64_t t, int T) {
     return (int)(t < 0 ? 0 : (t > T - 1 ? T - 1 : t));
 }
 
-template <typename T> __device__ __forceinline__ float4 ld4(const T* p, int64_t i);
+template <typename T> __device__ __forceinline__ float4 ld4(const T* p, int64_t i) {     // bf16 / fp16
+    uint2 r = *reinterpret_cast<const uint2*>(p + i);
+    float2 a = unpack2<T>(r.x);
+    float2 b = unpack2<T>(r.y);
+    return make_float4(a.x, a.y, b.x, b.y);
+}
+template <typename T> __device__ __forceinline__ void st4(T* p, int64_t i, float4 v) {     // bf16 / fp16
+    uint2 r;
+    pack2<T>(r.x, v.x, v.y);
+    pack2<T>(r.y, v.z, v.w);
+    *reinterpret_cast<uint2*>(p + i) = r;
+}
 template <> __device__ __forceinline__ float4 ld4<float>(const float* p, int64_t i) {
     return *reinterpret_cast<const float4*>(p + i);
 }
-template <> __device__ __forceinline__ float4 ld4<bf16>(const bf16* p, int64_t i) {
-    uint2 r = *reinterpret_cast<const uint2*>(p + i);
-    float2 a = __bfloat1622float2(*reinterpret_cast<__nv_bfloat162*>(&r.x));
-    float2 b = __bfloat1622float2(*reinterpret_cast<__nv_bfloat162*>(&r.y));
-    return make_float4(a.x, a.y, b.x, b.y);
-}
-template <typename T> __device__ __forceinline__ void st4(T* p, int64_t i, float4 v);
 template <> __device__ __forceinline__ void st4<float>(float* p, int64_t i, float4 v) {
     *reinterpret_cast<float4*>(p + i) = v;
-}
-template <> __device__ __forceinline__ void st4<bf16>(bf16* p, int64_t i, float4 v) {
-    uint2 r;
-    *reinterpret_cast<__nv_bfloat162*>(&r.x) = __floats2bfloat162_rn(v.x, v.y);
-    *reinterpret_cast<__nv_bfloat162*>(&r.y) = __floats2bfloat162_rn(v.z, v.w);
-    *reinterpret_cast<uint2*>(p + i) = r;
 }
 
 #define EW_THREADS 256
@@ -225,6 +223,9 @@ extern "C" int ddpm_mse_fwd(const void* pred, int pred_dtype, const float* noise
     } else if (pred_dtype == DDPM_BF16) {
         if (vec) mse_fwd_kernel<bf16, true><<<grid, EW_THREADS, 0, st>>>((const bf16*)pred, noise, weight, loss, B, chw);
         else mse_fwd_kernel<bf16, false><<<grid, EW_THREADS, 0, st>>>((const bf16*)pred, noise, weight, loss, B, chw);
+    } else if (pred_dtype == DDPM_F16) {
+        if (vec) mse_fwd_kernel<f16, true><<<grid, EW_THREADS, 0, st>>>((const f16*)pred, noise, weight, loss, B, chw);
+        else mse_fwd_kernel<f16, false><<<grid, EW_THREADS, 0, st>>>((const f16*)pred, noise, weight, loss, B, chw);
     } else return DDPM_E_ARG;
     LAUNCH_OK();
     return 0;
@@ -251,6 +252,9 @@ extern "C" int ddpm_mse_bwd(const void* pred, int pred_dtype, const float* noise
         return launch_ew(f, B, chw, al16(pred) && al16(noise) && al16(dpred), st);
     } else if (pred_dtype == DDPM_BF16) {
         MseBwd<bf16> f{(const bf16*)pred, noise, weight, gout, (bf16*)dpred, inv};
+        return launch_ew(f, B, chw, al8(pred) && al16(noise) && al8(dpred), st);
+    } else if (pred_dtype == DDPM_F16) {
+        MseBwd<f16> f{(const f16*)pred, noise, weight, gout, (f16*)dpred, inv};
         return launch_ew(f, B, chw, al8(pred) && al16(noise) && al8(dpred), st);
     }
     return DDPM_E_ARG;
@@ -322,6 +326,7 @@ extern "C" int ddpm_x0_absmax(void* sched, const float* xt, const void* eps, int
                      absmax_kernel<TE, CN><<<grid, EW_THREADS, 0, st>>>(a, chw); }
     if (eps_dtype == DDPM_F32) { if (uc) GO(float, true) else GO(float, false) }
     else if (eps_dtype == DDPM_BF16) { if (uc) GO(bf16, true) else GO(bf16, false) }
+    else if (eps_dtype == DDPM_F16) { if (uc) GO(f16, true) else GO(f16, false) }
     else return DDPM_E_ARG;
 #undef GO
     LAUNCH_OK();
@@ -371,6 +376,7 @@ extern "C" int ddpm_p_sample_step(void* sched, const float* xt, const void* eps,
                      return launch_ew(f, B, chw, al, st); }
     if (eps_dtype == DDPM_F32) { if (uc) GO(float, true) else GO(float, false) }
     else if (eps_dtype == DDPM_BF16) { if (uc) GO(bf16, true) else GO(bf16, false) }
+    else if (eps_dtype == DDPM_F16) { if (uc) GO(f16, true) else GO(f16, false) }
 #undef GO
     return DDPM_E_ARG;
 }
@@ -427,6 +433,7 @@ extern "C" int ddpm_ddim_step(void* sched, const float* xt, const void* eps, int
                      return launch_ew(f, B, chw, al, st); }
     if (eps_dtype == DDPM_F32) { if (uc) GO(float, true) else GO(float, false) }
     else if (eps_dtype == DDPM_BF16) { if (uc) GO(bf16, true) else GO(bf16, false) }
+    else if (eps_dtype == DDPM_F16) { if (uc) GO(f16, true) else GO(f16, false) }
 #undef GO
     return DDPM_E_ARG;
 }
@@ -551,10 +558,10 @@ __global__ void layout_pix_kernel(char* nchw, int64_t sn, int64_t sc, int64_t sh
 #pragma unroll
                 for (int j = 0; j < 8; ++j) f[j] = (c0 + j < srcC) ? ldf<TS>(sp + (int64_t)(c0 + j) * sc) : 0.f;
                 if (sizeof(TD) == 2 && c0 + 8 <= v.C && ((uintptr_t)(d + c0) & 15) == 0) {
-                    uint4 o; __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(&o);
+                    Vec16<TD> o;
 #pragma unroll
-                    for (int j = 0; j < 4; ++j) h[j] = __floats2bfloat162_rn(f[2 * j], f[2 * j + 1]);
-                    *reinterpret_cast<uint4*>(d + c0) = o;
+                    for (int j = 0; j < 8; ++j) o.v[j] = f[j];
+                    o.store(d + c0);
                 } else {
 #pragma unroll
                     for (int j = 0; j < 8; ++j) if (c0 + j < v.C) stf<TD>(d + c0 + j, f[j]);
@@ -572,6 +579,16 @@ __global__ void layout_pix_kernel(char* nchw, int64_t sn, int64_t sc, int64_t sh
             const int64_t px = (int64_t)v.N * v.H * v.W; int g = (int)((px + 255) / 256); if (g > 148 * 16) g = 148 * 16; \
             CUDA_TRY(launch_kernel(layout_pix_kernel<TS, TD, DIR>, dim3(g), dim3(256), 0, st, PTR, sn, sc, sh, sw, v, SRCC)); \
         } else layout_kernel<TS, TD, DIR><<<grid, 256, 0, st>>>(PTR, sn, sc, sh, sw, v, SRCC); }
+// every pair of the three element types (a caller's fp32 / bf16 / fp16 tensor <-> the compute dtype)
+#define LAYOUT_DST(TS, DIR, PTR, SRCC) \
+    if (dst_dtype == DDPM_F32) LAYOUT_GO(TS, float, DIR, PTR, SRCC) \
+    else if (dst_dtype == DDPM_BF16) LAYOUT_GO(TS, bf16, DIR, PTR, SRCC) \
+    else if (dst_dtype == DDPM_F16) LAYOUT_GO(TS, f16, DIR, PTR, SRCC) \
+    else return DDPM_E_ARG;
+#define LAYOUT_DISPATCH(DIR, PTR, SRCC) \
+    if (src_dtype == DDPM_F32) { LAYOUT_DST(float, DIR, PTR, SRCC) } \
+    else if (src_dtype == DDPM_BF16) { LAYOUT_DST(bf16, DIR, PTR, SRCC) } \
+    else if (src_dtype == DDPM_F16) { LAYOUT_DST(f16, DIR, PTR, SRCC) }
 
 extern "C" int ddpm_nchw_to_nhwc(const void* src, int src_dtype, int src_C, int64_t sn, int64_t sc, int64_t sh,
                                  int64_t sw, const ddpm_tensor* dst, int dst_dtype, void* stream) {
@@ -581,10 +598,7 @@ extern "C" int ddpm_nchw_to_nhwc(const void* src, int src_dtype, int src_C, int6
     int64_t total = (int64_t)v.N * v.H * v.W * v.C;
     int grid = (int)((total + 255) / 256); if (grid > 148 * 16) grid = 148 * 16;
     char* s = (char*)src;
-    if (src_dtype == DDPM_F32 && dst_dtype == DDPM_F32) LAYOUT_GO(float, float, true, s, srcC)
-    else if (src_dtype == DDPM_F32 && dst_dtype == DDPM_BF16) LAYOUT_GO(float, bf16, true, s, srcC)
-    else if (src_dtype == DDPM_BF16 && dst_dtype == DDPM_BF16) LAYOUT_GO(bf16, bf16, true, s, srcC)
-    else if (src_dtype == DDPM_BF16 && dst_dtype == DDPM_F32) LAYOUT_GO(bf16, float, true, s, srcC)
+    LAYOUT_DISPATCH(true, s, srcC)
     else return DDPM_E_ARG;
     LAUNCH_OK();
     return 0;
@@ -597,10 +611,7 @@ extern "C" int ddpm_nhwc_to_nchw(const ddpm_tensor* src, int src_dtype, void* ds
     int64_t total = (int64_t)v.N * v.H * v.W * v.C;
     int grid = (int)((total + 255) / 256); if (grid > 148 * 16) grid = 148 * 16;
     char* d = (char*)dst;
-    if (src_dtype == DDPM_F32 && dst_dtype == DDPM_F32) LAYOUT_GO(float, float, false, d, v.C)
-    else if (src_dtype == DDPM_BF16 && dst_dtype == DDPM_F32) LAYOUT_GO(bf16, float, false, d, v.C)
-    else if (src_dtype == DDPM_BF16 && dst_dtype == DDPM_BF16) LAYOUT_GO(bf16, bf16, false, d, v.C)
-    else if (src_dtype == DDPM_F32 && dst_dtype == DDPM_BF16) LAYOUT_GO(float, bf16, false, d, v.C)
+    LAYOUT_DISPATCH(false, d, v.C)
     else return DDPM_E_ARG;
     LAUNCH_OK();
     return 0;
@@ -630,6 +641,7 @@ extern "C" int ddpm_sinusoid(const void* t, int t_is_float, int B, int dim, void
     int grid = ceil_div((int64_t)B * dim, 256);
     if (dtype == DDPM_F32) sinusoid_kernel<float><<<grid, 256, 0, st>>>(t, t_is_float, B, dim, (float*)out);
     else if (dtype == DDPM_BF16) sinusoid_kernel<bf16><<<grid, 256, 0, st>>>(t, t_is_float, B, dim, (bf16*)out);
+    else if (dtype == DDPM_F16) sinusoid_kernel<f16><<<grid, 256, 0, st>>>(t, t_is_float, B, dim, (f16*)out);
     else return DDPM_E_ARG;
     LAUNCH_OK();
     return 0;

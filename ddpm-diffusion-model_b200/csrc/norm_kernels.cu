@@ -64,10 +64,10 @@ template <typename T, int VEC> __device__ __forceinline__ void unraw(const Raw<T
     else if constexpr (sizeof(T) == 4) {
         v[0] = __uint_as_float(r.q.x); v[1] = __uint_as_float(r.q.y); v[2] = __uint_as_float(r.q.z); v[3] = __uint_as_float(r.q.w);
     } else {
-        // low half: shift, high half: mask -- one integer instruction per element (__bfloat1622float2 costs 1.5: PRMT + shift)
+        // bf16: low half shift, high half mask -- one integer instruction per element (__bfloat1622float2 costs 1.5: PRMT + shift)
         const uint32_t w[4] = {r.q.x, r.q.y, r.q.z, r.q.w};
 #pragma unroll
-        for (int i = 0; i < 4; ++i) { v[2 * i] = __uint_as_float(w[i] << 16); v[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u); }
+        for (int i = 0; i < 4; ++i) Fmt16<T>::unpack(w[i], v[2 * i], v[2 * i + 1]);
     }
 }
 
@@ -245,7 +245,7 @@ template <typename T, int VEC, int MODE>
 __global__ void __launch_bounds__(NT, GN_FWD_OCC) gn_fwd_kernel(GnP a) {
     extern __shared__ __align__(16) unsigned char gsm[];
     const int C = a.x.C, G = a.G, cpg = C / G, HW = a.x.H * a.x.W;
-    constexpr bool FAST_ACT = sizeof(T) == 2;                // bf16 tensors: tanh-based SiLU (common.cuh)
+    constexpr bool FAST_ACT = std::is_same<T, bf16>::value;  // bf16 tensors: tanh-based SiLU; fp16 keeps the exact form (common.cuh)
     constexpr int RING = gn_ring_bytes<VEC, 1, GN_PIPE_D_FWD>();
     unsigned char* ring = gsm;
     float (*part)[NT] = reinterpret_cast<float (*)[NT]>(gsm);    // aliases the ring (see gn_ring_bytes)
@@ -341,7 +341,7 @@ template <typename T, int VEC, bool STASH>
 __global__ void __launch_bounds__(NT, STASH ? GN_BWD_OCC : 2) gn_bwd_kernel(GnP a) {
     extern __shared__ __align__(16) unsigned char gsm[];
     const int C = a.x.C, G = a.G, cpg = C / G, HW = a.x.H * a.x.W;
-    constexpr bool FAST_ACT = sizeof(T) == 2;                // bf16 tensors: tanh-based SiLU (common.cuh)
+    constexpr bool FAST_ACT = std::is_same<T, bf16>::value;  // bf16 tensors: tanh-based SiLU; fp16 keeps the exact form (common.cuh)
     constexpr int RING = gn_ring_bytes<VEC, 3>();
     unsigned char* ring = gsm;
     float (*part)[NT] = reinterpret_cast<float (*)[NT]>(gsm);    // aliases the ring (see gn_ring_bytes)
@@ -556,6 +556,7 @@ static int gn_fwd_dispatch(GnP& p, const ddpm_tensor* x, const ddpm_tensor* out,
     const bool v8 = vec_ok(x, 8, 2) && (MODE == 1 || vec_ok(out, 8, 2));
     const bool v4 = vec_ok(x, 4, 4) && (MODE == 1 || vec_ok(out, 4, 4));
     if (dtype == DDPM_BF16) { if (v8) GO(bf16, 8) else GO(bf16, 1) }
+    else if (dtype == DDPM_F16) { if (v8) GO(f16, 8) else GO(f16, 1) }
     else if (dtype == DDPM_F32) { if (v4) GO(float, 4) else GO(float, 1) }
 #undef GO
     return DDPM_E_ARG;
@@ -608,6 +609,7 @@ static int gn_bwd_impl(const ddpm_tensor* x, int dtype, int groups, const double
         if (p.stash) return launch_cluster(gn_bwd_kernel<T, VEC, true>, x->N * cs, cs, sm, st, p); \
         return launch_cluster(gn_bwd_kernel<T, VEC, false>, x->N * cs, cs, sm, st, p); }
     if (dtype == DDPM_BF16) { if (vec_ok(x, 8, 2) && vec_ok(dy, 8, 2) && vec_ok(dx, 8, 2)) GO(bf16, 8) else GO(bf16, 1) }
+    else if (dtype == DDPM_F16) { if (vec_ok(x, 8, 2) && vec_ok(dy, 8, 2) && vec_ok(dx, 8, 2)) GO(f16, 8) else GO(f16, 1) }
     else if (dtype == DDPM_F32) { if (vec_ok(x, 4, 4) && vec_ok(dy, 4, 4) && vec_ok(dx, 4, 4)) GO(float, 4) else GO(float, 1) }
 #undef GO
     return DDPM_E_ARG;
@@ -662,6 +664,7 @@ extern "C" int ddpm_upsample2x(const ddpm_tensor* x, const ddpm_tensor* out, int
 #define GO(T, VEC) { UpFwd<T, VEC> f{TV(*x), TV(*out)}; int64_t tot = (int64_t)out->N * out->H * out->W * (out->C / VEC); \
         if (launch_kernel(pix_kernel<T, VEC, decltype(f)>, dim3(pix_grid(tot)), dim3(NT), 0, st, out->N, out->H, out->W, out->C, f) != cudaSuccess) return (int)cudaGetLastError(); }
     if (dtype == DDPM_BF16) { if (vec_ok(x, 8, 2) && vec_ok(out, 8, 2)) GO(bf16, 8) else GO(bf16, 1) }
+    else if (dtype == DDPM_F16) { if (vec_ok(x, 8, 2) && vec_ok(out, 8, 2)) GO(f16, 8) else GO(f16, 1) }
     else if (dtype == DDPM_F32) { if (vec_ok(x, 4, 4) && vec_ok(out, 4, 4)) GO(float, 4) else GO(float, 1) }
     else return DDPM_E_ARG;
 #undef GO
@@ -691,6 +694,7 @@ extern "C" int ddpm_upsample2x_bwd(const ddpm_tensor* dy, const ddpm_tensor* dx,
 #define GO(T, VEC) { UpBwd<T, VEC> f{TV(*dy), TV(*dx), accumulate}; int64_t tot = (int64_t)dx->N * dx->H * dx->W * (dx->C / VEC); \
         if (launch_kernel(pix_kernel<T, VEC, decltype(f)>, dim3(pix_grid(tot)), dim3(NT), 0, st, dx->N, dx->H, dx->W, dx->C, f) != cudaSuccess) return (int)cudaGetLastError(); }
     if (dtype == DDPM_BF16) { if (vec_ok(dy, 8, 2) && vec_ok(dx, 8, 2)) GO(bf16, 8) else GO(bf16, 1) }
+    else if (dtype == DDPM_F16) { if (vec_ok(dy, 8, 2) && vec_ok(dx, 8, 2)) GO(f16, 8) else GO(f16, 1) }
     else if (dtype == DDPM_F32) { if (vec_ok(dy, 4, 4) && vec_ok(dx, 4, 4)) GO(float, 4) else GO(float, 1) }
     else return DDPM_E_ARG;
 #undef GO
@@ -716,6 +720,7 @@ extern "C" int ddpm_zero_upsample2x(const ddpm_tensor* x, const ddpm_tensor* out
 #define GO(T, VEC) { ZeroUp<T, VEC> f{TV(*x), TV(*out)}; int64_t tot = (int64_t)out->N * out->H * out->W * (out->C / VEC); \
         if (launch_kernel(pix_kernel<T, VEC, decltype(f)>, dim3(pix_grid(tot)), dim3(NT), 0, st, out->N, out->H, out->W, out->C, f) != cudaSuccess) return (int)cudaGetLastError(); }
     if (dtype == DDPM_BF16) { if (vec_ok(x, 8, 2) && vec_ok(out, 8, 2)) GO(bf16, 8) else GO(bf16, 1) }
+    else if (dtype == DDPM_F16) { if (vec_ok(x, 8, 2) && vec_ok(out, 8, 2)) GO(f16, 8) else GO(f16, 1) }
     else if (dtype == DDPM_F32) { if (vec_ok(x, 4, 4) && vec_ok(out, 4, 4)) GO(float, 4) else GO(float, 1) }
     else return DDPM_E_ARG;
 #undef GO
@@ -742,6 +747,7 @@ extern "C" int ddpm_add(const ddpm_tensor* a, const ddpm_tensor* b, const ddpm_t
 #define GO(T, VEC) { AddOp<T, VEC> f{TV(*a), TV(*b), TV(*out)}; int64_t tot = (int64_t)out->N * out->H * out->W * (out->C / VEC); \
         if (launch_kernel(pix_kernel<T, VEC, decltype(f)>, dim3(pix_grid(tot)), dim3(NT), 0, st, out->N, out->H, out->W, out->C, f) != cudaSuccess) return (int)cudaGetLastError(); }
     if (dtype == DDPM_BF16) { if (vec_ok(a, 8, 2) && vec_ok(b, 8, 2) && vec_ok(out, 8, 2)) GO(bf16, 8) else GO(bf16, 1) }
+    else if (dtype == DDPM_F16) { if (vec_ok(a, 8, 2) && vec_ok(b, 8, 2) && vec_ok(out, 8, 2)) GO(f16, 8) else GO(f16, 1) }
     else if (dtype == DDPM_F32) { if (vec_ok(a, 4, 4) && vec_ok(b, 4, 4) && vec_ok(out, 4, 4)) GO(float, 4) else GO(float, 1) }
     else return DDPM_E_ARG;
 #undef GO
@@ -789,6 +795,7 @@ extern "C" int ddpm_colsum(const ddpm_tensor* dy, int dtype, float* out_nc, floa
         dim3 grid(blocks_per_image(dy->N, HW, ppi * 8), dy->N); \
         if (launch_kernel(colsum_kernel<T, VEC>, grid, dim3(NT), sizeof(float) * dy->C, st, v, out_nc, dbias) != cudaSuccess) return (int)cudaGetLastError(); }
     if (dtype == DDPM_BF16) { if (vec_ok(dy, 8, 2)) GO(bf16, 8) else GO(bf16, 1) }
+    else if (dtype == DDPM_F16) { if (vec_ok(dy, 8, 2)) GO(f16, 8) else GO(f16, 1) }
     else if (dtype == DDPM_F32) { if (vec_ok(dy, 4, 4)) GO(float, 4) else GO(float, 1) }
     else return DDPM_E_ARG;
 #undef GO

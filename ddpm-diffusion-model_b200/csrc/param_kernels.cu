@@ -229,6 +229,7 @@ extern "C" int ddpm_pack_weights(const float* w, int Cout, int Cin, int KH, int 
     int grid = (int)((total + 255) / 256); if (grid > 148 * 8) grid = 148 * 8;
     if (dtype == DDPM_F32) pack_kernel<float><<<grid, 256, 0, st>>>(w, Cout, Cin, KH, KW, CiP, CoP, (float*)w_fwd, (float*)w_dgrad);
     else if (dtype == DDPM_BF16) pack_kernel<bf16><<<grid, 256, 0, st>>>(w, Cout, Cin, KH, KW, CiP, CoP, (bf16*)w_fwd, (bf16*)w_dgrad);
+    else if (dtype == DDPM_F16) pack_kernel<f16><<<grid, 256, 0, st>>>(w, Cout, Cin, KH, KW, CiP, CoP, (f16*)w_fwd, (f16*)w_dgrad);
     else return DDPM_E_ARG;
     LAUNCH_OK();
     return 0;
@@ -261,6 +262,7 @@ extern "C" int ddpm_pack_weights_up2x(const float* w, int Cout, int Cin, void* o
     int grid = (int)((total + 255) / 256); if (grid > 148 * 8) grid = 148 * 8;
     if (dtype == DDPM_F32) pack_up2x_kernel<float><<<grid, 256, 0, st>>>(w, Cout, Cin, (float*)out);
     else if (dtype == DDPM_BF16) pack_up2x_kernel<bf16><<<grid, 256, 0, st>>>(w, Cout, Cin, (bf16*)out);
+    else if (dtype == DDPM_F16) pack_up2x_kernel<f16><<<grid, 256, 0, st>>>(w, Cout, Cin, (f16*)out);
     else return DDPM_E_ARG;
     LAUNCH_OK();
     return 0;
@@ -272,6 +274,12 @@ extern "C" int ddpm_pack_weights_up2x(const float* w, int Cout, int Cin, void* o
 // (32*taps contiguous floats per output channel) and both packed layouts are written in 64-byte runs -- the element-wise
 // version read with a stride of `taps` floats and scattered the dgrad copy two bytes at a time (139 us for 100 MB).
 #define PK_T 32
+// the entries live in device memory, so an unknown dtype code cannot be refused by the call: its copies are not written
+__device__ __forceinline__ void pack_store(void* dst, int dtype, int64_t o, float v) {
+    if (dtype == DDPM_BF16) stf<bf16>((bf16*)dst + o, v);
+    else if (dtype == DDPM_F16) stf<f16>((f16*)dst + o, v);
+    else if (dtype == DDPM_F32) ((float*)dst)[o] = v;
+}
 __global__ void __launch_bounds__(256) pack_batched_kernel(const ddpm_pack_entry* __restrict__ entries) {
     __shared__ float tile[PK_T][PK_T * 9 + 1];               // +1: the co-fastest read of the dgrad pass is conflict-free
     const ddpm_pack_entry e = entries[blockIdx.y];
@@ -296,7 +304,7 @@ __global__ void __launch_bounds__(256) pack_batched_kernel(const ddpm_pack_entry
             if (co < CoP && ci < CiP && e.wf) {
                 const float v = tile[r][c * taps + tap];
                 const int64_t o = ((int64_t)co * taps + tap) * CiP + ci;
-                if (e.dtype == DDPM_BF16) stf<bf16>((bf16*)e.wf + o, v); else ((float*)e.wf)[o] = v;
+                pack_store(e.wf, e.dtype, o, v);
             }
             // dgrad copy [ci][taps-1-tap][co]: co fastest
             const int r2 = l % PK_T, ct = l / PK_T, tap2 = ct % taps, c2 = ct / taps;
@@ -304,7 +312,7 @@ __global__ void __launch_bounds__(256) pack_batched_kernel(const ddpm_pack_entry
             if (co2 < CoP && ci2 < CiP && e.wd) {
                 const float v = tile[r2][c2 * taps + tap2];
                 const int64_t o = ((int64_t)ci2 * taps + (taps - 1 - tap2)) * CoP + co2;
-                if (e.dtype == DDPM_BF16) stf<bf16>((bf16*)e.wd + o, v); else ((float*)e.wd)[o] = v;
+                pack_store(e.wd, e.dtype, o, v);
             }
         }
     }

@@ -1,7 +1,7 @@
 """Host-side executor of the UNet hot path on the C ABI (libddpm_b200.so).
 
 Data layout in HBM
-  * activations: NHWC, element type bf16 (autocast) or fp32, every buffer carries a one-pixel zero
+  * activations: NHWC, element type bf16 or fp16 (autocast) or fp32, every buffer carries a one-pixel zero
     halo (`[N][H+2][W+2][pitch]`) that no kernel ever writes -> 3x3 convolutions need no bounds
     logic on the tensor-core path and skip-concatenation is a channel slice of one wide buffer
     (producers write at a channel offset; `torch.cat` of unet_backbone.py:206 disappears);
@@ -24,8 +24,9 @@ import torch
 from . import _lib
 from ._lib import Tensor as CT
 
-_TORCH = {_lib.F32: torch.float32, _lib.BF16: torch.bfloat16}
-_ESZ = {_lib.F32: 4, _lib.BF16: 2}
+_TORCH = {_lib.F32: torch.float32, _lib.BF16: torch.bfloat16, _lib.F16: torch.float16}
+_CODE = {v: k for k, v in _TORCH.items()}
+_ESZ = {_lib.F32: 4, _lib.BF16: 2, _lib.F16: 2}
 
 
 # ----------------------------------------------------------------------------------------------
@@ -238,7 +239,7 @@ class Exec:
         self.wcache = wcache if wcache is not None else GLOBAL_WCACHE
         self.rng = rng
         self.prefer_tc = 1 if prefer_tc else 0
-        self.use_tc = bool(prefer_tc) and dt == _lib.BF16     # tcgen05 kernels (channel padding to 16)
+        self.use_tc = bool(prefer_tc) and dt in (_lib.BF16, _lib.F16)     # tcgen05 kernels (channel padding to 16)
         self.wgrad_side = self.use_tc                         # ResBlock weight gradients on the side stream (weight_grads)
         self.stream = _lib.stream_for(device)
 
@@ -381,7 +382,7 @@ def wgrad(E: Exec, act: Act, dy: Act, w: torch.nn.Parameter, k: int, stride: int
     a.cin_valid = w.shape[1] if act.C != w.shape[1] else 0
     a.cout_valid = w.shape[0] if dy.C != w.shape[0] else 0
     a.dbias = _gptr(bias)
-    if E.use_tc and act.dt == _lib.BF16 and stride == 1:
+    if E.use_tc and act.dt in (_lib.BF16, _lib.F16) and stride == 1:
         need = int(_lib.lib.ddpm_wgrad_workspace_bytes(C.byref(a)))
         if need > 0:
             ws = E.workspace(need)
@@ -444,13 +445,12 @@ def add(E: Exec, a: Act, b: Act, out: Act) -> Act:
 
 
 def to_nhwc(E: Exec, x: torch.Tensor, halo=1, cpad: int = 0) -> Act:
-    """NCHW-shaped torch tensor (any strides, fp32/bf16) -> pooled NHWC activation (optionally with the
+    """NCHW-shaped torch tensor (any strides, fp32/bf16/fp16) -> pooled NHWC activation (optionally with the
     channel count padded with zeros to `cpad` for the tensor-core kernels)."""
     B, Cc, H, W = x.shape
-    src_dt = _lib.F32 if x.dtype == torch.float32 else _lib.BF16
-    if x.dtype not in (torch.float32, torch.bfloat16):
+    if x.dtype not in _CODE:
         x = x.float()
-        src_dt = _lib.F32
+    src_dt = _CODE[x.dtype]
     out = E.act(B, H, W, max(Cc, cpad), halo)
     sn, sc, sh, sw = x.stride()
     _lib.call("ddpm_nchw_to_nhwc", x.data_ptr(), src_dt, Cc, sn, sc, sh, sw, C.byref(out.desc()), E.dt, E.stream)
@@ -459,7 +459,7 @@ def to_nhwc(E: Exec, x: torch.Tensor, halo=1, cpad: int = 0) -> Act:
 
 def to_nchw(E: Exec, a: Act, out_dtype: torch.dtype) -> torch.Tensor:
     out = torch.empty((a.N, a.C, a.H, a.W), dtype=out_dtype, device=E.device)
-    dd = _lib.F32 if out_dtype == torch.float32 else _lib.BF16
+    dd = _CODE[out_dtype]
     sn, sc, sh, sw = out.stride()
     _lib.call("ddpm_nhwc_to_nchw", C.byref(a.desc()), a.dt, out.data_ptr(), dd, sn, sc, sh, sw, E.stream)
     return out

@@ -39,15 +39,20 @@ def _require_cuda(x: torch.Tensor, what: str) -> None:
 
 def compute_dtype(x: torch.Tensor) -> tuple:
     """(engine dtype code, dtype of the returned tensor) following the reference's autocast policy:
-    bf16 autocast -> bf16 activations and a bf16 result (conv/linear are autocast-to-bf16 ops,
-    unet_backbone.py:215 ends in a conv); otherwise fp32."""
+    bf16 / fp16 autocast -> activations and result in that dtype (conv/linear are autocast-to-lower-precision
+    ops, unet_backbone.py:215 ends in a conv); outside autocast a bf16 / fp16 input runs in its own dtype;
+    otherwise fp32."""
     if torch.is_autocast_enabled("cuda"):
         adt = torch.get_autocast_dtype("cuda")
         if adt == torch.bfloat16:
             return _lib.BF16, torch.bfloat16
-        raise NotImplementedError("ddpm_b200 supports bf16 autocast only (the reference trains with dtype='bf16')")
+        if adt == torch.float16:
+            return _lib.F16, torch.float16
+        raise NotImplementedError(f"ddpm_b200 supports bf16 and fp16 autocast, not {adt}")
     if x.dtype == torch.bfloat16:
         return _lib.BF16, torch.bfloat16
+    if x.dtype == torch.float16:
+        return _lib.F16, torch.float16
     return _lib.F32, torch.float32
 
 
@@ -148,7 +153,7 @@ def resblock_apply(blk, x: torch.Tensor, t_emb: torch.Tensor) -> torch.Tensor:
         sv, temb32 = saved
         dx, dtb = engine.resblock_bwd(E, blk, sv, engine.to_nhwc(E, dy))
         dtemb = engine.linear_bwd(E, temb32, blk.time_proj[1], True, dtb, None, False)
-        return engine.to_nchw(E, dx, x.dtype if x.dtype in (torch.float32, torch.bfloat16) else torch.float32), dtemb.to(t_emb.dtype)
+        return engine.to_nchw(E, dx, x.dtype if x.dtype in (torch.float32, torch.bfloat16, torch.float16) else torch.float32), dtemb.to(t_emb.dtype)
 
     return block_apply(blk, fwd, bwd, x, t_emb)
 

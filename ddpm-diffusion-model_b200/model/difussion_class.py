@@ -21,7 +21,9 @@ def _dt(x: torch.Tensor) -> int:
         return _lib.F32
     if x.dtype == torch.bfloat16:
         return _lib.BF16
-    raise TypeError(f"ddpm_b200: unsupported tensor dtype {x.dtype} (fp32 / bf16 only)")
+    if x.dtype == torch.float16:
+        return _lib.F16
+    raise TypeError(f"ddpm_b200: unsupported tensor dtype {x.dtype} (fp32 / bf16 / fp16 only)")
 
 
 def _f32c(x: torch.Tensor) -> torch.Tensor:
@@ -165,7 +167,7 @@ class Diffusion(nn.Module):
         if x0.dim() == 4 and x0.is_contiguous(memory_format=torch.channels_last) and not x0.is_contiguous():
             x_t = x_t.contiguous(memory_format=torch.channels_last)
         eps_pred = model_eps_pred_fn(x_t, t)
-        if eps_pred.dtype not in (torch.float32, torch.bfloat16):
+        if eps_pred.dtype not in (torch.float32, torch.bfloat16, torch.float16):
             eps_pred = eps_pred.float()
         w = _f32c(weight) if weight is not None else None
         return _MSE.apply(eps_pred, noise_c, w)
@@ -216,7 +218,7 @@ class Diffusion(nn.Module):
         if clip_x0 is None:
             clip_x0 = self.clamp_x0
         eps = model_eps_pred_fn(x_t, t)
-        if eps.dtype not in (torch.float32, torch.bfloat16):
+        if eps.dtype not in (torch.float32, torch.bfloat16, torch.float16):
             eps = eps.float()
         eps = eps if eps.is_contiguous() else eps.contiguous()
         x = _f32c(x_t)
@@ -244,7 +246,7 @@ class Diffusion(nn.Module):
         if noise is None:
             noise = torch.randn_like(x_t)
         eps = model_eps_pred_fn(x_t, t)
-        if eps.dtype not in (torch.float32, torch.bfloat16):
+        if eps.dtype not in (torch.float32, torch.bfloat16, torch.float16):
             eps = eps.float()
         eps = eps if eps.is_contiguous() else eps.contiguous()
         x = _f32c(x_t)

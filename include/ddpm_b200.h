@@ -11,8 +11,12 @@
  *   - no allocation, no host synchronisation, no hidden state except the schedule handle;
  *   - `stream` is a cudaStream_t passed as void*; all work is ordered on it (graph-capturable);
  *   - activations are NHWC with an optional zero halo of one pixel (struct ddpm_tensor), element
- *     type chosen by `dtype` (DDPM_F32 / DDPM_BF16); parameters and their gradients are fp32 in
- *     the reference's OIHW / [out,in] layouts;
+ *     type chosen by `dtype` (DDPM_F32 / DDPM_BF16 / DDPM_F16); parameters and their gradients are
+ *     fp32 in the reference's OIHW / [out,in] layouts;
+ *   - every entry point that accepts DDPM_BF16 accepts DDPM_F16 with the same shapes, the same
+ *     paths (tcgen05 wherever bf16 takes the tensor cores) and the same semantics; any other dtype
+ *     code returns DDPM_E_ARG.  fp32 -> fp16 conversions round to nearest and give +-inf beyond
+ *     65504 (IEEE, as torch.autocast does), so a GradScaler sees the overflow in the fp32 gradients;
  *   - kernels never write the halo, so a buffer whose halo was zeroed once stays valid.
  */
 #ifndef DDPM_B200_H
@@ -26,6 +30,7 @@ extern "C" {
 
 #define DDPM_F32 0
 #define DDPM_BF16 1
+#define DDPM_F16 2   /* IEEE binary16 */
 
 #define DDPM_E_ARG (-1)      /* invalid argument / unsupported shape */
 #define DDPM_E_NOTREADY (-2) /* schedule handle not initialised */
@@ -61,7 +66,7 @@ int ddpm_schedule_destroy(void* handle);
 int ddpm_q_sample(void* sched, const float* x0, const float* eps, const int64_t* t, float* xt,
                   int B, int64_t chw, void* stream);
 /* loss_simple tail (:113-116).  loss[0] += mean_b(w_b * mean_chw((noise-pred)^2)); caller zeroes
- * loss.  pred dtype f32/bf16, contiguous [B][chw].  weight may be NULL. */
+ * loss.  pred dtype f32/bf16/f16, contiguous [B][chw].  weight may be NULL. */
 int ddpm_mse_fwd(const void* pred, int pred_dtype, const float* noise, const float* weight,
                  float* loss, int B, int64_t chw, void* stream);
 /* d loss / d pred = 2 (pred-noise) w_b / (B*chw) * gout[0]; written in pred's dtype. */
@@ -163,7 +168,7 @@ int ddpm_colsum(const ddpm_tensor* dy, int dtype, float* out_nc, float* dbias, v
                                 * in[n, y+ty+py-1, x+tx+px-1] with the phase's pre-summed weights (ddpm_pack_weights_up2x).
                                 * `in` is [N,H,W,Cin], `out` the [N,2H,2W,Cout] view; KH = KW = 2, stride 1, up_phase = 2*py+px.
                                 * Four calls cover the output: 16 instead of 36 multiply-adds per low-resolution pixel pair
-                                * and the up-sampled tensor is never materialised.  Tensor-core path (bf16) only. */
+                                * and the up-sampled tensor is never materialised.  Tensor-core path (bf16 / fp16) only. */
 #define DDPM_EPI_ACCUM 1       /* out += result (in place; gradient fan-in, residual) */
 #define DDPM_EPI_DSILU 2       /* result *= silu'(z[n,c])  (time path backward) */
 typedef struct {
@@ -180,7 +185,7 @@ typedef struct {
     int32_t a_silu;        /* apply SiLU to the input operand on load (time path) */
     int32_t epi;           /* DDPM_EPI_* flags */
     int32_t dtype;
-    int32_t prefer_tc;     /* 1: use the tcgen05 kernel when the shape qualifies (bf16 only) */
+    int32_t prefer_tc;     /* 1: use the tcgen05 kernel when the shape qualifies (bf16 / fp16 only) */
     int32_t bias_n;        /* entries in `bias` (0: out.C); fewer when out carries zero-padded channels */
     /* Optional second operand: out = conv(in; w) + conv1x1(in2; w2) (+ bias ...), i.e. the ResBlock's `conv2(h) + skip(x)`
      * (unet_backbone.py:35,46) as ONE implicit GEMM whose K dimension is 9*Cin + Cin2.  in2 has the geometry of `out`
@@ -253,6 +258,7 @@ typedef struct {
     void* wd;            /* packed dgrad copy or NULL */
     int32_t Cout, Cin, taps, CiP, CoP, dtype;
 } ddpm_pack_entry;
+/* An entry whose dtype is not DDPM_F32 / DDPM_BF16 / DDPM_F16 is skipped (the entries are in device memory). */
 int ddpm_pack_weights_batched(const ddpm_pack_entry* entries_dev, int n, void* stream);
 
 /* ---------------- attention: attention.py:56-74 -------------------------------------------- */
@@ -268,7 +274,7 @@ int ddpm_attn_bwd(const ddpm_tensor* qkv, const ddpm_tensor* out, const ddpm_ten
                   int dtype, void* stream);
 /* fp32 elements of `scratch` ddpm_attn_bwd needs for this problem, from qkv / out alone: N*N-sized P and dS matrices
  * ([N][heads][HW][HW] * 2) for the CUDA-core kernels, one value per (image, head, query) for the tensor-core kernels
- * (bf16, head_dim 32 / 64 / 128, W <= 128, any H; 16-byte aligned, pitch a multiple of 8), which recompute P from the
+ * (bf16 / fp16, head_dim 32 / 64 / 128, W <= 128, any H; 16-byte aligned, pitch a multiple of 8), which recompute P from the
  * forward's log-sum-exp. */
 int64_t ddpm_attn_bwd_scratch_floats(const ddpm_tensor* qkv, const ddpm_tensor* out, int heads, int d, int dtype);
 
